@@ -8,7 +8,9 @@ A "step" is one pass of the hot path over one batch: `sampling_ihqgpt` for `--ba
 positions (320 codes per image), random-init weights of the named architecture (the reference's own
 `measure_throughput` protocol: config only, no checkpoint; top-k/top-p None, T = 1, measure_throughput/__main__.py:93-104).
 Weak scaling: the per-GPU batch is fixed, ranks share nothing but one final all-gather of the code grids.
-Prints ONE JSON line on rank 0.
+Prints ONE JSON line on rank 0.  `--dump-outputs DIR` also writes the code grids of the last timed step (float32 .npy);
+inputs, weights and Philox keys depend only on the arguments, so two builds run with the same arguments can be compared
+output for output.
 """
 from __future__ import annotations
 
@@ -33,7 +35,8 @@ CONFIGS = {"imagenet_l12": "imagenet_l12.yaml", "imagenet_l24": "imagenet_l24.ya
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps; --impl reference times at most 3 when it falls back to "
+                    "the oracle port, and fewer when --ref-budget-s runs out (its JSON line reports both counts)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="graft", choices=["graft", "reference"])
     ap.add_argument("--model", default="imagenet_l12", choices=sorted(CONFIGS))
@@ -51,7 +54,37 @@ def parse_args():
     ap.add_argument("--ref-budget-s", type=float, default=150.0, help="--impl reference: wall-clock budget of the timed steps")
     ap.add_argument("--no-ref-gpu", action="store_true", help="skip extras.reference_gpu_fp16_autocast")
     ap.add_argument("--ref-gpu-batch", type=int, default=0, help="batch of the reference-on-GPU extra (0 = --batch)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the code grids of the last timed step as DIR/<name>.npy (float32) for output comparison")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and args.impl != "graft":
+        ap.error("--dump-outputs applies to --impl graft")
+    return args
+
+
+DUMP_LIMIT_BYTES = (64 << 20) - 4096        # 64 MB in all, less room for the .npy headers
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Writes each [rows, ...] array as out_dir/<name>.npy in float32 (the codes are integers < 2^24, exact in it).
+    When all of them together exceed DUMP_LIMIT_BYTES, the same fixed, seeded sample of rows is taken from each, and
+    the sorted row indices go to out_dir/sampled_rows.npy."""
+    import numpy as np
+    import torch
+    rows = next(iter(arrays.values())).shape[0]
+    row_bytes = sum(t[0].numel() * 4 for t in arrays.values())
+    keep = None
+    if rows * row_bytes > DUMP_LIMIT_BYTES:
+        n = DUMP_LIMIT_BYTES // (row_bytes + 4)     # + 4: the row's index in sampled_rows.npy
+        keep = torch.randperm(rows, generator=torch.Generator().manual_seed(0))[:n].sort().values
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().cpu()
+        np.save(os.path.join(out_dir, f"{name}.npy"), (t if keep is None else t[keep]).numpy().astype(np.float32))
+    if keep is not None:
+        np.save(os.path.join(out_dir, "sampled_rows.npy"), keep.numpy().astype(np.float32))
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -460,6 +493,10 @@ def run_graft_arm(args, rank: int, world: int, local_rank: int):
     note(f"timed region done: {ms / args.steps:.1f} ms/step")
     launches = eng.last_launch_count * args.steps
     assert int(ct.min()) >= 0 and int(ct.max()) < s2.vocab_size_top and tuple(ct.shape) == (world * B, S)
+    if args.dump_outputs and rank == 0:
+        # now, before the kernel table's replay writes into these buffers again
+        dump_outputs(args.dump_outputs, {"codes_top": ct, "codes_bot": cb})
+        note(f"outputs of the last timed step written to {args.dump_outputs}")
 
     # ---- sharding invariance, checked on the grids of the last timed step: rank 0 re-samples ANOTHER shard of the global
     #      batch on its own GPU (that shard's conditioning, its global row offset, the same Philox key) and compares it

@@ -8,6 +8,8 @@ Run in the build container (where /root/reference exists):
     python -m oracle.make_golden --stage1       # only the stage-1 decode golden (SimRQGAN2Generator.decode_code)
     python -m oracle.make_golden --variants     # only the 8f-3 model variants (reduce / 2d / top2bot / bidirectional)
     python -m oracle.make_golden --all
+    python -m oracle.make_golden --live-checks  # only the seeded runs the tests also repeat against the live reference
+                                                # (written from the oracle; re-checked against the reference when present)
 
 The reference has no tests or golden vectors of its own (SURVEY.md section 4), so these files are the
 pinned known answers for the hot path: they are produced by the reference's own code
@@ -259,7 +261,70 @@ def golden_filters(name):
     print(name, "done")
 
 
+SKW = dict(top_k_top=8, top_p_top=0.9, top_k_bot=16, top_p_bot=0.95, softmax_temperature=[0.9, 1.1])
+# seeded runs that tests/test_oracle_golden.py compares with these files, and with the live reference when it is present
+LIVE_CHECKS = {
+    "tiny_cls_scalar_class.npz": [
+        dict(run="greedy", cfg={}, seed=11, cond=4, B=3, S=16, torch_seed=None, kw=GREEDY),
+        dict(run="stochastic", cfg={}, seed=11, cond=2, B=3, S=8, torch_seed=5,
+             kw=dict(top_k_top=20, top_p_top=0.9, top_k_bot=30, top_p_bot=0.8, softmax_temperature=[0.9, 1.2]))],
+    "tiny_variants_stochastic.npz": [
+        dict(run="top2bot", cfg=dict(model_type="top2bot"), seed=3, cond=4, B=3, S=6, torch_seed=5, kw=SKW),
+        dict(run="bidirectional", cfg=dict(model_type="bidirectional"), seed=3, cond=4, B=3, S=6, torch_seed=5, kw=SKW),
+        dict(run="reduce_2d_uncond", cfg=dict(embedding_type="reduce", position_embedding="2d", cond="uncond"), seed=3,
+             cond=None, B=3, S=6, torch_seed=5, kw=SKW)],
+    "tiny3_cls_stochastic.npz": [
+        dict(run="stochastic", cfg={}, seed=56, cond=4, B=3, S=5, torch_seed=5,
+             kw=dict(top_k=[8, 16, 32], top_p=[0.9, 0.95, 0.8], softmax_temperature=[0.9, 1.1, 1.0]))],
+}
+
+
+def live_check_run(name, run, reference=False):
+    """Code grids of one LIVE_CHECKS run: the oracle's, or with reference=True the unmodified reference's (on CPU, the same
+    weights and torch seed)."""
+    if name.startswith("tiny3"):
+        from oracle import hq3_oracle as O3
+        cfg = O3.HQ3Config.from_dict({**O3.TINY3.to_dict(), **run["cfg"]})
+        P = O3.make_params(cfg, seed=run["seed"])
+    else:
+        cfg = O.HQConfig(**{**O.TINY.to_dict(), **run["cfg"]})
+        P = O.make_params(cfg, seed=run["seed"], init="rich")
+    if run["torch_seed"] is not None:
+        torch.manual_seed(run["torch_seed"])
+    S = run["S"]
+    if name.startswith("tiny3"):
+        if reference:
+            return R.reference_sample_hq3(R.build_reference_hq3(cfg, P), run["B"], run["cond"], max_seq_len=S, **run["kw"])
+        return O3.sample(P, cfg, run["cond"], run["B"], max_seq_len=S, **run["kw"])
+    if reference:
+        return R.reference_sample(R.build_reference_model(cfg, P), run["B"], run["cond"], max_seq_len=S, **run["kw"])
+    return O.sample(P, cfg, run["cond"], run["B"], max_seq_len=S, **run["kw"])
+
+
+def golden_live_checks():
+    """Known answers of the LIVE_CHECKS runs, so that a checkout without the reference tree still compares with them.
+    The grids are the oracle's; the live tests showed them bit-identical to the unmodified reference's on exactly these
+    inputs, and when the reference tree is present every run is checked against it again before anything is written."""
+    checked = R.reference_available()
+    for name, runs in LIVE_CHECKS.items():
+        out = {}
+        for run in runs:
+            got = live_check_run(name, run)
+            if checked:
+                assert all(torch.equal(a, b) for a, b in zip(got, live_check_run(name, run, reference=True))), (name, run)
+            for level, codes in zip(("top", "mid", "bot") if len(got) == 3 else ("top", "bot"), got):
+                out[f"{run['run']}_{level}"] = codes.numpy()
+        src = ("oracle output, checked bit-identical to the reference on these inputs when written" if checked else
+               "oracle output; the live tests found the oracle bit-identical to the reference on these inputs")
+        np.savez_compressed(os.path.join(GOLDEN_DIR, name),
+                            meta=np.array(json.dumps(dict(torch=torch.__version__, runs=runs, source=src))), **out)
+        print(name, "done", "(re-checked against the reference)" if checked else "")
+
+
 def main():
+    if "--live-checks" in sys.argv:
+        golden_live_checks()
+        return 0
     if not R.reference_available():
         print("reference tree absent - goldens can only be generated in the build container", file=sys.stderr)
         return 1

@@ -6,6 +6,8 @@ import re
 import pytest
 import torch
 
+from oracle import ref_shim as R
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -81,11 +83,12 @@ def test_config_loader_restates_reference_defaults():
         engine_kwargs(H.merge_config({"stage2": {"type": "top", "hparams": {}}}))
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/configs"), reason="reference tree only exists in the build container")
+@pytest.mark.skipif(not os.path.isdir(os.path.join(R.REFERENCE_ROOT, "configs")),
+                    reason="needs the original project's configs/ tree (HQ_REFERENCE_ROOT); not part of this repository")
 def test_reference_yaml_files_load_unchanged():
     import hqtransformer_b200 as H
     from hqtransformer_b200.config import engine_kwargs
-    base = "/root/reference/configs/master/stage2"
+    base = os.path.join(R.REFERENCE_ROOT, "configs", "master", "stage2")
     for rel, L, Ld in (("imagenet/hqtransformer-embtrans1-soft1-layer12-top8x8.yaml", 12, None),
                        ("imagenet/hqtransformer-embtrans1-soft1-layer42-top8x8.yaml", 42, 6),
                        ("cc15m/hqtransformer-embtrans1-soft1-layer12-top8x8-cc15m.yaml", 12, None)):
@@ -168,6 +171,28 @@ def test_committed_bench_evidence_carries_the_contract_keys():
     assert not set(d["clocks"]["reasons"]) & {"hw_slowdown", "hw_thermal_slowdown", "sw_thermal_slowdown"}
     ra = d["roofline_attention"]
     assert ra["bound"] == "hbm" and abs(ra["frac"] - ra["achieved"] / ra["peak"]) < 1e-9
+
+
+def test_bench_dump_outputs_is_exact_and_samples_rows_over_the_limit(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: code grids round-trip exactly through float32 .npy; above the size limit every array keeps
+    the same seeded sample of rows, listed in sampled_rows.npy."""
+    import numpy as np
+    import bench
+    g = torch.Generator().manual_seed(0)
+    ct, cb = torch.randint(0, 16384, (40, 64), generator=g), torch.randint(0, 16384, (40, 64, 4), generator=g)
+    bench.dump_outputs(str(tmp_path / "all"), {"codes_top": ct, "codes_bot": cb})
+    assert sorted(os.listdir(tmp_path / "all")) == ["codes_bot.npy", "codes_top.npy"]
+    top = np.load(tmp_path / "all" / "codes_top.npy")
+    assert top.dtype == np.float32 and np.array_equal(top, ct.numpy())
+    assert np.array_equal(np.load(tmp_path / "all" / "codes_bot.npy"), cb.numpy())
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 10 * (64 + 256) * 4 + 40)
+    for d in ("s1", "s2"):
+        bench.dump_outputs(str(tmp_path / d), {"codes_top": ct, "codes_bot": cb})
+    rows = np.load(tmp_path / "s1" / "sampled_rows.npy").astype(np.int64)
+    assert len(rows) == 10 and np.all(np.diff(rows) > 0)
+    assert np.array_equal(rows, np.load(tmp_path / "s2" / "sampled_rows.npy").astype(np.int64))
+    assert np.array_equal(np.load(tmp_path / "s1" / "codes_top.npy"), ct.numpy()[rows])
+    assert np.array_equal(np.load(tmp_path / "s1" / "codes_bot.npy"), cb.numpy()[rows])
 
 
 def test_encode_prompts_pads_and_truncates_like_the_reference_dataset():
