@@ -40,6 +40,13 @@ class HQRunArgs(C.Structure):
                 ("shared_prefix", C.c_int32), ("reserved", C.c_int32)]
 
 
+class HQDebugEpi(C.Structure):
+    _fields_ = [(n, C.c_int32) for n in (
+        "epi", "tile", "ks1", "D", "sec0", "rpb", "t_stride", "t0", "w_row_off", "ldo", "splits", "reserved")] + \
+        [("split_stride", C.c_uint64)] + \
+        [(n, C.c_void_p) for n in ("bias", "q", "kdst", "vdst", "vdup", "x", "out", "outf")]
+
+
 class HQS1Config(C.Structure):
     _fields_ = [("embed_dim", C.c_int32), ("n_embed", C.c_int32), ("z_channels", C.c_int32), ("resolution", C.c_int32),
                 ("ch", C.c_int32), ("ch_mult", C.c_int32 * 8), ("n_levels", C.c_int32), ("num_res_blocks", C.c_int32),
@@ -63,6 +70,11 @@ PROTOTYPES = {
     "hq_chain_launch_count": (C.c_int64, [C.c_void_p]),
     "hq_debug_gemm": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
                              C.c_void_p]),
+    "hq_debug_gemm_epi": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
+                                    C.POINTER(HQDebugEpi), C.c_void_p]),
+    "hq_debug_layernorm": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
+                                     C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_size_t, C.c_void_p,
+                                     C.c_void_p]),
     "hq_debug_philox": (C.c_int, [C.c_uint64, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
     "hq_debug_sample": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_float, C.c_int, C.c_float, C.c_uint64, C.c_uint64,
                                   C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -2023,6 +2023,162 @@ extern "C" int hq_debug_gemm(int prec, const void* A, const void* W, float* C, i
   return HQ_OK;
 }
 
+// The fused epilogue of one hq_debug_gemm_epi launch as the GEMM kernels take it.
+template <typename AT>
+static EpiParams<AT> debug_epi_params(const hq_debug_epi* d) {
+  EpiParams<AT> ep;
+  memset(&ep, 0, sizeof(ep));
+  ep.bias = d->bias;
+  ep.q = static_cast<AT*>(d->q); ep.kdst = static_cast<AT*>(d->kdst); ep.vdst = static_cast<AT*>(d->vdst);
+  ep.vdup = static_cast<AT*>(d->vdup);
+  ep.D = d->D; ep.sec0 = d->sec0; ep.rpb = d->rpb; ep.t_stride = d->t_stride; ep.t0 = d->t0;
+  ep.x = d->x;
+  ep.out = static_cast<AT*>(d->out);
+  ep.outf = d->outf; ep.ldo = d->ldo; ep.split_stride = static_cast<size_t>(d->split_stride);
+  return ep;
+}
+
+static const char* debug_epi_invalid(int prec, int w_rows, int M, int N, int K, const hq_debug_epi* d) {
+  if (prec != HQ_PREC_BF16 && prec != HQ_PREC_FP32) return "unknown precision";
+  if (M < 1 || N < 32 || N % 32 != 0 || K < 64 || K % 64 != 0) return "shape: need M >= 1, N % 32 == 0, K % 64 == 0";
+  if (d->w_row_off < 0 || w_rows < d->w_row_off + N) return "W needs w_rows >= w_row_off + N rows";
+  if (d->epi < EPI_QKV || d->epi > EPI_F32) return "epi must be QKV, RESID, GELU or F32";
+  if (d->splits < 1 || d->splits > LN_MAXFOLD || (K / 64) % d->splits != 0) return "splits must divide K / 64 (1..6)";
+  if (d->splits > 1 && d->epi != EPI_F32) return "split-K is an EPI_F32 launch only";
+  if (prec == HQ_PREC_FP32) {
+    if (d->tile != 0 || d->splits != 1) return "the fp32 engine has one kernel: tile 0, splits 1";
+  } else {
+    const int t = d->tile;
+    const bool pair = t == 32 || t == 64 || t == 96 || t == 128 || t == 192 || t == 256;
+    if (pair ? N % t != 0 : (t == -128 ? N % 128 != 0 : ((t == 0 || t == -64) ? N % 64 != 0 : true)))
+      return "tile must be 0, 32, 64, 96, 128, 192, 256, -64 or -128 and divide N";
+  }
+  switch (d->epi) {
+    case EPI_QKV:
+      if (d->D < 32 || d->D % 32 != 0 || N % d->D != 0 || d->sec0 < 0 || d->sec0 + N / d->D > 3)
+        return "QKV: D % 32 == 0 and the columns sec0 .. sec0 + N / D - 1 within q, k, v";
+      if (d->rpb < 1 || d->t0 < 0 || d->t_stride < d->t0 + d->rpb) return "QKV: cache slots t0 .. t0 + rpb - 1 within t_stride";
+      if ((d->sec0 == 0 && d->q == nullptr) || d->kdst == nullptr || d->vdst == nullptr) return "QKV: q, kdst, vdst";
+      break;
+    case EPI_RESID:
+      if (d->x == nullptr) return "RESID: x";
+      break;
+    case EPI_GELU:
+      if (d->out == nullptr) return "GELU: out";
+      break;
+    default:
+      if (d->outf == nullptr || d->ldo < N || d->ldo % 4 != 0 || d->split_stride % 4 != 0) return "F32: outf, ldo >= N, ldo % 4 == 0";
+  }
+  return nullptr;
+}
+
+extern "C" int hq_debug_gemm_epi(int prec, const void* A, const void* W, int w_rows, int M, int N, int K,
+                                 const hq_debug_epi* d, void* stream) {
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const char* bad = (A == nullptr || W == nullptr || d == nullptr) ? "null operand" : debug_epi_invalid(prec, w_rows, M, N, K, d);
+  if (bad != nullptr) {
+    set_err(nullptr, "hq_debug_gemm_epi: %s", bad);
+    return HQ_ERR_INVALID;
+  }
+  hq_ctx tmp;   // launch bookkeeping, the pinned tile width and ring-stage depth
+  tmp.dbg.force_bn = d->tile;
+  tmp.dbg.gemm_ks1 = d->ks1 != 0;
+  if (prec == HQ_PREC_FP32) {
+    // as gemm_any: the weight rows start w_row_off rows in
+    const float* A32 = static_cast<const float*>(A);
+    const float* W32 = static_cast<const float*>(W) + static_cast<size_t>(d->w_row_off) * K;
+    const EpiParams<float> ep = debug_epi_params<float>(d);
+    switch (d->epi) {
+      case EPI_QKV: gemm_f32<EPI_QKV>(&tmp, st, A32, W32, M, N, K, ep); break;
+      case EPI_RESID: gemm_f32<EPI_RESID>(&tmp, st, A32, W32, M, N, K, ep); break;
+      case EPI_GELU: gemm_f32<EPI_GELU>(&tmp, st, A32, W32, M, N, K, ep); break;
+      default: gemm_f32<EPI_F32>(&tmp, st, A32, W32, M, N, K, ep);
+    }
+  } else {
+    int dev = 0;
+    HQ_CUDA(nullptr, cudaGetDevice(&dev));
+    int rc = check_device(&tmp, dev);
+    if (rc == HQ_OK) rc = get_encode_fn(&tmp, &tmp.encode);
+    if (rc == HQ_OK) rc = set_gemm_attrs(&tmp);
+    // A rows padded to the 128-row tile by a zero-filled staging copy, as hq_debug_gemm
+    const int Mp = (M + 127) / 128 * 128;
+    void* Ap = nullptr;
+    if (rc == HQ_OK) {
+      HQ_CUDA(nullptr, cudaMalloc(&Ap, static_cast<size_t>(Mp) * K * 2));
+      cudaMemsetAsync(Ap, 0, static_cast<size_t>(Mp) * K * 2, st);
+      cudaMemcpyAsync(Ap, A, static_cast<size_t>(M) * K * 2, cudaMemcpyDeviceToDevice, st);
+    }
+    CUtensorMap mA, mA3, mW;
+    PairMaps mWp;
+    if (rc == HQ_OK) rc = make_map(&tmp, &mA, Ap, Mp, K, 128);
+    if (rc == HQ_OK && K >= 128) rc = make_map3(&tmp, &mA3, Ap, Mp, K, 128, 2);
+    if (rc == HQ_OK) rc = make_map(&tmp, &mW, const_cast<void*>(W), w_rows, K, 64);
+    if (rc == HQ_OK) rc = make_pair_maps(&tmp, &mWp, const_cast<void*>(W), w_rows, K);
+    if (rc == HQ_OK) {
+      const EpiParams<bf16> ep = debug_epi_params<bf16>(d);
+      const CUtensorMap* a3 = K >= 128 ? &mA3 : nullptr;
+      const int off = d->w_row_off;
+      switch (d->epi) {
+        case EPI_QKV: gemm_bf16<EPI_QKV>(&tmp, st, mA, a3, mW, mWp, off, M, N, K, ep); break;
+        case EPI_RESID: gemm_bf16<EPI_RESID>(&tmp, st, mA, a3, mW, mWp, off, M, N, K, ep); break;
+        case EPI_GELU: gemm_bf16<EPI_GELU>(&tmp, st, mA, a3, mW, mWp, off, M, N, K, ep); break;
+        default: gemm_bf16<EPI_F32>(&tmp, st, mA, a3, mW, mWp, off, M, N, K, ep, d->splits);
+      }
+    }
+    cudaError_t se = cudaStreamSynchronize(st);
+    if (Ap) cudaFree(Ap);
+    if (rc != HQ_OK) {
+      g_last_error = tmp.err;
+      return rc;
+    }
+    if (se != cudaSuccess) {
+      set_err(nullptr, "hq_debug_gemm_epi: %s", cudaGetErrorString(se));
+      return HQ_ERR_CUDA;
+    }
+  }
+  cudaError_t e = tmp.launch_err;
+  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+  if (e != cudaSuccess) {
+    set_err(nullptr, "hq_debug_gemm_epi: %s", cudaGetErrorString(e));
+    return HQ_ERR_CUDA;
+  }
+  return HQ_OK;
+}
+
+extern "C" int hq_debug_layernorm(int prec_out, float* x, const float* gamma, const float* beta, const float* add, void* out,
+                                  int rows, int D, int in_group, int in_mul, int in_off, int out_mul, const float* fold,
+                                  int n_fold, size_t fold_stride, const float* fold_bias, void* stream) {
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const char* bad = nullptr;
+  if (prec_out != HQ_PREC_BF16 && prec_out != HQ_PREC_FP32) bad = "unknown precision";
+  else if (!x || !gamma || !beta || !out) bad = "null x, gamma, beta or out";
+  else if (rows < 1 || D < 4 || D % 4 != 0) bad = "rows >= 1 and D % 4 == 0";
+  else if (in_group < 1 || in_mul < 0 || in_off < 0 || out_mul < 1) bad = "row map";
+  else if (n_fold < 0 || n_fold > LN_MAXFOLD || (n_fold > 0) != (fold != nullptr) || fold_stride % 4 != 0)
+    bad = "fold: n_fold 0..6 partial sums, given iff n_fold > 0";
+  if (bad != nullptr) {
+    set_err(nullptr, "hq_debug_layernorm: %s", bad);
+    return HQ_ERR_INVALID;
+  }
+  hq_ctx tmp;   // launch bookkeeping + the row width
+  tmp.D = D;
+  Fold f;
+  f.partial = fold; f.n = n_fold; f.stride = fold_stride; f.bias = fold_bias;
+  if (prec_out == HQ_PREC_BF16)
+    layernorm_rows<bf16>(&tmp, st, "layernorm", x, gamma, beta, add, static_cast<bf16*>(out), rows, in_group, in_mul, in_off,
+                         out_mul, f);
+  else
+    layernorm_rows<float>(&tmp, st, "layernorm", x, gamma, beta, add, static_cast<float*>(out), rows, in_group, in_mul, in_off,
+                          out_mul, f);
+  cudaError_t e = tmp.launch_err;
+  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+  if (e != cudaSuccess) {
+    set_err(nullptr, "hq_debug_layernorm: %s", cudaGetErrorString(e));
+    return HQ_ERR_CUDA;
+  }
+  return HQ_OK;
+}
+
 extern "C" int hq_debug_philox(uint64_t seed, const uint32_t counter[4], uint32_t out[4]) {
   uint32_t o[4];
   philox4x32_10(static_cast<uint32_t>(seed), static_cast<uint32_t>(seed >> 32), counter[0], counter[1], counter[2],

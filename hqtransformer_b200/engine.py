@@ -272,6 +272,61 @@ def debug_gemm(A: torch.Tensor, W: torch.Tensor, tile: int = 0) -> torch.Tensor:
     return out
 
 
+EPI_QKV, EPI_RESID, EPI_GELU, EPI_F32 = 0, 1, 2, 3
+
+
+def debug_gemm_epi(A: torch.Tensor, W: torch.Tensor, epi: int, *, N: Optional[int] = None, w_row_off: int = 0,
+                   tile: int = 0, ks1: bool = False, bias: Optional[torch.Tensor] = None,
+                   q: Optional[torch.Tensor] = None, kdst: Optional[torch.Tensor] = None, vdst: Optional[torch.Tensor] = None,
+                   vdup: Optional[torch.Tensor] = None, D: int = 0, sec0: int = 0, rpb: int = 1, t_stride: int = 1, t0: int = 0,
+                   x: Optional[torch.Tensor] = None, out: Optional[torch.Tensor] = None, outf: Optional[torch.Tensor] = None,
+                   ldo: int = 0, splits: int = 1, split_stride: int = 0) -> None:
+    """A [M, K] @ W[w_row_off : w_row_off + N]^T through the engine's GEMM kernels with fused epilogue `epi` (EPI_QKV,
+    EPI_RESID, EPI_GELU or EPI_F32), writing into the caller's buffers in place; see hq_debug_epi in include/hqgraft.h.
+    bf16 A / W take the tcgen05 kernels (`tile` and `ks1` pin the plan), fp32 the CUDA-core kernel.  Synchronous."""
+    lib = _lib.load()
+    assert A.is_cuda and W.is_cuda and A.dtype == W.dtype and A.is_contiguous() and W.is_contiguous()
+    act = A.dtype
+    for t in (q, kdst, vdst, vdup, out):
+        assert t is None or (t.dtype == act and t.is_contiguous() and t.device == A.device)
+    for t in (bias, x, outf):
+        assert t is None or (t.dtype == torch.float32 and t.is_contiguous() and t.device == A.device)
+    M, K = A.shape
+    w_rows = W.shape[0]
+    if N is None:
+        N = w_rows - w_row_off
+    e = _lib.HQDebugEpi(epi=epi, tile=tile, ks1=int(bool(ks1)), D=D, sec0=sec0, rpb=rpb, t_stride=t_stride, t0=t0,
+                        w_row_off=w_row_off, ldo=ldo, splits=splits, reserved=0, split_stride=split_stride,
+                        bias=_ptr(bias), q=_ptr(q), kdst=_ptr(kdst), vdst=_ptr(vdst), vdup=_ptr(vdup), x=_ptr(x),
+                        out=_ptr(out), outf=_ptr(outf))
+    prec = _lib.HQ_PREC_BF16 if act == torch.bfloat16 else _lib.HQ_PREC_FP32
+    with torch.cuda.device(A.device):
+        st = torch.cuda.current_stream(A.device).cuda_stream
+        check(lib.hq_debug_gemm_epi(prec, A.data_ptr(), W.data_ptr(), w_rows, M, N, K, C.byref(e), C.c_void_p(st)), None,
+              "hq_debug_gemm_epi")
+
+
+def debug_layernorm(x: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, out: torch.Tensor, rows: int, *,
+                    add: Optional[torch.Tensor] = None, in_group: int = 1, in_mul: int = 1, in_off: int = 0,
+                    out_mul: int = 1, fold: Optional[torch.Tensor] = None, n_fold: int = 0, fold_stride: int = 0,
+                    fold_bias: Optional[torch.Tensor] = None) -> None:
+    """The engine's LayerNorm launch (layernorm_kernel, instantiation chosen by n_fold as in the sampler) on fp32 x
+    [*, D], in place: out[r * out_mul] = LN(x[(r // in_group) * in_mul + in_off + r % in_group]) * gamma + beta (+ add);
+    with n_fold > 0 that x row first gets fold_bias + the partial sums fold.view(-1)[s * fold_stride + row * D ...] added
+    and written back.  `out` is bf16 or fp32.  Synchronous."""
+    lib = _lib.load()
+    D = x.shape[-1]
+    for t in (x, gamma, beta, add, fold, fold_bias):
+        assert t is None or (t.is_cuda and t.dtype == torch.float32 and t.is_contiguous())
+    assert out.is_contiguous() and out.dtype in (torch.bfloat16, torch.float32)
+    prec = _lib.HQ_PREC_BF16 if out.dtype == torch.bfloat16 else _lib.HQ_PREC_FP32
+    with torch.cuda.device(x.device):
+        st = torch.cuda.current_stream(x.device).cuda_stream
+        check(lib.hq_debug_layernorm(prec, x.data_ptr(), gamma.data_ptr(), beta.data_ptr(), _ptr(add), out.data_ptr(), rows,
+                                     D, in_group, in_mul, in_off, out_mul, _ptr(fold), n_fold, fold_stride, _ptr(fold_bias),
+                                     C.c_void_p(st)), None, "hq_debug_layernorm")
+
+
 def debug_attention(q: torch.Tensor, K: torch.Tensor, V: torch.Tensor, n_keys: int, variant: int = 0) -> torch.Tensor:
     """Single-query attention of every row of q [B, D] over the first n_keys rows of its cache K / V [B, T, D]
     (head size 64) through the engine's decode kernels; variant 0 = engine choice, 1 = scalar bulk-staged kernel."""

@@ -214,6 +214,41 @@ size_t hq_device_bytes(const hq_ctx* ctx);
  * -64 / -128 = single-CTA kernel. */
 int hq_debug_gemm(int prec, const void* A, const void* W, float* C, int M, int N, int K, int tile, void* stream);
 
+/* Fused epilogue of one hq_debug_gemm_epi launch (the sampler's EpiParams).  Device pointers; q, kdst, vdst, vdup and out
+ * in the precision's activation type (bf16 | fp32), bias, x and outf fp32. */
+typedef struct hq_debug_epi {
+  int32_t epi;          /* 0 QKV, 1 RESID, 2 GELU, 3 F32 (the sampler's EPI_* values) */
+  int32_t tile;         /* as hq_debug_gemm's `tile` (bf16 only; the fp32 engine has one kernel: 0) */
+  int32_t ks1;          /* 1: one 64-wide k-block per ring stage even where the engine would stage two */
+  int32_t D, sec0, rpb, t_stride, t0;   /* QKV: column n is section sec0 + n / D (0 q, 1 k, 2 v); row m goes to q[m] and
+                                           to cache row (m / rpb) * t_stride + t0 + m % rpb of kdst / vdst */
+  int32_t w_row_off;    /* the product uses W rows w_row_off .. w_row_off + N - 1 */
+  int32_t ldo, splits;  /* F32: row stride of outf; K slices, slice s writes outf + s * split_stride (bf16 only) */
+  int32_t reserved;
+  uint64_t split_stride;
+  const float* bias;    /* [N] or NULL; QKV / RESID / GELU */
+  void* q;              /* QKV: [M, D] (sec0 == 0) */
+  void* kdst;
+  void* vdst;
+  void* vdup;           /* QKV: optional [M, D] second copy of the v columns */
+  float* x;             /* RESID: [M, N], x += C + bias */
+  void* out;            /* GELU: [M, N] = gelu(C + bias) */
+  float* outf;          /* F32: [M, ldo] per K slice */
+} hq_debug_epi;
+
+/* C = A[M,K] * W[w_row_off .. w_row_off + N - 1, K]^T (W has w_rows rows) through the sampler's GEMM kernels and the
+ * epilogue `e` describes, synchronously on `stream`.  HQ_ERR_INVALID for combinations the engine never launches
+ * (a tile that does not divide N, splits that do not divide K / 64, split-K outside EPI_F32, ...). */
+int hq_debug_gemm_epi(int prec, const void* A, const void* W, int w_rows, int M, int N, int K, const hq_debug_epi* e,
+                      void* stream);
+
+/* The sampler's LayerNorm launch: out[r * out_mul] = LN(x[(r / in_group) * in_mul + in_off + r % in_group]) * gamma + beta
+ * (+ add), rows r < rows, out bf16 (prec_out == HQ_PREC_BF16) or fp32.  n_fold > 0: x row += fold_bias + the n_fold
+ * partial sums fold + s * fold_stride (same row index), written back before the normalisation.  fp32 device pointers. */
+int hq_debug_layernorm(int prec_out, float* x, const float* gamma, const float* beta, const float* add, void* out, int rows,
+                       int D, int in_group, int in_mul, int in_off, int out_mul, const float* fold, int n_fold,
+                       size_t fold_stride, const float* fold_bias, void* stream);
+
 /* Philox4x32-10 block for (seed, counter) - known-answer test of the RNG; host pointers. */
 int hq_debug_philox(uint64_t seed, const uint32_t counter[4], uint32_t out[4]);
 
