@@ -10,7 +10,8 @@ ABI_VERSION = 8
 
 HQ_OK = 0
 HQ_COND_CLS, HQ_COND_TXT, HQ_COND_UNCOND = 0, 1, 2
-HQ_PREC_BF16, HQ_PREC_FP32 = 0, 1
+HQ_PREC_BF16, HQ_PREC_FP32, HQ_PREC_F16 = 0, 1, 2
+HQ_PREC = {"bf16": HQ_PREC_BF16, "fp32": HQ_PREC_FP32, "fp16": HQ_PREC_F16}
 HQ_F32, HQ_BF16, HQ_F16 = 0, 1, 2
 HQ_MODEL = {"parallel": 0, "top2bot": 1, "bidirectional": 2}
 HQ_EMB = {"transformer1": 0, "reduce": 1}

@@ -4,12 +4,16 @@
 
 #include <cuda.h>
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
+
+#include <type_traits>
 
 namespace hq {
 
 typedef __nv_bfloat16 bf16;
+typedef __half f16;   // IEEE binary16: the element type of the HQ_PREC_F16 engine
 
 // ------------------------------------------------------------------------------------------------
 // small utilities
@@ -38,6 +42,28 @@ template <> struct ActT<bf16> {
   static __device__ __forceinline__ float to_f(bf16 v) { return __bfloat162float(v); }
   static __device__ __forceinline__ bf16 from_f(float v) { return __float2bfloat16_rn(v); }
 };
+template <> struct ActT<f16> {
+  static __device__ __forceinline__ float to_f(f16 v) { return __half2float(v); }
+  static __device__ __forceinline__ f16 from_f(float v) { return __float2half_rn(v); }
+};
+
+// Two fp32 values rounded to nearest-even into one 32-bit pair of a 2-byte type (low half = a), and back.
+template <typename AT> __device__ __forceinline__ uint32_t pack2_rn(float a, float b);
+template <> __device__ __forceinline__ uint32_t pack2_rn<bf16>(float a, float b) {
+  __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
+  return *reinterpret_cast<uint32_t*>(&h);
+}
+template <> __device__ __forceinline__ uint32_t pack2_rn<f16>(float a, float b) {
+  __half2 h = __floats2half2_rn(a, b);
+  return *reinterpret_cast<uint32_t*>(&h);
+}
+template <typename AT> __device__ __forceinline__ float2 unpack2(uint32_t u);
+template <> __device__ __forceinline__ float2 unpack2<bf16>(uint32_t u) {
+  return __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&u));
+}
+template <> __device__ __forceinline__ float2 unpack2<f16>(uint32_t u) {
+  return __half22float2(*reinterpret_cast<const __half2*>(&u));
+}
 
 // 8 consecutive activations -> fp32 (16-byte load for bf16, 2x16 for fp32). p must be 16B aligned.
 __device__ __forceinline__ void load8(const bf16* p, float (&o)[8]) {
@@ -46,6 +72,16 @@ __device__ __forceinline__ void load8(const bf16* p, float (&o)[8]) {
 #pragma unroll
   for (int i = 0; i < 4; ++i) {
     float2 f = __bfloat1622float2(h[i]);
+    o[2 * i] = f.x;
+    o[2 * i + 1] = f.y;
+  }
+}
+__device__ __forceinline__ void load8(const f16* p, float (&o)[8]) {
+  uint4 u = *reinterpret_cast<const uint4*>(p);
+  const uint32_t w[4] = {u.x, u.y, u.z, u.w};
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const float2 f = unpack2<f16>(w[i]);
     o[2 * i] = f.x;
     o[2 * i + 1] = f.y;
   }
@@ -69,6 +105,18 @@ __device__ __forceinline__ void load8_stream(const bf16* p, float (&o)[8]) {
     o[2 * i + 1] = f.y;
   }
 }
+__device__ __forceinline__ void load8_stream(const f16* p, float (&o)[8]) {
+  uint4 u;
+  asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0,%1,%2,%3}, [%4];"
+               : "=r"(u.x), "=r"(u.y), "=r"(u.z), "=r"(u.w) : "l"(p));
+  const uint32_t w[4] = {u.x, u.y, u.z, u.w};
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const float2 f = unpack2<f16>(w[i]);
+    o[2 * i] = f.x;
+    o[2 * i + 1] = f.y;
+  }
+}
 __device__ __forceinline__ void load8_stream(const float* p, float (&o)[8]) { load8(p, o); }
 
 __device__ __forceinline__ void store8(bf16* p, const float (&v)[8]) {
@@ -77,6 +125,10 @@ __device__ __forceinline__ void store8(bf16* p, const float (&v)[8]) {
 #pragma unroll
   for (int i = 0; i < 4; ++i) h[i] = __floats2bfloat162_rn(v[2 * i], v[2 * i + 1]);
   *reinterpret_cast<uint4*>(p) = u;
+}
+__device__ __forceinline__ void store8(f16* p, const float (&v)[8]) {
+  *reinterpret_cast<uint4*>(p) = make_uint4(pack2_rn<f16>(v[0], v[1]), pack2_rn<f16>(v[2], v[3]), pack2_rn<f16>(v[4], v[5]),
+                                            pack2_rn<f16>(v[6], v[7]));
 }
 __device__ __forceinline__ void store8(float* p, const float (&v)[8]) {
   *reinterpret_cast<float4*>(p) = make_float4(v[0], v[1], v[2], v[3]);
@@ -115,6 +167,18 @@ __host__ __device__ constexpr uint32_t umma_idesc_bf16(int M, int N) {
          | (1u << 10)                            // b_format = BF16
          | (static_cast<uint32_t>(N >> 3) << 17) // n_dim
          | (static_cast<uint32_t>(M >> 4) << 24);// m_dim
+}
+// The same with IEEE fp16 A/B: a_format = b_format = F16 (0) under kind::f16.
+__host__ __device__ constexpr uint32_t umma_idesc_f16(int M, int N) {
+  return (1u << 4)                               // c_format = F32
+         | (static_cast<uint32_t>(N >> 3) << 17) // n_dim
+         | (static_cast<uint32_t>(M >> 4) << 24);// m_dim
+}
+// The descriptor for operands of the 2-byte type AT (bf16 | f16)
+template <typename AT>
+__host__ __device__ constexpr uint32_t umma_idesc(int M, int N) {
+  static_assert(std::is_same<AT, bf16>::value || std::is_same<AT, f16>::value, "kind::f16 takes bf16 or fp16 operands");
+  return std::is_same<AT, bf16>::value ? umma_idesc_bf16(M, N) : umma_idesc_f16(M, N);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -314,7 +378,7 @@ __device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 
-// D[tmem] (+)= A[smem] * B[smem]^T, bf16 x bf16 -> fp32; issued by ONE thread
+// D[tmem] (+)= A[smem] * B[smem]^T, bf16 x bf16 (or fp16 x fp16, as the descriptor says) -> fp32; issued by ONE thread
 __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
                                           uint32_t accumulate) {
   asm volatile(

@@ -55,15 +55,15 @@ struct PairMaps {
 struct Weight {          // a GEMM weight [N, K] in the precision's storage type
   void* ptr = nullptr;
   int N = 0, K = 0;
-  CUtensorMap map;       // bf16 only: [N, K], box {64, 64}, SWIZZLE_128B (single-CTA kernel)
-  PairMaps mapp;         // bf16 only: box {64, BN/2} per pair-tile width BN (CTA-pair kernel: one load per stage per CTA)
+  CUtensorMap map;       // 2-byte engines only: [N, K], box {64, 64}, SWIZZLE_128B (single-CTA kernel)
+  PairMaps mapp;         // 2-byte engines only: box {64, BN/2} per pair-tile width BN (CTA-pair kernel: one load per stage per CTA)
   int map_idx = -1;      // index of mapp.m[0] in the ctx's device tensor-map table (chain kernel)
 };
 struct ABuf {            // a GEMM A operand buffer [rows_pad, K]
   void* ptr = nullptr;
   int rows = 0, K = 0;
-  CUtensorMap map;       // bf16 only: box {64, 128}
-  CUtensorMap map3;      // bf16 only, K >= 128: 3-D box {64, 128, 2} over the [K/64][rows][64] view (pair kernel, KS = 2)
+  CUtensorMap map;       // 2-byte engines only: box {64, 128}
+  CUtensorMap map3;      // 2-byte engines only, K >= 128: 3-D box {64, 128, 2} over the [K/64][rows][64] view (pair kernel, KS = 2)
   bool have3 = false;
   int map_idx = -1;      // index in the ctx's device tensor-map table (chain kernel)
 };
@@ -73,7 +73,7 @@ struct BlockW {
 };
 struct ParamSlot {
   void* dst = nullptr;
-  int dst_is_weight = 0;   // 1: stored in the GEMM storage type (bf16 | fp32); 0: fp32
+  int dst_is_weight = 0;   // 1: stored in the GEMM storage type (bf16 | fp16 | fp32); 0: fp32
   std::vector<int64_t> shape;
   bool loaded = false;
   bool ignored = false;    // accepted for strict loading, never read by the sampler
@@ -149,7 +149,10 @@ struct GraphKey {
 struct hq_ctx {
   hq_config cfg;
   int device = 0, max_batch = 0;
-  bool bf16 = true;
+  // The 2-byte tensor-core engine (HQ_PREC_BF16 / HQ_PREC_F16): tcgen05 GEMMs, split-K, the mma.sync decode attention,
+  // the fused head sampler; false: the fp32 CUDA-core engine.  `prec` names the element type.
+  bool half = true;
+  int prec = HQ_PREC_BF16;
   int D = 0, nh = 0, L = 0, Ld = 0, Vt = 0, Vb = 0, Vmax = 0, T0 = 1, Tc = 0, Smax = 0;
   size_t wsize = 2;  // bytes per GEMM weight / activation element
   std::string err;
@@ -184,7 +187,7 @@ struct hq_ctx {
   float2* samp_part = nullptr;     // fused head + sampler: [depth_rows * B, Vmax / 32] (log-sum-exp, drawn index) per 32-column chunk
   float* splitk_ws = nullptr;   // [LN_MAXFOLD][rows][D] fp32 partial sums of split-K fc2 GEMMs (folded in by the next LayerNorm)
   unsigned int* att_sched = nullptr;   // [2] work-ticket / finished-CTA counters of attention_decode_mma_kernel (rest at 0)
-  CUtensorMap kmap, vmap;              // spatial KV cache as [rows = L*B*Tc][heads][64] bf16, box {64, hpc, 8}, SWIZZLE_128B
+  CUtensorMap kmap, vmap;              // spatial KV cache as [rows = L*B*Tc][heads][64] 2-byte, box {64, hpc, 8}, SWIZZLE_128B
   bool kv_maps = false;
   int num_sms = 0;
   int ws_rows = 0;
@@ -256,12 +259,17 @@ static int dev_alloc(hq_ctx* ctx, void** p, size_t bytes) {
   return HQ_OK;
 }
 
+// Element type of the tensor maps of a 2-byte engine (TMA moves the same bytes either way; the map names what the kernels read)
+static CUtensorMapDataType tmap_dtype(const hq_ctx* ctx) {
+  return ctx->prec == HQ_PREC_F16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+}
+
 static int make_map(hq_ctx* ctx, CUtensorMap* m, void* base, uint64_t rows, uint64_t cols, uint32_t box_rows) {
   cuuint64_t dims[2] = {cols, rows};
   cuuint64_t strides[1] = {cols * 2};
   cuuint32_t box[2] = {64, box_rows};
   cuuint32_t estr[2] = {1, 1};
-  CUresult r = ctx->encode(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, base, dims, strides, box, estr,
+  CUresult r = ctx->encode(m, tmap_dtype(ctx), 2, base, dims, strides, box, estr,
                            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
@@ -272,14 +280,14 @@ static int make_map(hq_ctx* ctx, CUtensorMap* m, void* base, uint64_t rows, uint
   return HQ_OK;
 }
 
-// [rows, cols] bf16 viewed as [cols / 64][rows][64]: one box {64, box_rows, ks} stages ks consecutive 64-wide k-blocks of
-// box_rows rows as ks consecutive SWIZZLE_128B tiles (what the UMMA descriptors of ks k-blocks expect)
+// [rows, cols] 2-byte elements viewed as [cols / 64][rows][64]: one box {64, box_rows, ks} stages ks consecutive 64-wide
+// k-blocks of box_rows rows as ks consecutive SWIZZLE_128B tiles (what the UMMA descriptors of ks k-blocks expect)
 static int make_map3(hq_ctx* ctx, CUtensorMap* m, void* base, uint64_t rows, uint64_t cols, uint32_t box_rows, uint32_t ks) {
   cuuint64_t dims[3] = {64, rows, cols / 64};
   cuuint64_t strides[2] = {cols * 2, 128};
   cuuint32_t box[3] = {64, box_rows, ks};
   cuuint32_t estr[3] = {1, 1, 1};
-  CUresult r = ctx->encode(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, base, dims, strides, box, estr,
+  CUresult r = ctx->encode(m, tmap_dtype(ctx), 3, base, dims, strides, box, estr,
                            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
@@ -308,7 +316,7 @@ static int make_kv_map(hq_ctx* ctx, CUtensorMap* m, const void* base, int n_head
   cuuint64_t strides[2] = {128, static_cast<cuuint64_t>(n_heads) * 128};
   cuuint32_t box[3] = {64, static_cast<cuuint32_t>(hpc), 8};
   cuuint32_t estr[3] = {1, 1, 1};
-  CUresult r = ctx->encode(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(base), dims, strides, box, estr,
+  CUresult r = ctx->encode(m, tmap_dtype(ctx), 3, const_cast<void*>(base), dims, strides, box, estr,
                            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
@@ -324,7 +332,7 @@ static int alloc_weight(hq_ctx* ctx, Weight* w, int N, int K) {
   w->K = K;
   int rc = dev_alloc(ctx, &w->ptr, static_cast<size_t>(N) * K * ctx->wsize);
   if (rc) return rc;
-  if (ctx->bf16) {
+  if (ctx->half) {
     if ((rc = make_map(ctx, &w->map, w->ptr, N, K, 64))) return rc;
     return make_pair_maps(ctx, &w->mapp, w->ptr, N, K);
   }
@@ -335,7 +343,7 @@ static int alloc_abuf(hq_ctx* ctx, ABuf* a, int rows, int K) {
   a->K = K;
   int rc = dev_alloc(ctx, &a->ptr, static_cast<size_t>(a->rows) * K * ctx->wsize);
   if (rc) return rc;
-  if (ctx->bf16) {
+  if (ctx->half) {
     if ((rc = make_map(ctx, &a->map, a->ptr, a->rows, K, 128))) return rc;
     a->have3 = K >= 128;
     if (a->have3) return make_map3(ctx, &a->map3, a->ptr, a->rows, K, 128, 2);
@@ -396,22 +404,34 @@ static int set_smem(hq_ctx* ctx, K kernel, int bytes) {
   return HQ_OK;
 }
 
+template <typename AT>
 static int set_gemm_attrs(hq_ctx* ctx) {
   int rc;
 #define HQ_SET(BN, EPI) \
-  if ((rc = set_smem(ctx, gemm_tc_kernel<BN, EPI, bf16, 1>, TcCfg<BN, 1>::SMEM_BYTES))) return rc; \
-  if ((rc = set_smem(ctx, gemm_tc_kernel<BN, EPI, bf16, 2>, TcCfg<BN, 2>::SMEM_BYTES))) return rc;
+  if ((rc = set_smem(ctx, gemm_tc_kernel<BN, EPI, AT, 1>, TcCfg<BN, 1>::SMEM_BYTES))) return rc; \
+  if ((rc = set_smem(ctx, gemm_tc_kernel<BN, EPI, AT, 2>, TcCfg<BN, 2>::SMEM_BYTES))) return rc;
   HQ_SET(64, EPI_QKV) HQ_SET(64, EPI_RESID) HQ_SET(64, EPI_GELU) HQ_SET(64, EPI_F32) HQ_SET(64, EPI_SAMPLE)
   HQ_SET(128, EPI_QKV) HQ_SET(128, EPI_RESID) HQ_SET(128, EPI_GELU) HQ_SET(128, EPI_F32) HQ_SET(128, EPI_SAMPLE)
 #undef HQ_SET
 #define HQ_SET2(BN, EPI) \
-  if ((rc = set_smem(ctx, gemm_tc2_kernel<BN, EPI, bf16, 1>, Tc2Cfg<BN, 1>::SMEM_BYTES))) return rc; \
-  if ((rc = set_smem(ctx, gemm_tc2_kernel<BN, EPI, bf16, 2>, Tc2Cfg<BN, 2>::SMEM_BYTES))) return rc;
+  if ((rc = set_smem(ctx, gemm_tc2_kernel<BN, EPI, AT, 1>, Tc2Cfg<BN, 1>::SMEM_BYTES))) return rc; \
+  if ((rc = set_smem(ctx, gemm_tc2_kernel<BN, EPI, AT, 2>, Tc2Cfg<BN, 2>::SMEM_BYTES))) return rc;
 #define HQ_SET2_ALL(BN) HQ_SET2(BN, EPI_QKV) HQ_SET2(BN, EPI_RESID) HQ_SET2(BN, EPI_GELU) HQ_SET2(BN, EPI_F32) HQ_SET2(BN, EPI_SAMPLE)
   HQ_SET2_ALL(32) HQ_SET2_ALL(64) HQ_SET2_ALL(96) HQ_SET2_ALL(128) HQ_SET2_ALL(192) HQ_SET2_ALL(256)
 #undef HQ_SET2_ALL
 #undef HQ_SET2
   return HQ_OK;
+}
+static int set_gemm_attrs_for(hq_ctx* ctx) {
+  return ctx->prec == HQ_PREC_F16 ? set_gemm_attrs<f16>(ctx) : set_gemm_attrs<bf16>(ctx);
+}
+
+// Calls f(AT()) with the activation type of precision `prec`: bf16, f16 (HQ_PREC_F16) or float (HQ_PREC_FP32).
+template <typename F>
+static void with_act(int prec, F&& f) {
+  if (prec == HQ_PREC_BF16) f(bf16());
+  else if (prec == HQ_PREC_F16) f(f16());
+  else f(float());
 }
 
 static int get_encode_fn(hq_ctx* ctx, PFN_encodeTiled* fn) {
@@ -445,6 +465,15 @@ static int check_device(hq_ctx* ctx, int device) {
 
 static void free_activations(hq_ctx* ctx);
 static int reserve_impl(hq_ctx* ctx, int max_batch);
+
+static int set_attn_attrs(hq_ctx* ctx) {
+  int rc;
+  if ((rc = set_smem(ctx, attention_decode_kernel<bf16>, 64 * 1024))) return rc;
+  if ((rc = set_smem(ctx, attention_decode_kernel<f16>, 64 * 1024))) return rc;
+  if ((rc = set_smem(ctx, attention_decode_kernel<float>, 64 * 1024))) return rc;
+  if ((rc = set_smem(ctx, attention_decode_mma_kernel<bf16>, 112 * 1024))) return rc;
+  return set_smem(ctx, attention_decode_mma_kernel<f16>, 112 * 1024);
+}
 
 // Head groups per image of the decode attention kernels: (image, group) work items, nh / groups heads (warps) each.
 static int attn_groups(const hq_ctx* ctx, int nh) {
@@ -541,12 +570,12 @@ static int reserve_alloc(hq_ctx* ctx, int max_batch) {
     ctx->samp_part = reinterpret_cast<float2*>(sp2);
   }
   ctx->ws_rows = Mmax;
-  if (ctx->bf16 && (rc = alloc_f32(ctx, &ctx->splitk_ws, static_cast<size_t>(LN_MAXFOLD) * Mmax * D))) return rc;
+  if (ctx->half && (rc = alloc_f32(ctx, &ctx->splitk_ws, static_cast<size_t>(LN_MAXFOLD) * Mmax * D))) return rc;
   const size_t kvn = static_cast<size_t>(ctx->L) * B * ctx->Tc * D * ctx->wsize;
   if ((rc = dev_alloc(ctx, &ctx->kc, kvn))) return rc;
   if ((rc = dev_alloc(ctx, &ctx->vc, kvn))) return rc;
   ctx->kv_maps = false;
-  if (ctx->bf16) {
+  if (ctx->half) {
     const int groups = attn_groups(ctx, ctx->nh);
     if (groups > 0) {
       const uint64_t rows = static_cast<uint64_t>(ctx->L) * B * ctx->Tc;
@@ -566,8 +595,8 @@ static int reserve_alloc(hq_ctx* ctx, int max_batch) {
       (rc = dev_alloc(ctx, reinterpret_cast<void**>(&ctx->codes_mid), static_cast<size_t>(B) * ctx->Smax * 32))) return rc;
   if ((rc = alloc_f32(ctx, &ctx->sos_override, static_cast<size_t>(Mx) * D))) return rc;
   if ((rc = dev_alloc(ctx, reinterpret_cast<void**>(&ctx->d_sp), sizeof(hq_sampling_params)))) return rc;
-  if (ctx->bf16) {
-    // tensor-map table of the chain kernel: the three A buffers, then the six pair-tile maps of every GEMM weight
+  if (ctx->prec == HQ_PREC_BF16) {
+    // tensor-map table of the chain kernel (bf16 only): the three A buffers, then the six pair-tile maps of every GEMM weight
     std::vector<CUtensorMap> table;
     ABuf* abufs[3] = {&ctx->h, &ctx->att, &ctx->mlp};
     for (ABuf* a : abufs) {
@@ -596,9 +625,10 @@ static int create_impl(hq_ctx* ctx, const hq_config* cfg, int device, int max_ba
   ctx->cfg = *cfg;
   ctx->device = device;
   ctx->max_batch = max_batch;
-  ctx->bf16 = cfg->precision == HQ_PREC_BF16;
+  ctx->prec = cfg->precision;
+  ctx->half = cfg->precision != HQ_PREC_FP32;
   ctx->use_pdl = cfg->use_pdl != 0;
-  ctx->wsize = ctx->bf16 ? 2 : 4;
+  ctx->wsize = ctx->half ? 2 : 4;
   const int D = ctx->D = cfg->embed_dim;
   ctx->nh = cfg->n_heads;
   ctx->L = cfg->n_layers;
@@ -639,7 +669,7 @@ static int create_impl(hq_ctx* ctx, const hq_config* cfg, int device, int max_ba
             cfg->ctx_len_img, cfg->ctx_len_txt, ctx->Tc, ATT_MAX_KEYS);
     return HQ_ERR_UNSUPPORTED;
   }
-  if (cfg->cond_kind < 0 || cfg->cond_kind > 2 || cfg->precision < 0 || cfg->precision > 1) {
+  if (cfg->cond_kind < 0 || cfg->cond_kind > 2 || cfg->precision < HQ_PREC_BF16 || cfg->precision > HQ_PREC_F16) {
     set_err(ctx, "bad cond_kind / precision");
     return HQ_ERR_INVALID;
   }
@@ -658,20 +688,19 @@ static int create_impl(hq_ctx* ctx, const hq_config* cfg, int device, int max_ba
     while ((H + 1) * (H + 1) <= cfg->ctx_len_img) ++H;        // int(math.sqrt(ctx_len_img)), hierarchical_ar.py:122
     ctx->Hpos = H;
   }
-  if (ctx->bf16) {
+  if (ctx->half) {
     if ((rc = get_encode_fn(ctx, &ctx->encode))) return rc;
-    if ((rc = set_gemm_attrs(ctx))) return rc;
+    if ((rc = set_gemm_attrs_for(ctx))) return rc;
   }
-  if ((rc = set_smem(ctx, attention_decode_kernel<bf16>, 64 * 1024))) return rc;
-  if ((rc = set_smem(ctx, attention_decode_kernel<float>, 64 * 1024))) return rc;
-  if ((rc = set_smem(ctx, attention_decode_mma_kernel, 112 * 1024))) return rc;
+  if ((rc = set_attn_attrs(ctx))) return rc;
   if ((rc = dev_alloc(ctx, reinterpret_cast<void**>(&ctx->att_sched), 16))) return rc;
   HQ_CUDA(ctx, cudaMemset(ctx->att_sched, 0, 16));
   HQ_CUDA(ctx, cudaDeviceGetAttribute(&ctx->num_sms, cudaDevAttrMultiProcessorCount, device));
   HQ_CUDA(ctx, cudaStreamCreateWithFlags(&ctx->own_stream, cudaStreamNonBlocking));
-  if (ctx->bf16 && cfg->use_chain && !ctx->dbg.no_chain) {
-    // persistent chain kernel: every launch uses the same grid of co-resident CTA pairs (its ops are separated by a
-    // grid barrier, so a CTA that is not resident would deadlock the rest)
+  if (ctx->prec == HQ_PREC_BF16 && cfg->use_chain && !ctx->dbg.no_chain) {
+    // persistent chain kernel (bf16 engine only; the fp16 and fp32 engines ignore use_chain): every launch uses the same
+    // grid of co-resident CTA pairs (its ops are separated by a grid barrier, so a CTA that is not resident would deadlock
+    // the rest)
     if ((rc = set_smem(ctx, chain_kernel, CH_SMEM_BYTES))) return rc;
     cudaLaunchConfig_t lc;
     memset(&lc, 0, sizeof(lc));
@@ -805,16 +834,18 @@ __global__ void convert_kernel(const S* __restrict__ s, Dt* __restrict__ d, size
     if (sizeof(S) == 4) v = *reinterpret_cast<const float*>(&s[i]);
     else if (std::is_same<S, bf16>::value) v = __bfloat162float(*reinterpret_cast<const bf16*>(&s[i]));
     else v = __half2float(*reinterpret_cast<const __half*>(&s[i]));
-    if (sizeof(Dt) == 4) *reinterpret_cast<float*>(&d[i]) = v;
-    else *reinterpret_cast<bf16*>(&d[i]) = __float2bfloat16_rn(v);
+    d[i] = ActT<Dt>::from_f(v);
   }
 }
 
+// dst_prec: the storage type of the destination (HQ_PREC_BF16 | HQ_PREC_F16 | HQ_PREC_FP32)
 template <typename S>
-static void launch_convert(const void* src, void* dst, bool dst_bf16, size_t n) {
+static void launch_convert(const void* src, void* dst, int dst_prec, size_t n) {
   const int grid = static_cast<int>((n + 255) / 256 > 4096 ? 4096 : (n + 255) / 256);
-  if (dst_bf16) convert_kernel<S, bf16><<<grid, 256>>>(static_cast<const S*>(src), static_cast<bf16*>(dst), n);
-  else convert_kernel<S, float><<<grid, 256>>>(static_cast<const S*>(src), static_cast<float*>(dst), n);
+  with_act(dst_prec, [&](auto tag) {
+    using Dt = decltype(tag);
+    convert_kernel<S, Dt><<<grid, 256>>>(static_cast<const S*>(src), static_cast<Dt*>(dst), n);
+  });
 }
 
 extern "C" int hq_load_param(hq_ctx* ctx, const char* name, const void* data, int dtype, const int64_t* shape, int ndim,
@@ -860,10 +891,10 @@ extern "C" int hq_load_param(hq_ctx* ctx, const char* name, const void* data, in
     }
     src = staged;
   }
-  const bool dst_bf16 = s.dst_is_weight && ctx->bf16;
-  if (dtype == HQ_F32) launch_convert<float>(src, s.dst, dst_bf16, n);
-  else if (dtype == HQ_BF16) launch_convert<bf16>(src, s.dst, dst_bf16, n);
-  else launch_convert<__half>(src, s.dst, dst_bf16, n);
+  const int dst_prec = s.dst_is_weight ? ctx->prec : HQ_PREC_FP32;
+  if (dtype == HQ_F32) launch_convert<float>(src, s.dst, dst_prec, n);
+  else if (dtype == HQ_BF16) launch_convert<bf16>(src, s.dst, dst_prec, n);
+  else launch_convert<__half>(src, s.dst, dst_prec, n);
   cudaError_t e = cudaDeviceSynchronize();
   if (staged) cudaFree(staged);
   if (e != cudaSuccess) {
@@ -1075,16 +1106,17 @@ static int pick_pair_bn(int M, int N, int K) {
   return best;
 }
 
-template <int EPI>
-static void gemm_bf16(hq_ctx* ctx, cudaStream_t st, const CUtensorMap& mA, const CUtensorMap* mA3, const CUtensorMap& mW64,
-                      const PairMaps& mWp, int w_row_off, int M, int N, int K, const EpiParams<bf16>& ep,
-                      int splits = 1, int bn_hint = 0, int ia = -1, int iw = -1) {
+// The tcgen05 GEMM of the 2-byte engines (AT = bf16 | f16) on the operands' tensor maps.
+template <int EPI, typename AT>
+static void gemm_tc(hq_ctx* ctx, cudaStream_t st, const CUtensorMap& mA, const CUtensorMap* mA3, const CUtensorMap& mW64,
+                    const PairMaps& mWp, int w_row_off, int M, int N, int K, const EpiParams<AT>& ep,
+                    int splits = 1, int bn_hint = 0, int ia = -1, int iw = -1) {
   int bn = ctx->dbg.force_bn ? ctx->dbg.force_bn : bn_hint;
   if (bn == 0) bn = (M > 128) ? pick_pair_bn(M, N, K) : 0;
   if (bn_hint == 0 && !ctx->dbg.force_bn && ctx->dbg.bn_m256 > 0 && M > 128 && M <= 256 && N % ctx->dbg.bn_m256 == 0) bn = ctx->dbg.bn_m256;
   if (ctx->recording) {
-    // an op of the persistent chain kernel: CTA-pair tiles only (chain_enabled guarantees M > 128)
-    if (bn <= 0 || N % bn != 0 || ia < 0 || iw < 0 || (K / 64) % splits != 0) {
+    // an op of the persistent chain kernel (bf16): CTA-pair tiles only (chain_enabled guarantees M > 128)
+    if (!std::is_same<AT, bf16>::value || bn <= 0 || N % bn != 0 || ia < 0 || iw < 0 || (K / 64) % splits != 0) {
       if (ctx->launch_err == cudaSuccess) ctx->launch_err = cudaErrorInvalidValue;
       return;
     }
@@ -1097,7 +1129,7 @@ static void gemm_bf16(hq_ctx* ctx, cudaStream_t st, const CUtensorMap& mA, const
     op->map_a = ia;
     op->map_w = iw + PairMaps::index(bn);
     op->M = M; op->N = N; op->K = K; op->bn = bn; op->splits = splits; op->epi = EPI; op->w_row_off = w_row_off;
-    op->ep = ep;
+    if constexpr (std::is_same<AT, bf16>::value) op->ep = ep;   // the chain kernel is bf16 only (refused above otherwise)
     if (op->flags & CH_F_T0_RT) op->ep.t0 = 0;
     return;
   }
@@ -1116,10 +1148,10 @@ static void gemm_bf16(hq_ctx* ctx, cudaStream_t st, const CUtensorMap& mA, const
 #define HQ_LAUNCH2(BN)                                                                                             \
   case BN:                                                                                                         \
     if (ks2)                                                                                                       \
-      launch_k(ctx, st, tag, gemm_tc2_kernel<BN, EPI, bf16, 2>, grid, dim3(Tc2Cfg<BN, 2>::THREADS), Tc2Cfg<BN, 2>::SMEM_BYTES, *mA3,  \
+      launch_k(ctx, st, tag, gemm_tc2_kernel<BN, EPI, AT, 2>, grid, dim3(Tc2Cfg<BN, 2>::THREADS), Tc2Cfg<BN, 2>::SMEM_BYTES, *mA3,  \
                mWp.m3[PairMaps::index(BN)], M, N, K, w_row_off, splits, ep);                                       \
     else                                                                                                           \
-      launch_k(ctx, st, tag, gemm_tc2_kernel<BN, EPI, bf16, 1>, grid, dim3(Tc2Cfg<BN, 1>::THREADS), Tc2Cfg<BN, 1>::SMEM_BYTES, mA,  \
+      launch_k(ctx, st, tag, gemm_tc2_kernel<BN, EPI, AT, 1>, grid, dim3(Tc2Cfg<BN, 1>::THREADS), Tc2Cfg<BN, 1>::SMEM_BYTES, mA,  \
                mWp.m[PairMaps::index(BN)], M, N, K, w_row_off, splits, ep);                                        \
     break;
     switch (bn) {
@@ -1137,17 +1169,17 @@ static void gemm_bf16(hq_ctx* ctx, cudaStream_t st, const CUtensorMap& mA, const
   dim3 grid(N / tbn, mt, splits);
   if (wide) {
     if (ks2)
-      launch_k(ctx, st, tag, gemm_tc_kernel<128, EPI, bf16, 2>, grid, dim3(192), TcCfg<128, 2>::SMEM_BYTES, *mA3,
+      launch_k(ctx, st, tag, gemm_tc_kernel<128, EPI, AT, 2>, grid, dim3(192), TcCfg<128, 2>::SMEM_BYTES, *mA3,
                mWp.m3[PairMaps::index(256)], M, N, K, w_row_off, ep);
     else
-      launch_k(ctx, st, tag, gemm_tc_kernel<128, EPI, bf16, 1>, grid, dim3(192), TcCfg<128, 1>::SMEM_BYTES, mA, mW64, M, N, K,
+      launch_k(ctx, st, tag, gemm_tc_kernel<128, EPI, AT, 1>, grid, dim3(192), TcCfg<128, 1>::SMEM_BYTES, mA, mW64, M, N, K,
                w_row_off, ep);
   } else {
     if (ks2)
-      launch_k(ctx, st, tag, gemm_tc_kernel<64, EPI, bf16, 2>, grid, dim3(192), TcCfg<64, 2>::SMEM_BYTES, *mA3,
+      launch_k(ctx, st, tag, gemm_tc_kernel<64, EPI, AT, 2>, grid, dim3(192), TcCfg<64, 2>::SMEM_BYTES, *mA3,
                mWp.m3[PairMaps::index(128)], M, N, K, w_row_off, ep);
     else
-      launch_k(ctx, st, tag, gemm_tc_kernel<64, EPI, bf16, 1>, grid, dim3(192), TcCfg<64, 1>::SMEM_BYTES, mA, mW64, M, N, K,
+      launch_k(ctx, st, tag, gemm_tc_kernel<64, EPI, AT, 1>, grid, dim3(192), TcCfg<64, 1>::SMEM_BYTES, mA, mW64, M, N, K,
                w_row_off, ep);
   }
 }
@@ -1159,10 +1191,10 @@ static void gemm_f32(hq_ctx* ctx, cudaStream_t st, const float* A, const float* 
   launch_k(ctx, st, gemm_tag<EPI>(M), gemm_simt_kernel<EPI>, grid, dim3(256), 0, A, W, M, N, K, ep);
 }
 
-template <int EPI>
+template <int EPI, typename AT>
 static void gemm_any(hq_ctx* ctx, cudaStream_t st, const ABuf& A, const Weight& W, int w_row_off, int M, int N, int K,
-                     const EpiParams<bf16>& ep) {
-  gemm_bf16<EPI>(ctx, st, A.map, A.have3 ? &A.map3 : nullptr, W.map, W.mapp, w_row_off, M, N, K, ep, 1, 0, A.map_idx, W.map_idx);
+                     const EpiParams<AT>& ep) {
+  gemm_tc<EPI, AT>(ctx, st, A.map, A.have3 ? &A.map3 : nullptr, W.map, W.mapp, w_row_off, M, N, K, ep, 1, 0, A.map_idx, W.map_idx);
 }
 template <int EPI>
 static void gemm_any(hq_ctx* ctx, cudaStream_t st, const ABuf& A, const Weight& W, int w_row_off, int M, int N, int K,
@@ -1233,11 +1265,11 @@ static bool attn_decode_plan(const hq_ctx* ctx, int* CH, int* hpc, int* groups, 
   return *smem <= 64 * 1024;
 }
 
-// Launch plan of attention_decode_mma_kernel (bf16): ring stages of one 8-key K tile + one 8-value V tile (hpc KB each);
+// Launch plan of attention_decode_mma_kernel (2-byte engines): ring stages of one 8-key K tile + one 8-value V tile (hpc KB each);
 // grid = resident CTAs (registers allow four 7-warp CTAs per SM; each takes one item, then tickets), capped by the
 // number of items.
 static bool attn_mma_plan(const hq_ctx* ctx, int groups, int hpc, int n_items, int* stages, size_t* smem, int* grid) {
-  if (ctx->dbg.attn_scalar || !ctx->bf16 || ctx->num_sms <= 0 || !ctx->kv_maps) return false;
+  if (ctx->dbg.attn_scalar || !ctx->half || ctx->num_sms <= 0 || !ctx->kv_maps) return false;
   const size_t stage = static_cast<size_t>(2 * ATTM_CH) * hpc * 128;     // K tile + V tile
   // Two stages (24 KB for 6 heads): measured equal end to end to a 4-deep ring and ~1 us faster per launch in the loop
   // (profiles/r1_attn_sweep.txt) - requests beyond the bandwidth-delay product only lengthen every request's latency,
@@ -1265,23 +1297,23 @@ static bool attn_mma_plan(const hq_ctx* ctx, int groups, int hpc, int n_items, i
 }
 
 template <typename AT>
-static void launch_attn_mma(hq_ctx*, cudaStream_t, const AT*, const AT*, AT*, int, int, int, int, int, int, int, size_t) {}
-template <>
-void launch_attn_mma<bf16>(hq_ctx* ctx, cudaStream_t st, const bf16* q, const bf16* K, bf16* out, int t_stride, int n_keys,
-                           int hpc, int groups, int n_items, int stages, int grid, size_t smem) {
+static void launch_attn_mma(hq_ctx* ctx, cudaStream_t st, const AT* q, const AT* K, AT* out, int t_stride, int n_keys,
+                            int hpc, int groups, int n_items, int stages, int grid, size_t smem) {
   // K (and V, at the same offset in its own cache) as a row offset into the cache-wide tensor maps
-  const int row_base = static_cast<int>((K - static_cast<const bf16*>(ctx->kc)) / ctx->D);
-  launch_k(ctx, st, "attention_decode", attention_decode_mma_kernel, dim3(grid), dim3((hpc + 1) * 32), smem, ctx->kmap, ctx->vmap,
+  const int row_base = static_cast<int>((K - static_cast<const AT*>(ctx->kc)) / ctx->D);
+  launch_k(ctx, st, "attention_decode", attention_decode_mma_kernel<AT>, dim3(grid), dim3((hpc + 1) * 32), smem, ctx->kmap, ctx->vmap,
            row_base, q, out, ctx->D, t_stride, n_keys, hpc, groups, n_items, attn_prefetch_ok(ctx) ? stages : -stages,
            ctx->att_sched);
 }
+template <>
+void launch_attn_mma<float>(hq_ctx*, cudaStream_t, const float*, const float*, float*, int, int, int, int, int, int, int, size_t) {}
 
 template <typename AT>
 static void attention(hq_ctx* ctx, cudaStream_t st, const AT* q, const AT* K, const AT* V, AT* out, int M, int Tq,
                       int t_stride, int kbase, int causal) {
   int CH = 0, hpc = 0, groups = 0;
   size_t smem = 0;
-  if (ctx->recording && sizeof(AT) == 2 && !causal && kbase <= ATT_DEPTH_KEYS && Tq == 4) {
+  if (ctx->recording && std::is_same<AT, bf16>::value && !causal && kbase <= ATT_DEPTH_KEYS && Tq == 4) {
     ChainOp* op = chain_push(ctx, CH_OP_ATTN4, "attention_depth4");
     op->q = reinterpret_cast<const bf16*>(q); op->kc = reinterpret_cast<const bf16*>(K);
     op->vc = reinterpret_cast<const bf16*>(V); op->att = reinterpret_cast<bf16*>(out);
@@ -1337,15 +1369,17 @@ static void launch_sample(hq_ctx* ctx, cudaStream_t st, const SampleArgs& a) {
 //   mode 0: spatial decode / prefill  - q, k, v; attention over the spatial cache
 //   mode 1: depth pass 0              - k, v only (softmax over one key == identity, a = v)
 //   mode 2: depth pass 1              - q, k, v; 4 queries over the 5 depth keys
+template <typename AT>
 static void gemm_fc2_split(hq_ctx* ctx, cudaStream_t st, const ABuf& A, const Weight& W, int M, int N, int K, int splits,
-                           int bn, bf16*) {
-  EpiParams<bf16> e;
+                           int bn, AT*) {
+  EpiParams<AT> e;
   memset(&e, 0, sizeof(e));
   e.outf = ctx->splitk_ws; e.ldo = N; e.split_stride = static_cast<size_t>(ctx->ws_rows) * N;
   ctx->gemm_tag_override = "gemm_resid";
-  gemm_bf16<EPI_F32>(ctx, st, A.map, A.have3 ? &A.map3 : nullptr, W.map, W.mapp, 0, M, N, K, e, splits, bn, A.map_idx, W.map_idx);
+  gemm_tc<EPI_F32, AT>(ctx, st, A.map, A.have3 ? &A.map3 : nullptr, W.map, W.mapp, 0, M, N, K, e, splits, bn, A.map_idx, W.map_idx);
 }
-static void gemm_fc2_split(hq_ctx*, cudaStream_t, const ABuf&, const Weight&, int, int, int, int, int, float*) {}
+template <>
+void gemm_fc2_split<float>(hq_ctx*, cudaStream_t, const ABuf&, const Weight&, int, int, int, int, int, float*) {}
 
 // Residual GEMMs (proj [D, D], fc2 [D, 4D]): the narrowest outputs of a block (few CTA pairs) and, for fc2, the longest
 // serial K loop.  The K range is cut in up to LN_MAXFOLD slices; the slices write fp32 partial sums that the next
@@ -1384,7 +1418,7 @@ static int resid_splits(const hq_ctx* ctx, int N, int K, int rows_per_image) {
 // Tile width for this M given the split (bn = 0: the single-CTA kernel, M <= 128, K slices on grid.z).
 static Fc2Plan pick_resid_plan(const hq_ctx* ctx, int M, int N, int K, int rows_per_image) {
   Fc2Plan best{0, 1};
-  if (!ctx->bf16 || N % 64 != 0 || K % 64 != 0 || ctx->dbg.no_splitk) return best;
+  if (!ctx->half || N % 64 != 0 || K % 64 != 0 || ctx->dbg.no_splitk) return best;
   static const int cand[6] = {256, 192, 128, 96, 64, 32};
   const int kb = K / 64;
   int s = resid_splits(ctx, N, K, rows_per_image);
@@ -1465,7 +1499,7 @@ struct RunFlags {
 };
 
 // Head GEMM of the draw described by `sa` (hierarchical_ar.py:695 / 715).  When the draw has no top-k / top-p cut (the
-// measure_throughput protocol) the bf16 engine samples inside the GEMM epilogue (gemm.cuh: EPI_SAMPLE) and the [rows, V]
+// measure_throughput protocol) the 2-byte engines sample inside the GEMM epilogue (gemm.cuh: EPI_SAMPLE) and the [rows, V]
 // logits are never written; otherwise the logits go to ctx->logits for sample_kernel.  Returns whether it fused.
 template <typename AT>
 static bool head_gemm(hq_ctx* ctx, cudaStream_t st, const Weight& w, int rows, int V, const SampleArgs& sa, const RunFlags& f) {
@@ -1537,7 +1571,7 @@ static void run_position(hq_ctx* ctx, cudaStream_t st, int B, int S, int pos, co
   // ---- spatial transformer: L blocks over the KV cache ----
   const int tok = (pos == 0) ? 0 : T0 + pos - 1;     // cache slot of this position's (first) token
   // persistent chain kernel: every run of ops between two cache attentions (and the whole depth transformer) is one launch
-  const bool chain = sizeof(AT) == 2 && !prefill && chain_enabled(ctx, B);
+  const bool chain = std::is_same<AT, bf16>::value && !prefill && chain_enabled(ctx, B);
   if (chain) chain_begin(ctx, tok, pos, S);
   for (int l = 0; l < ctx->L; ++l) {
     if (prefill) run_block<AT>(ctx, st, ctx->blocks[l], ctx->x, M, 0, kc + l * lstride, vc + l * lstride, T0, Tc, 0, 0, 1, &fold_x);
@@ -1700,17 +1734,13 @@ static void run_position3(hq_ctx* ctx, cudaStream_t st, int B, int S, int pos, c
 }
 
 static void run_range(hq_ctx* ctx, cudaStream_t st, int B, int S, int p0, int p1, const RunFlags& f) {
-  if (ctx->levels == 3) {
+  with_act(ctx->prec, [&](auto tag) {
+    using AT = decltype(tag);
     for (int pos = p0; pos < p1; ++pos) {
-      if (ctx->bf16) run_position3<bf16>(ctx, st, B, S, pos, f);
-      else run_position3<float>(ctx, st, B, S, pos, f);
+      if (ctx->levels == 3) run_position3<AT>(ctx, st, B, S, pos, f);
+      else run_position<AT>(ctx, st, B, S, pos, f);
     }
-    return;
-  }
-  for (int pos = p0; pos < p1; ++pos) {
-    if (ctx->bf16) run_position<bf16>(ctx, st, B, S, pos, f);
-    else run_position<float>(ctx, st, B, S, pos, f);
-  }
+  });
 }
 
 static int validate_run(hq_ctx* ctx, const hq_run_args* a) {
@@ -1773,7 +1803,7 @@ static int run_impl(hq_ctx* ctx, const hq_run_args* a, cudaStream_t st, cudaMemc
                     ctx->cfg.model_type != HQ_MODEL_BIDIRECTIONAL;
   f.sos_override = a->sos != nullptr;
   f.fuse_mask = 0;
-  if (ctx->cfg.fuse_head_sampler && ctx->bf16) {
+  if (ctx->cfg.fuse_head_sampler && ctx->half) {
     const hq_sampling_params& q = a->sampling;
     auto none = [](int k, float p2, int V) { return (k <= 0 || k >= V) && !(p2 > 0.f && p2 < 1.f); };
     if (none(q.top_k_top, q.top_p_top, ctx->Vt)) f.fuse_mask |= 1;
@@ -1917,16 +1947,15 @@ extern "C" int hq_debug_attention(int prec, const void* q, const void* K, const 
   HQ_CUDA(nullptr, cudaGetDevice(&dev));
   int rc = check_device(&tmp, dev);
   if (rc) return rc;
-  tmp.bf16 = prec == HQ_PREC_BF16;
+  tmp.prec = (prec == HQ_PREC_BF16 || prec == HQ_PREC_F16) ? prec : HQ_PREC_FP32;
+  tmp.half = tmp.prec != HQ_PREC_FP32;
   tmp.D = n_heads * 64;
   tmp.nh = n_heads;
   HQ_CUDA(nullptr, cudaDeviceGetAttribute(&tmp.num_sms, cudaDevAttrMultiProcessorCount, dev));
-  if ((rc = set_smem(&tmp, attention_decode_kernel<bf16>, 64 * 1024))) return rc;
-  if ((rc = set_smem(&tmp, attention_decode_kernel<float>, 64 * 1024))) return rc;
-  if ((rc = set_smem(&tmp, attention_decode_mma_kernel, 112 * 1024))) return rc;
+  if ((rc = set_attn_attrs(&tmp))) return rc;
   HQ_CUDA(nullptr, cudaMalloc(reinterpret_cast<void**>(&tmp.att_sched), 16));
   cudaMemsetAsync(tmp.att_sched, 0, 16, st);
-  if (tmp.bf16 && variant != 1) {
+  if (tmp.half && variant != 1) {
     const int groups = attn_groups(&tmp, n_heads);
     tmp.kc = const_cast<void*>(K);
     tmp.vc = const_cast<void*>(V);
@@ -1941,12 +1970,11 @@ extern "C" int hq_debug_attention(int prec, const void* q, const void* K, const 
     }
   }
   if (variant == 1) tmp.dbg.attn_scalar = 1;
-  if (tmp.bf16)
-    attention<bf16>(&tmp, st, static_cast<const bf16*>(q), static_cast<const bf16*>(K), static_cast<const bf16*>(V),
-                    static_cast<bf16*>(out), B, 1, t_stride, n_keys, 0);
-  else
-    attention<float>(&tmp, st, static_cast<const float*>(q), static_cast<const float*>(K), static_cast<const float*>(V),
-                     static_cast<float*>(out), B, 1, t_stride, n_keys, 0);
+  with_act(tmp.prec, [&](auto tag) {
+    using AT = decltype(tag);
+    attention<AT>(&tmp, st, static_cast<const AT*>(q), static_cast<const AT*>(K), static_cast<const AT*>(V), static_cast<AT*>(out),
+                  B, 1, t_stride, n_keys, 0);
+  });
   cudaError_t e = cudaStreamSynchronize(st);
   cudaFree(tmp.att_sched);
   if (e == cudaSuccess) e = tmp.launch_err;
@@ -1975,15 +2003,20 @@ extern "C" int hq_debug_gemm(int prec, const void* A, const void* W, float* C, i
     e.outf = C; e.ldo = N;
     gemm_f32<EPI_F32>(&tmp, st, static_cast<const float*>(A), static_cast<const float*>(W), M, N, K, e);
   } else {
-    if (K % 64 != 0 || N % 64 != 0) {
-      set_err(nullptr, "hq_debug_gemm(bf16): K %% 64 and N %% 64 must be 0");
+    if (prec != HQ_PREC_BF16 && prec != HQ_PREC_F16) {
+      set_err(nullptr, "hq_debug_gemm: unknown precision %d", prec);
       return HQ_ERR_INVALID;
     }
+    if (K % 64 != 0 || N % 64 != 0) {
+      set_err(nullptr, "hq_debug_gemm(bf16 / fp16): K %% 64 and N %% 64 must be 0");
+      return HQ_ERR_INVALID;
+    }
+    tmp.prec = prec;
     int dev = 0;
     HQ_CUDA(nullptr, cudaGetDevice(&dev));
     int rc = check_device(&tmp, dev);
     if (rc == HQ_OK) rc = get_encode_fn(&tmp, &tmp.encode);
-    if (rc == HQ_OK) rc = set_gemm_attrs(&tmp);
+    if (rc == HQ_OK) rc = set_gemm_attrs_for(&tmp);
     // A rows are padded to the 128-row tile by a zero-filled staging copy so that the TMA box never leaves the tensor
     const int Mp = (M + 127) / 128 * 128;
     void* Ap = nullptr;
@@ -1999,11 +2032,16 @@ extern "C" int hq_debug_gemm(int prec, const void* A, const void* W, float* C, i
     if (rc == HQ_OK) rc = make_map(&tmp, &mW, const_cast<void*>(W), N, K, 64);
     if (rc == HQ_OK) rc = make_pair_maps(&tmp, &mWp, const_cast<void*>(W), N, K);
     if (rc == HQ_OK) {
-      EpiParams<bf16> e;
-      memset(&e, 0, sizeof(e));
-      e.outf = C; e.ldo = N;
       tmp.dbg.force_bn = tile;
-      gemm_bf16<EPI_F32>(&tmp, st, mA, K >= 128 ? &mA3 : nullptr, mW, mWp, 0, M, N, K, e);
+      with_act(prec, [&](auto tag) {
+        using AT = decltype(tag);
+        if constexpr (sizeof(AT) == 2) {
+          EpiParams<AT> e;
+          memset(&e, 0, sizeof(e));
+          e.outf = C; e.ldo = N;
+          gemm_tc<EPI_F32, AT>(&tmp, st, mA, K >= 128 ? &mA3 : nullptr, mW, mWp, 0, M, N, K, e);
+        }
+      });
     }
     cudaError_t se = cudaStreamSynchronize(st);
     if (Ap) cudaFree(Ap);
@@ -2039,7 +2077,7 @@ static EpiParams<AT> debug_epi_params(const hq_debug_epi* d) {
 }
 
 static const char* debug_epi_invalid(int prec, int w_rows, int M, int N, int K, const hq_debug_epi* d) {
-  if (prec != HQ_PREC_BF16 && prec != HQ_PREC_FP32) return "unknown precision";
+  if (prec != HQ_PREC_BF16 && prec != HQ_PREC_F16 && prec != HQ_PREC_FP32) return "unknown precision";
   if (M < 1 || N < 32 || N % 32 != 0 || K < 64 || K % 64 != 0) return "shape: need M >= 1, N % 32 == 0, K % 64 == 0";
   if (d->w_row_off < 0 || w_rows < d->w_row_off + N) return "W needs w_rows >= w_row_off + N rows";
   if (d->epi < EPI_QKV || d->epi > EPI_F32) return "epi must be QKV, RESID, GELU or F32";
@@ -2095,11 +2133,12 @@ extern "C" int hq_debug_gemm_epi(int prec, const void* A, const void* W, int w_r
       default: gemm_f32<EPI_F32>(&tmp, st, A32, W32, M, N, K, ep);
     }
   } else {
+    tmp.prec = prec;
     int dev = 0;
     HQ_CUDA(nullptr, cudaGetDevice(&dev));
     int rc = check_device(&tmp, dev);
     if (rc == HQ_OK) rc = get_encode_fn(&tmp, &tmp.encode);
-    if (rc == HQ_OK) rc = set_gemm_attrs(&tmp);
+    if (rc == HQ_OK) rc = set_gemm_attrs_for(&tmp);
     // A rows padded to the 128-row tile by a zero-filled staging copy, as hq_debug_gemm
     const int Mp = (M + 127) / 128 * 128;
     void* Ap = nullptr;
@@ -2115,15 +2154,20 @@ extern "C" int hq_debug_gemm_epi(int prec, const void* A, const void* W, int w_r
     if (rc == HQ_OK) rc = make_map(&tmp, &mW, const_cast<void*>(W), w_rows, K, 64);
     if (rc == HQ_OK) rc = make_pair_maps(&tmp, &mWp, const_cast<void*>(W), w_rows, K);
     if (rc == HQ_OK) {
-      const EpiParams<bf16> ep = debug_epi_params<bf16>(d);
       const CUtensorMap* a3 = K >= 128 ? &mA3 : nullptr;
       const int off = d->w_row_off;
-      switch (d->epi) {
-        case EPI_QKV: gemm_bf16<EPI_QKV>(&tmp, st, mA, a3, mW, mWp, off, M, N, K, ep); break;
-        case EPI_RESID: gemm_bf16<EPI_RESID>(&tmp, st, mA, a3, mW, mWp, off, M, N, K, ep); break;
-        case EPI_GELU: gemm_bf16<EPI_GELU>(&tmp, st, mA, a3, mW, mWp, off, M, N, K, ep); break;
-        default: gemm_bf16<EPI_F32>(&tmp, st, mA, a3, mW, mWp, off, M, N, K, ep, d->splits);
-      }
+      with_act(prec, [&](auto tag) {
+        using AT = decltype(tag);
+        if constexpr (sizeof(AT) == 2) {
+          const EpiParams<AT> ep = debug_epi_params<AT>(d);
+          switch (d->epi) {
+            case EPI_QKV: gemm_tc<EPI_QKV, AT>(&tmp, st, mA, a3, mW, mWp, off, M, N, K, ep); break;
+            case EPI_RESID: gemm_tc<EPI_RESID, AT>(&tmp, st, mA, a3, mW, mWp, off, M, N, K, ep); break;
+            case EPI_GELU: gemm_tc<EPI_GELU, AT>(&tmp, st, mA, a3, mW, mWp, off, M, N, K, ep); break;
+            default: gemm_tc<EPI_F32, AT>(&tmp, st, mA, a3, mW, mWp, off, M, N, K, ep, d->splits);
+          }
+        }
+      });
     }
     cudaError_t se = cudaStreamSynchronize(st);
     if (Ap) cudaFree(Ap);
@@ -2150,7 +2194,7 @@ extern "C" int hq_debug_layernorm(int prec_out, float* x, const float* gamma, co
                                   int n_fold, size_t fold_stride, const float* fold_bias, void* stream) {
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const char* bad = nullptr;
-  if (prec_out != HQ_PREC_BF16 && prec_out != HQ_PREC_FP32) bad = "unknown precision";
+  if (prec_out != HQ_PREC_BF16 && prec_out != HQ_PREC_F16 && prec_out != HQ_PREC_FP32) bad = "unknown precision";
   else if (!x || !gamma || !beta || !out) bad = "null x, gamma, beta or out";
   else if (rows < 1 || D < 4 || D % 4 != 0) bad = "rows >= 1 and D % 4 == 0";
   else if (in_group < 1 || in_mul < 0 || in_off < 0 || out_mul < 1) bad = "row map";
@@ -2164,12 +2208,11 @@ extern "C" int hq_debug_layernorm(int prec_out, float* x, const float* gamma, co
   tmp.D = D;
   Fold f;
   f.partial = fold; f.n = n_fold; f.stride = fold_stride; f.bias = fold_bias;
-  if (prec_out == HQ_PREC_BF16)
-    layernorm_rows<bf16>(&tmp, st, "layernorm", x, gamma, beta, add, static_cast<bf16*>(out), rows, in_group, in_mul, in_off,
-                         out_mul, f);
-  else
-    layernorm_rows<float>(&tmp, st, "layernorm", x, gamma, beta, add, static_cast<float*>(out), rows, in_group, in_mul, in_off,
-                          out_mul, f);
+  with_act(prec_out, [&](auto tag) {
+    using AT = decltype(tag);
+    layernorm_rows<AT>(&tmp, st, "layernorm", x, gamma, beta, add, static_cast<AT*>(out), rows, in_group, in_mul, in_off, out_mul,
+                       f);
+  });
   cudaError_t e = tmp.launch_err;
   if (e == cudaSuccess) e = cudaStreamSynchronize(st);
   if (e != cudaSuccess) {
@@ -2223,15 +2266,12 @@ extern "C" int hq_bench_attention(hq_ctx* ctx, int B, int n_keys, int iters, flo
   ctx->launch_err = cudaSuccess;
   struct PdlOff { hq_ctx* c; bool saved; PdlOff(hq_ctx* x) : c(x), saved(x->use_pdl) { x->use_pdl = false; } ~PdlOff() { c->use_pdl = saved; } } pdl_off(ctx);
   auto launch = [&](int l) {
-    if (ctx->bf16) {
-      bf16* kc = static_cast<bf16*>(ctx->kc) + l * lstride;
-      bf16* vc = static_cast<bf16*>(ctx->vc) + l * lstride;
-      attention<bf16>(ctx, st, static_cast<bf16*>(ctx->q), kc, vc, static_cast<bf16*>(ctx->att.ptr), B, 1, ctx->Tc, n_keys, 0);
-    } else {
-      float* kc = static_cast<float*>(ctx->kc) + l * lstride;
-      float* vc = static_cast<float*>(ctx->vc) + l * lstride;
-      attention<float>(ctx, st, static_cast<float*>(ctx->q), kc, vc, static_cast<float*>(ctx->att.ptr), B, 1, ctx->Tc, n_keys, 0);
-    }
+    with_act(ctx->prec, [&](auto tag) {
+      using AT = decltype(tag);
+      AT* kc = static_cast<AT*>(ctx->kc) + l * lstride;
+      AT* vc = static_cast<AT*>(ctx->vc) + l * lstride;
+      attention<AT>(ctx, st, static_cast<AT*>(ctx->q), kc, vc, static_cast<AT*>(ctx->att.ptr), B, 1, ctx->Tc, n_keys, 0);
+    });
   };
   for (int i = 0; i < 3; ++i) launch(i % ctx->L);
   HQ_CUDA(ctx, cudaEventRecord(e0, st));
@@ -2269,15 +2309,12 @@ extern "C" int hq_debug_attention_phases(hq_ctx* ctx, int B, int n_keys, int war
   struct PdlOff { hq_ctx* c; bool saved; PdlOff(hq_ctx* x) : c(x), saved(x->use_pdl) { x->use_pdl = false; } ~PdlOff() { c->use_pdl = saved; } } pdl_off(ctx);
   const int64_t before = ctx->launches;
   auto launch = [&](int l) {
-    if (ctx->bf16) {
-      bf16* kc = static_cast<bf16*>(ctx->kc) + l * lstride;
-      bf16* vc = static_cast<bf16*>(ctx->vc) + l * lstride;
-      attention<bf16>(ctx, st, static_cast<bf16*>(ctx->q), kc, vc, static_cast<bf16*>(ctx->att.ptr), B, 1, ctx->Tc, n_keys, 0);
-    } else {
-      float* kc = static_cast<float*>(ctx->kc) + l * lstride;
-      float* vc = static_cast<float*>(ctx->vc) + l * lstride;
-      attention<float>(ctx, st, static_cast<float*>(ctx->q), kc, vc, static_cast<float*>(ctx->att.ptr), B, 1, ctx->Tc, n_keys, 0);
-    }
+    with_act(ctx->prec, [&](auto tag) {
+      using AT = decltype(tag);
+      AT* kc = static_cast<AT*>(ctx->kc) + l * lstride;
+      AT* vc = static_cast<AT*>(ctx->vc) + l * lstride;
+      attention<AT>(ctx, st, static_cast<AT*>(ctx->q), kc, vc, static_cast<AT*>(ctx->att.ptr), B, 1, ctx->Tc, n_keys, 0);
+    });
   };
   for (int i = 0; i < warm; ++i) launch(i % ctx->L);
   HQ_CUDA(ctx, cudaStreamSynchronize(st));
@@ -2321,18 +2358,19 @@ extern "C" int hq_bench_gemm(hq_ctx* ctx, int kind, int M, int iters, float* use
   struct PdlOff { hq_ctx* c; bool saved; PdlOff(hq_ctx* x) : c(x), saved(x->use_pdl) { x->use_pdl = false; } ~PdlOff() { c->use_pdl = saved; } } pdl_off(ctx);
   auto launch = [&](int i) {
     const BlockW& w = ctx->blocks[i % ctx->L];
-    if (ctx->bf16) {
-      EpiParams<bf16> e;
+    with_act(ctx->prec, [&](auto tag) {
+      using AT = decltype(tag);
+      EpiParams<AT> e;
       memset(&e, 0, sizeof(e));
       if (kind == 0) {
-        e.bias = w.bqkv; e.q = static_cast<bf16*>(ctx->q); e.kdst = static_cast<bf16*>(ctx->kd); e.vdst = static_cast<bf16*>(ctx->vd);
+        e.bias = w.bqkv; e.q = static_cast<AT*>(ctx->q); e.kdst = static_cast<AT*>(ctx->kd); e.vdst = static_cast<AT*>(ctx->vd);
         e.D = D; e.rpb = 4; e.t_stride = 5; e.t0 = 1;
         gemm_any<EPI_QKV>(ctx, st, ctx->h, w.qkv, 0, M, 3 * D, D, e);
       } else if (kind == 1) {
         e.bias = w.bproj; e.x = ctx->yd;
         gemm_any<EPI_RESID>(ctx, st, ctx->att, w.proj, 0, M, D, D, e);
       } else if (kind == 2) {
-        e.bias = w.b1; e.out = static_cast<bf16*>(ctx->mlp.ptr);
+        e.bias = w.b1; e.out = static_cast<AT*>(ctx->mlp.ptr);
         gemm_any<EPI_GELU>(ctx, st, ctx->h, w.fc1, 0, M, 4 * D, D, e);
       } else if (kind == 3) {
         e.bias = w.b2; e.x = ctx->yd;
@@ -2341,27 +2379,7 @@ extern "C" int hq_bench_gemm(hq_ctx* ctx, int kind, int M, int iters, float* use
         e.outf = ctx->logits; e.ldo = ctx->Vmax;
         gemm_any<EPI_F32>(ctx, st, ctx->h, ctx->head_top, 0, M, ctx->Vt, D, e);
       }
-    } else {
-      EpiParams<float> e;
-      memset(&e, 0, sizeof(e));
-      if (kind == 0) {
-        e.bias = w.bqkv; e.q = static_cast<float*>(ctx->q); e.kdst = static_cast<float*>(ctx->kd); e.vdst = static_cast<float*>(ctx->vd);
-        e.D = D; e.rpb = 4; e.t_stride = 5; e.t0 = 1;
-        gemm_any<EPI_QKV>(ctx, st, ctx->h, w.qkv, 0, M, 3 * D, D, e);
-      } else if (kind == 1) {
-        e.bias = w.bproj; e.x = ctx->yd;
-        gemm_any<EPI_RESID>(ctx, st, ctx->att, w.proj, 0, M, D, D, e);
-      } else if (kind == 2) {
-        e.bias = w.b1; e.out = static_cast<float*>(ctx->mlp.ptr);
-        gemm_any<EPI_GELU>(ctx, st, ctx->h, w.fc1, 0, M, 4 * D, D, e);
-      } else if (kind == 3) {
-        e.bias = w.b2; e.x = ctx->yd;
-        gemm_any<EPI_RESID>(ctx, st, ctx->mlp, w.fc2, 0, M, D, 4 * D, e);
-      } else {
-        e.outf = ctx->logits; e.ldo = ctx->Vmax;
-        gemm_any<EPI_F32>(ctx, st, ctx->h, ctx->head_top, 0, M, ctx->Vt, D, e);
-      }
-    }
+    });
   };
   // rows >= max_batch of kd/vd would be out of range for the qkv epilogue: clamp M for kind 0
   if (kind == 0 && M > 4 * ctx->max_batch) M = 4 * ctx->max_batch;
@@ -2417,7 +2435,7 @@ extern "C" int hq_bench_gemm_shape(int M, int N, int K, int tile, int iters, int
   HQ_CUDA(nullptr, cudaGetDevice(&dev));
   int rc = check_device(&tmp, dev);
   if (rc == HQ_OK) rc = get_encode_fn(&tmp, &tmp.encode);
-  if (rc == HQ_OK) rc = set_gemm_attrs(&tmp);
+  if (rc == HQ_OK) rc = set_gemm_attrs<bf16>(&tmp);
   if (rc != HQ_OK) {
     g_last_error = tmp.err;
     return rc;
@@ -2461,7 +2479,7 @@ extern "C" int hq_bench_gemm_shape(int M, int N, int K, int tile, int iters, int
       if (flush == 1) cudaMemsetAsync(flushbuf, i & 0xff, flush_bytes, st);
       if (flush == 2) read_sweep_kernel<<<1184, 256, 0, st>>>(static_cast<const uint4*>(flushbuf), flush_bytes / 16, sink);
       if (i >= 0) cudaEventRecord(ev[2 * i], st);
-      gemm_bf16<EPI_F32>(&tmp, st, mA, K >= 128 ? &mA3 : nullptr, mW[c], mWp[c], 0, M, N, K, e, splits);
+      gemm_tc<EPI_F32, bf16>(&tmp, st, mA, K >= 128 ? &mA3 : nullptr, mW[c], mWp[c], 0, M, N, K, e, splits);
       if (i >= 0) cudaEventRecord(ev[2 * i + 1], st);
     }
   }

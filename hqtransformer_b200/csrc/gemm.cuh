@@ -1,6 +1,6 @@
 // GEMM family of libhqgraft: C[M,N] = A[M,K] * W[N,K]^T with fused epilogues.
 //
-//   gemm_tc_kernel    bf16 x bf16 -> fp32 on the 5th-gen tensor cores: TMA (SWIZZLE_128B) stages A and W
+//   gemm_tc_kernel    bf16 x bf16 (or fp16 x fp16: AT) -> fp32 on the 5th-gen tensor cores: TMA (SWIZZLE_128B) stages A and W
 //                     tiles into a ring of shared-memory slots, one thread issues tcgen05.mma with the
 //                     accumulator in TMEM, four warps drain TMEM with tcgen05.ld and apply the epilogue.
 //   gemm_simt_kernel  fp32 on CUDA cores, for HQ_PREC_FP32 (the reference's use_fp16=False path).
@@ -51,13 +51,15 @@ struct EpiParams {
 
 __device__ __forceinline__ float gelu_erf(float v) { return 0.5f * v * (1.0f + erff(v * 0.70710678118654752440f)); }
 
-// The same function for outputs that are rounded to bf16 (the tcgen05 engine): x * Phi(x) with
+// The same function for outputs that are rounded to a 2-byte type (the tcgen05 engines, bf16 and fp16): x * Phi(x) with
 // Phi(x) = 1 - erfc(|x| / sqrt 2) / 2 (x >= 0), erfc(|x| / sqrt 2) / 2 (x < 0) and erfc by Abramowitz & Stegun 7.1.26
 // (|error| <= 1.5e-7 on erfc): one rcp, one ex2 and a degree-5 Horner form, ~15 instructions against ~35 for erff.  The
 // bound is absolute: |gelu_bf16out(x) - gelu(x)| <= ~4.3e-7 over [-12, 12] (fp32 restatement), below half a bf16 ulp of
 // the result wherever |gelu(x)| >~ 1e-4; for x < -6, where |gelu(x)| < 1e-8, the RELATIVE error reaches a few percent
 // (several bf16 ulps of a value that is ~0 next to the rest of the row).  tests/test_gpu_epilogues.py holds the kernel
-// to |got - gelu| <= half a bf16 ulp of gelu + 5e-7.  The exact-erf epilogue of fc1 was issue-bound on erff: 1.1 of the
+// to |got - gelu| <= half a bf16 ulp of gelu + 5e-7.  The same absolute bound is far below half an fp16 ulp wherever
+// |gelu(x)| >~ 1e-3 (fp16 keeps 11 significant bits); tests/test_gpu_fp16.py holds the fp16 epilogue to half an fp16
+// ulp + 5e-7.  The exact-erf epilogue of fc1 was issue-bound on erff: 1.1 of the
 // 1.65 us per 32-column chunk, on the critical path of every fc1 launch (profiles/r2_gemm_phases.txt).  The fp32 engine
 // (bit-exact parity with the reference) keeps gelu_erf.
 __device__ __forceinline__ float gelu_bf16out(float v) {
@@ -263,14 +265,13 @@ __device__ __forceinline__ void epilogue_tile(uint32_t tmem_base, uint8_t* slab_
             if (row_ok[it]) *reinterpret_cast<float4*>(dstf + row_a[it]) = w;
           } else {
             const size_t ro = use_b ? row_b[it] : row_a[it];
-            if (sizeof(AT) == 4) {
+            if constexpr (sizeof(AT) == 4) {
               if (row_ok[it]) *reinterpret_cast<float4*>(dst + ro) = w;
               if (row_ok[it] && dup != nullptr) *reinterpret_cast<float4*>(dup + row_a[it]) = w;
             } else {
               uint2 u;
-              __nv_bfloat162 h0 = __floats2bfloat162_rn(w.x, w.y), h1 = __floats2bfloat162_rn(w.z, w.w);
-              u.x = *reinterpret_cast<uint32_t*>(&h0);
-              u.y = *reinterpret_cast<uint32_t*>(&h1);
+              u.x = pack2_rn<AT>(w.x, w.y);
+              u.y = pack2_rn<AT>(w.z, w.w);
               if (row_ok[it]) *reinterpret_cast<uint2*>(dst + ro) = u;
               if (row_ok[it] && dup != nullptr) *reinterpret_cast<uint2*>(dup + row_a[it]) = u;
             }
@@ -465,7 +466,7 @@ gemm_tc_kernel(int trace_id, const __grid_constant__ CUtensorMap tmA, const __gr
     }
   } else if (warp == 1) {
     // ---- MMA issuer (warp-uniform loop, the elected lane issues the MMAs and their commits) ----
-    constexpr uint32_t idesc = umma_idesc_bf16(C::BM, BN);
+    constexpr uint32_t idesc = umma_idesc<AT>(C::BM, BN);
     const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);
     for (int st = 0; st < num_st; ++st) {
       const int s = st % C::STAGES;
@@ -689,7 +690,7 @@ gemm_tc2_kernel(int trace_id, const __grid_constant__ CUtensorMap tmA, const __g
   } else if (warp == 1) {
     if (leader) {
       // ---- MMA issuer (leader CTA only; warp-uniform loop, the elected lane issues the MMAs and their commits) ----
-      constexpr uint32_t idesc = umma_idesc_bf16(256, BN);
+      constexpr uint32_t idesc = umma_idesc<AT>(256, BN);
       const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);
       int g = 0, it = 0;
       for (int tile = pair; tile < total_tiles; tile += npairs, ++it) {

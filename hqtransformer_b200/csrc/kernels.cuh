@@ -278,7 +278,7 @@ depth_pos_rows_kernel(int trace_id, float* y, const float* P_depth, int D) {
 
 // ------------------------------------------------------------------------------------------------
 // K2: LayerNorm (eps 1e-5, affine), one warp per row, fp32 statistics (two-pass).
-//   out[r * out_mul] = LN(x[(r / in_group) * in_mul + in_off + r % in_group]) * gamma + beta (+ add)    OutT = float | bf16
+//   out[r * out_mul] = LN(x[(r / in_group) * in_mul + in_off + r % in_group]) * gamma + beta (+ add)    OutT = float | bf16 | f16
 // (in_group = out_mul = 1 everywhere except the 'bidirectional' depth pass, whose five-token stacks are normalised by
 //  ln_top (token 0) and ln_bot (tokens 1..4) and whose token 0 comes from ln_f of the spatial stream)
 // The (+ add) form produces the depth transformer's start token hs + sos_depth (hierarchical_ar.py:561, 685).
@@ -289,14 +289,13 @@ constexpr int LN_MAXFOLD = 6; // split-K partial sums a LayerNorm can fold in (k
 
 template <typename OutT>
 __device__ __forceinline__ void ln_store4(OutT* o, int i, float y0, float y1, float y2, float y3) {
-  if (sizeof(OutT) == 4) {
+  if constexpr (sizeof(OutT) == 4) {
     *reinterpret_cast<float4*>(reinterpret_cast<float*>(o) + i) = make_float4(y0, y1, y2, y3);
   } else {
     uint2 u;
-    __nv_bfloat162 h0 = __floats2bfloat162_rn(y0, y1), h1 = __floats2bfloat162_rn(y2, y3);
-    u.x = *reinterpret_cast<uint32_t*>(&h0);
-    u.y = *reinterpret_cast<uint32_t*>(&h1);
-    *reinterpret_cast<uint2*>(reinterpret_cast<bf16*>(o) + i) = u;
+    u.x = pack2_rn<OutT>(y0, y1);
+    u.y = pack2_rn<OutT>(y2, y3);
+    *reinterpret_cast<uint2*>(o + i) = u;
   }
 }
 
@@ -587,7 +586,7 @@ attention_fewkeys_kernel(int trace_id, const AT* __restrict__ q, const AT* __res
 // pieces - is issued before anything is used (one memory round trip), and each lane owns one 16-byte piece of one
 // output row, so the value pass needs no cross-lane reduction.
 // ------------------------------------------------------------------------------------------------
-// 8 consecutive activations kept as loaded (bf16: one 16-byte register quad) until they are used
+// 8 consecutive activations kept as loaded (bf16 / fp16: one 16-byte register quad) until they are used
 template <typename AT> struct Raw8;
 template <> struct Raw8<bf16> {
   uint4 u;
@@ -597,6 +596,19 @@ template <> struct Raw8<bf16> {
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
       const float2 f = __bfloat1622float2(h[i]);
+      o[2 * i] = f.x;
+      o[2 * i + 1] = f.y;
+    }
+  }
+};
+template <> struct Raw8<f16> {
+  uint4 u;
+  __device__ __forceinline__ void load(const f16* p) { u = *reinterpret_cast<const uint4*>(p); }
+  __device__ __forceinline__ void get(float (&o)[8]) const {
+    const uint32_t w[4] = {u.x, u.y, u.z, u.w};
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      const float2 f = unpack2<f16>(w[i]);
       o[2 * i] = f.x;
       o[2 * i + 1] = f.y;
     }
@@ -844,7 +856,7 @@ attention_decode_kernel(int trace_id, const AT* __restrict__ q, const AT* __rest
 }
 
 // ------------------------------------------------------------------------------------------------
-// K5a (bf16): the same single-query attention as ONE streaming pass, persistent, on the mma.sync register path.
+// K5a (bf16 / fp16): the same single-query attention as ONE streaming pass, persistent, on the mma.sync register path.
 // Measured on the scalar kernel above (profiles/r1_attn_phases.txt): with ~25 MB of bulk copies in flight a request
 // takes ~4 us to land, and every point where the computation waits for "all of K" (the softmax between the score pass
 // and the value pass, the next item) pays that latency again; its score pass is also issue-bound (3 shuffles per 4 keys).
@@ -859,7 +871,8 @@ attention_decode_kernel(int trace_id, const AT* __restrict__ q, const AT* __rest
 //   * consumer warp = one head, ONLINE softmax (running max m, running sum l, rescaled accumulator): per stage
 //     scores = mma.m16n8k16(A = 8 keys x 16 dims via ldmatrix.x2, B = q in column 0), then
 //     acc = acc * exp(m_old - m_new) + mma.m16n8k8(A = V^T via ldmatrix.x2.trans, B = (p_hi, p_lo) in columns 0 / 1):
-//     the bf16 head and tail of the fp32 weight p = exp(s - m_new), so p keeps ~16 mantissa bits.  out = acc / l.
+//     the bf16 head and tail of the fp32 weight p = exp(s - m_new), so p keeps ~16 mantissa bits (fp16: ~22 near
+//     p = 1, an absolute floor below, noted at the split).  out = acc / l.
 // Same function as the reference's bmm / softmax / bmm (layers.py:102, 183-186); the online form differs from the
 // two-pass form only by fp32 rounding of the rescale factors.  Scores scaled by hs^-1/2 = 2^-3 (exact).
 // ------------------------------------------------------------------------------------------------
@@ -894,9 +907,40 @@ __device__ __forceinline__ void mma_bf16_1688(float (&c)[4], uint32_t a0, uint32
 #endif
 }
 
+// D (16x8 fp32) += A (16x16 fp16, row) * B (16x8 fp16, col)
+__device__ __forceinline__ void mma_f16_16816(float (&c)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t b0,
+                                              uint32_t b1) {
+#if defined(__CUDA_ARCH__)
+  asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
+               : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
+               : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
+#endif
+}
+// D (16x8 fp32) += A (16x8 fp16, row) * B (8x8 fp16, col)
+__device__ __forceinline__ void mma_f16_1688(float (&c)[4], uint32_t a0, uint32_t a1, uint32_t b0) {
+#if defined(__CUDA_ARCH__)
+  asm volatile("mma.sync.aligned.m16n8k8.row.col.f32.f16.f16.f32 {%0,%1,%2,%3}, {%4,%5}, {%6}, {%0,%1,%2,%3};"
+               : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
+               : "r"(a0), "r"(a1), "r"(b0));
+#endif
+}
+// the two forms for the element type AT of the operands
+template <typename AT>
+__device__ __forceinline__ void mma_16816(float (&c)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t b0, uint32_t b1) {
+  if constexpr (std::is_same<AT, bf16>::value) mma_bf16_16816(c, a0, a1, a2, a3, b0, b1);
+  else mma_f16_16816(c, a0, a1, a2, a3, b0, b1);
+}
+template <typename AT>
+__device__ __forceinline__ void mma_1688(float (&c)[4], uint32_t a0, uint32_t a1, uint32_t b0) {
+  if constexpr (std::is_same<AT, bf16>::value) mma_bf16_1688(c, a0, a1, b0);
+  else mma_f16_1688(c, a0, a1, b0);
+}
+
+// AT = bf16 | f16 (the element type of q, K, V and out)
+template <typename AT>
 __global__ void __launch_bounds__((ATTD_MAXHPC + 1) * 32)
 attention_decode_mma_kernel(int trace_id, const __grid_constant__ CUtensorMap tmK, const __grid_constant__ CUtensorMap tmV,
-                            int row_base, const bf16* __restrict__ q, bf16* __restrict__ out, int D, int t_stride, int n_keys,
+                            int row_base, const AT* __restrict__ q, AT* __restrict__ out, int D, int t_stride, int n_keys,
                             int hpc, int groups, int n_items, int stages, unsigned int* __restrict__ sched) {
 #if defined(__CUDA_ARCH__)
   TraceScope trace_scope(trace_id);
@@ -1049,7 +1093,7 @@ attention_decode_mma_kernel(int trace_id, const __grid_constant__ CUtensorMap tm
       for (int ks = 0; ks < 4; ++ks) {
         uint32_t a0, a2;
         ldmatrix_x2(kbase + frag_off[ks], a0, a2);
-        mma_bf16_16816(sc, a0, 0u, a2, 0u, qb[ks][0], qb[ks][1]);
+        mma_16816<AT>(sc, a0, 0u, a2, 0u, qb[ks][0], qb[ks][1]);
       }
       float sk = __shfl_sync(0xffffffffu, sc[0], lane & ~3) * 0.125f;   // every lane of quad gq: score of key gq
       if (gq >= left) sk = -INFINITY;                                    // rows past the cache end are not keys
@@ -1066,17 +1110,20 @@ attention_decode_mma_kernel(int trace_id, const __grid_constant__ CUtensorMap tm
       ps += __shfl_xor_sync(0xffffffffu, ps, 16);
       l_run = l_run * alpha + ps;
       m_run = m_new;
-      // ---- B operand of the value MMA: keys 2*tq, 2*tq+1; column 0 = bf16 head of p, column 1 = bf16 tail ----
+      // ---- B operand of the value MMA: keys 2*tq, 2*tq+1; column 0 = AT head of p, column 1 = AT tail ----
+      // fp16: the tail lies below the normal range (2^-14) for every p < 1/4, so it is rounded on the subnormal grid (spacing
+      // 2^-24): head + tail carry p to an absolute ~2^-25 (~3e-8; weights below that vanish), not to a relative 2^-22 -
+      // at most ~3e-8 per key next to l_run >= 1.
       const float p0 = __shfl_sync(0xffffffffu, pk, 8 * tq);
       const float p1 = __shfl_sync(0xffffffffu, pk, 8 * tq + 4);
       uint32_t pb = 0u;
       {
-        __nv_bfloat162 h = __floats2bfloat162_rn(p0, p1);
+        uint32_t h = pack2_rn<AT>(p0, p1);
         if (gq == 1) {
-          const float2 f = __bfloat1622float2(h);
-          h = __floats2bfloat162_rn(p0 - f.x, p1 - f.y);
+          const float2 f = unpack2<AT>(h);
+          h = pack2_rn<AT>(p0 - f.x, p1 - f.y);
         }
-        if (gq < 2) pb = *reinterpret_cast<uint32_t*>(&h);
+        if (gq < 2) pb = h;
       }
       // value rows past the cache end (other cache slots, or whatever the allocation held): 0 * NaN must not
       // reach the accumulator
@@ -1092,7 +1139,7 @@ attention_decode_mma_kernel(int trace_id, const __grid_constant__ CUtensorMap tm
       for (int mt = 0; mt < 4; ++mt) {
         uint32_t a0, a1;
         ldmatrix_x2_trans(vbase + frag_off[mt], a0, a1);
-        mma_bf16_1688(o[mt], a0 & vmask, a1 & vmask, pb);
+        mma_1688<AT>(o[mt], a0 & vmask, a1 & vmask, pb);
       }
       __syncwarp();
       if (lane == 0) mbar_arrive(&empty_bar[s]);

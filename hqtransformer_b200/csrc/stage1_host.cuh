@@ -304,9 +304,9 @@ extern "C" int hq_s1_load_param(hq_s1_ctx* ctx, const char* name, const void* da
     }
     f32 = tmp;
   }
-  if (dtype == HQ_F32) launch_convert<float>(src, f32, false, n);
-  else if (dtype == HQ_BF16) launch_convert<bf16>(src, f32, false, n);
-  else launch_convert<__half>(src, f32, false, n);
+  if (dtype == HQ_F32) launch_convert<float>(src, f32, HQ_PREC_FP32, n);
+  else if (dtype == HQ_BF16) launch_convert<bf16>(src, f32, HQ_PREC_FP32, n);
+  else launch_convert<__half>(src, f32, HQ_PREC_FP32, n);
   if (s.kind == 1) {
     S1Conv* c = s.conv;
     bf16* dst = c->w + static_cast<size_t>(s.row_off) * c->taps * c->Cin;

@@ -11,6 +11,8 @@ from . import _lib
 from ._lib import HQConfig, HQRunArgs, HQSamplingParams, check
 
 _TORCH2HQ = {torch.float32: _lib.HQ_F32, torch.bfloat16: _lib.HQ_BF16, torch.float16: _lib.HQ_F16}
+# activation dtype of the debug hooks -> engine precision (bf16 / fp16: the tcgen05 engines, fp32: the CUDA-core engine)
+_ACT2PREC = {torch.bfloat16: _lib.HQ_PREC_BF16, torch.float16: _lib.HQ_PREC_F16, torch.float32: _lib.HQ_PREC_FP32}
 
 
 @dataclass
@@ -63,6 +65,8 @@ class Engine:
                  use_pdl: bool = True, use_chain: bool = False, model_type: str = "parallel",
                  embedding_type: str = "transformer1", position_embedding: str = "1d", code_levels: int = 2,
                  vocab_mid: int = 0, fuse_head_sampler: bool = True):
+        if precision not in _lib.HQ_PREC:
+            raise ValueError(f"precision={precision!r}: one of {sorted(_lib.HQ_PREC)}")
         self._lib = _lib.load()
         self._ctx = C.c_void_p()
         dev = torch.device(device) if not isinstance(device, int) else torch.device("cuda", device)
@@ -77,7 +81,7 @@ class Engine:
                        vocab_top=vocab_top, vocab_bot=vocab_bot, vocab_txt=vocab_txt, n_classes=n_classes or 0,
                        ctx_len_img=ctx_len_img, ctx_len_txt=ctx_len_txt,
                        cond_kind={"cls": _lib.HQ_COND_CLS, "txt": _lib.HQ_COND_TXT, "uncond": _lib.HQ_COND_UNCOND}[cond],
-                       precision={"bf16": _lib.HQ_PREC_BF16, "fp32": _lib.HQ_PREC_FP32}[precision],
+                       precision=_lib.HQ_PREC[precision],
                        max_seq_len=max_seq_len, use_cuda_graph=1 if use_cuda_graph else 0,
                        use_pdl=1 if use_pdl else 0, use_chain=1 if use_chain else 0,
                        model_type=_lib.HQ_MODEL[model_type], embedding_kind=_lib.HQ_EMB[embedding_type],
@@ -257,14 +261,14 @@ class Engine:
 
 # ---- stand-alone hooks used by tests / bench ----
 def debug_gemm(A: torch.Tensor, W: torch.Tensor, tile: int = 0) -> torch.Tensor:
-    """C = A @ W^T through the engine's GEMM kernels (bf16 -> tcgen05 path, fp32 -> CUDA-core path).
+    """C = A @ W^T through the engine's GEMM kernels (bf16 / fp16 -> tcgen05 path, fp32 -> CUDA-core path).
     tile: 0 = engine heuristic, 32..256 = CTA-pair kernel of that width, -64/-128 = single-CTA kernel."""
     lib = _lib.load()
     assert A.is_cuda and W.is_cuda and A.dtype == W.dtype and A.is_contiguous() and W.is_contiguous()
     M, K = A.shape
     N = W.shape[0]
     out = torch.empty(M, N, dtype=torch.float32, device=A.device)
-    prec = _lib.HQ_PREC_BF16 if A.dtype == torch.bfloat16 else _lib.HQ_PREC_FP32
+    prec = _ACT2PREC[A.dtype]
     with torch.cuda.device(A.device):
         st = torch.cuda.current_stream(A.device).cuda_stream
         check(lib.hq_debug_gemm(prec, A.data_ptr(), W.data_ptr(), out.data_ptr(), M, N, K, tile, C.c_void_p(st)), None,
@@ -283,7 +287,7 @@ def debug_gemm_epi(A: torch.Tensor, W: torch.Tensor, epi: int, *, N: Optional[in
                    ldo: int = 0, splits: int = 1, split_stride: int = 0) -> None:
     """A [M, K] @ W[w_row_off : w_row_off + N]^T through the engine's GEMM kernels with fused epilogue `epi` (EPI_QKV,
     EPI_RESID, EPI_GELU or EPI_F32), writing into the caller's buffers in place; see hq_debug_epi in include/hqgraft.h.
-    bf16 A / W take the tcgen05 kernels (`tile` and `ks1` pin the plan), fp32 the CUDA-core kernel.  Synchronous."""
+    bf16 / fp16 A / W take the tcgen05 kernels (`tile` and `ks1` pin the plan), fp32 the CUDA-core kernel.  Synchronous."""
     lib = _lib.load()
     assert A.is_cuda and W.is_cuda and A.dtype == W.dtype and A.is_contiguous() and W.is_contiguous()
     act = A.dtype
@@ -299,7 +303,7 @@ def debug_gemm_epi(A: torch.Tensor, W: torch.Tensor, epi: int, *, N: Optional[in
                         w_row_off=w_row_off, ldo=ldo, splits=splits, reserved=0, split_stride=split_stride,
                         bias=_ptr(bias), q=_ptr(q), kdst=_ptr(kdst), vdst=_ptr(vdst), vdup=_ptr(vdup), x=_ptr(x),
                         out=_ptr(out), outf=_ptr(outf))
-    prec = _lib.HQ_PREC_BF16 if act == torch.bfloat16 else _lib.HQ_PREC_FP32
+    prec = _ACT2PREC[act]
     with torch.cuda.device(A.device):
         st = torch.cuda.current_stream(A.device).cuda_stream
         check(lib.hq_debug_gemm_epi(prec, A.data_ptr(), W.data_ptr(), w_rows, M, N, K, C.byref(e), C.c_void_p(st)), None,
@@ -313,13 +317,13 @@ def debug_layernorm(x: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, ou
     """The engine's LayerNorm launch (layernorm_kernel, instantiation chosen by n_fold as in the sampler) on fp32 x
     [*, D], in place: out[r * out_mul] = LN(x[(r // in_group) * in_mul + in_off + r % in_group]) * gamma + beta (+ add);
     with n_fold > 0 that x row first gets fold_bias + the partial sums fold.view(-1)[s * fold_stride + row * D ...] added
-    and written back.  `out` is bf16 or fp32.  Synchronous."""
+    and written back.  `out` is bf16, fp16 or fp32.  Synchronous."""
     lib = _lib.load()
     D = x.shape[-1]
     for t in (x, gamma, beta, add, fold, fold_bias):
         assert t is None or (t.is_cuda and t.dtype == torch.float32 and t.is_contiguous())
-    assert out.is_contiguous() and out.dtype in (torch.bfloat16, torch.float32)
-    prec = _lib.HQ_PREC_BF16 if out.dtype == torch.bfloat16 else _lib.HQ_PREC_FP32
+    assert out.is_contiguous() and out.dtype in _ACT2PREC
+    prec = _ACT2PREC[out.dtype]
     with torch.cuda.device(x.device):
         st = torch.cuda.current_stream(x.device).cuda_stream
         check(lib.hq_debug_layernorm(prec, x.data_ptr(), gamma.data_ptr(), beta.data_ptr(), _ptr(add), out.data_ptr(), rows,
@@ -331,13 +335,13 @@ def debug_attention(q: torch.Tensor, K: torch.Tensor, V: torch.Tensor, n_keys: i
     """Single-query attention of every row of q [B, D] over the first n_keys rows of its cache K / V [B, T, D]
     (head size 64) through the engine's decode kernels; variant 0 = engine choice, 1 = scalar bulk-staged kernel."""
     lib = _lib.load()
-    assert q.is_cuda and q.dtype == K.dtype == V.dtype and q.dtype in (torch.bfloat16, torch.float32)
+    assert q.is_cuda and q.dtype == K.dtype == V.dtype and q.dtype in _ACT2PREC
     assert q.is_contiguous() and K.is_contiguous() and V.is_contiguous() and K.shape == V.shape
     B, D = q.shape
     T = K.shape[1]
     assert K.shape == (B, T, D) and D % 64 == 0 and 1 <= n_keys <= T
     out = torch.empty_like(q)
-    prec = _lib.HQ_PREC_BF16 if q.dtype == torch.bfloat16 else _lib.HQ_PREC_FP32
+    prec = _ACT2PREC[q.dtype]
     with torch.cuda.device(q.device):
         st = torch.cuda.current_stream(q.device).cuda_stream
         check(lib.hq_debug_attention(prec, q.data_ptr(), K.data_ptr(), V.data_ptr(), out.data_ptr(), B, D // 64, T, n_keys,

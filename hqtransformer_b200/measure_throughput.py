@@ -44,6 +44,7 @@ class Experiment:                      # measure_throughput/__main__.py:34-48
     n_samples: int = 1000              # extension: images per loop (the reference hard-codes 1000, :76)
     stage1: int = 1                    # extension: 1 = build and time the stage-1 decoder too
     decode_chunks: int = 1             # extension: chunks the batch is decoded in (batch_size = the reference's protocol)
+    precision: str = "bf16"            # extension: engine of use_fp16=True - "bf16", or "fp16" (the reference's autocast type)
 
 
 def parse_cli(argv) -> Experiment:
@@ -64,10 +65,11 @@ def parse_cli(argv) -> Experiment:
     return args
 
 
-def load_model(result_path: str, device="cuda", max_batch: int = 50, with_stage1: bool = True) -> ImageGPT2:
+def load_model(result_path: str, device="cuda", max_batch: int = 50, with_stage1: bool = True,
+               precision: str = "bf16") -> ImageGPT2:
     """:25-31 - config only, no checkpoint: random-init weights of the named architecture."""
     dev = torch.device(device)
-    return ImageGPT2.from_config(result_path, device=dev.index or 0, precision="bf16", max_batch=max_batch,
+    return ImageGPT2.from_config(result_path, device=dev.index or 0, precision=precision, max_batch=max_batch,
                                  with_stage1=with_stage1, stage1_max_batch=min(max_batch, 32))
 
 
@@ -76,8 +78,10 @@ def main(args: Experiment):
     if args.code_levels not in (2, 3):
         raise NotImplementedError("code_levels must be 2 (iHQGPT) or 3 (HQTransformer)")
     device = torch.device("cuda")
+    if args.precision not in ("bf16", "fp16"):
+        raise SystemExit(f"precision={args.precision!r}: bf16 or fp16 (the engines use_fp16=True selects)")
     model_ar = load_model(args.model_path, device, args.batch_size,
-                          with_stage1=bool(args.stage1) and args.code_levels == 2).to(device).eval()
+                          with_stage1=bool(args.stage1) and args.code_levels == 2, precision=args.precision).to(device).eval()
     if (args.code_levels == 3) != hasattr(model_ar.stage2, "code_level"):
         raise SystemExit(f"code_levels={args.code_levels} does not match the model type of {args.model_path}")
     title = f"bs{args.batch_size}, sampling loops {args.warmup + 1}-{args.n_loop}"

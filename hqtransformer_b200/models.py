@@ -125,7 +125,8 @@ class iHQGPT:
         return self._engines[precision]
 
     def _engine_for(self, use_fp16: bool, batch: int) -> Engine:
-        eng = self.engine("bf16" if use_fp16 else "fp32")
+        # use_fp16=True: the model's 2-byte engine - fp16 when it was built with precision="fp16", bf16 otherwise
+        eng = self.engine(("fp16" if self.precision == "fp16" else "bf16") if use_fp16 else "fp32")
         if batch > eng.max_batch:
             eng.reserve_batch(batch)
         return eng

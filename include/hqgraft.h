@@ -39,11 +39,18 @@ enum hq_status {
 enum hq_cond_kind { HQ_COND_CLS = 0, HQ_COND_TXT = 1, HQ_COND_UNCOND = 2 };
 
 /* HQ_PREC_BF16: bf16 weights / GEMM inputs / KV cache, fp32 accumulate, residual, LayerNorm, softmax
- *               (tcgen05 + TMA GEMMs) - what `use_fp16=True` selects in the reference
- *               (torch.cuda.amp.autocast, hierarchical_ar.py:445).
+ *               (tcgen05 + TMA GEMMs) - the engine `use_fp16=True` selects by default, the same split as the
+ *               reference's fp16 autocast (torch.cuda.amp.autocast, hierarchical_ar.py:445) with bf16 for fp16.
  * HQ_PREC_FP32: everything fp32 on CUDA cores - the reference's `use_fp16=False`; used for the
- *               bit-exact greedy parity tests. */
-enum hq_precision { HQ_PREC_BF16 = 0, HQ_PREC_FP32 = 1 };
+ *               bit-exact greedy parity tests.
+ * HQ_PREC_F16:  the bf16 engine with IEEE fp16 as the 2-byte type - the reference's own autocast format.  Rounded to
+ *               fp16: GEMM weights, GEMM-input activations (LayerNorm outputs, attention outputs, GELU outputs), q / k / v
+ *               and the KV cache.  fp32: accumulation, biases, the residual stream, LayerNorm statistics, softmax, logits
+ *               and the sampler (the same kernels and rounding points as HQ_PREC_BF16).  No saturation or overflow
+ *               detection: an activation beyond the fp16 range (|x| > 65504) becomes inf, as under the reference's
+ *               autocast.  use_chain is ignored (no persistent chain kernel); fuse_head_sampler applies.  Libraries
+ *               older than this value reject it in hq_create (HQ_ERR_INVALID). */
+enum hq_precision { HQ_PREC_BF16 = 0, HQ_PREC_FP32 = 1, HQ_PREC_F16 = 2 };
 
 enum hq_dtype { HQ_F32 = 0, HQ_BF16 = 1, HQ_F16 = 2 };
 
@@ -84,7 +91,7 @@ typedef struct hq_config {
   int32_t use_cuda_graph;  /* 1: capture each run shape once and replay it; 0: plain stream launches */
   int32_t use_pdl;         /* 1: chain the kernels with programmatic dependent launch (prologue of kernel n+1 and
                               its first weight tiles overlap the tail of kernel n); 0: plain stream order */
-  int32_t use_chain;       /* 1 (bf16 engine, batches > 128): the depth transformer of a position
+  int32_t use_chain;       /* 1 (bf16 engine only, batches > 128): the depth transformer of a position
                               (sampling_step_depth_parallel, hierarchical_ar.py:667-719) and the GEMM / LayerNorm runs of the
                               spatial blocks execute as persistent multi-op kernels (one launch per run of dependent ops,
                               grid barrier between ops); 0: one kernel per op.  Results are bit-identical either way. */
@@ -95,7 +102,7 @@ typedef struct hq_config {
                               (hqvae/models/stage2/hqtransformer.py, decoding_type 'parallel-add', embedding 'transformer1'):
                               1 top + 4 middle + 16 bottom codes per position in three depth passes.  0 is read as 2. */
   int32_t vocab_mid;       /* code_levels == 3: vocab_sizes[1] (vocab_top = vocab_sizes[0], vocab_bot = vocab_sizes[2]) */
-  int32_t fuse_head_sampler; /* 1 (bf16 engine): a draw with top_k None and top_p None (the measure_throughput protocol) is made
+  int32_t fuse_head_sampler; /* 1 (bf16 and fp16 engines): a draw with top_k None and top_p None (the measure_throughput protocol) is made
                               inside the head GEMM's epilogue - exact two-stage categorical sampling over 32-column chunks,
                               the [rows, V] logits are never written.  Same distribution as the unfused sampler, different
                               Philox counters (so a different, equally valid stream for a given seed); greedy, top-k, top-p,
@@ -174,7 +181,7 @@ int hq_reserve_batch(hq_ctx* ctx, int max_batch);
 int hq_max_batch(const hq_ctx* ctx);
 
 /* Copies one parameter into the engine layout (q/k/v fused to [3D, D]; GEMM weights cast to bf16 in
- * HQ_PREC_BF16).  `name` is the reference state_dict key without the 'stage2.' prefix, e.g.
+ * HQ_PREC_BF16 and to fp16 in HQ_PREC_F16, from fp32, bf16 or fp16 sources; everything else stays fp32).  `name` is the reference state_dict key without the 'stage2.' prefix, e.g.
  * "blocks.3.attn.query.weight", "depths.0.mlp.2.bias", "tok_emb_top.weight", "sos_depth", "head_bot.weight"
  * (module definitions hierarchical_ar.py:63-209, layers.py:43-52, 290-317).
  * Stands behind `load_state_dict(strict=True)` (sampling_hqmodel.py:79): unknown names and wrong
@@ -200,7 +207,7 @@ int hq_run_host(hq_ctx* ctx, const hq_run_args* args);
 int64_t hq_last_launch_count(const hq_ctx* ctx);
 
 /* Launches of the persistent chain kernel (hq_config.use_chain) enqueued or captured since hq_create; 0 means every op
- * ran as a kernel of its own (batch <= 128, fp32 engine, use_chain == 0). */
+ * ran as a kernel of its own (batch <= 128, fp32 or fp16 engine, use_chain == 0). */
 int64_t hq_chain_launch_count(const hq_ctx* ctx);
 
 /* Bytes of device memory owned by the ctx (weights + KV cache + workspaces). */
@@ -208,22 +215,22 @@ size_t hq_device_bytes(const hq_ctx* ctx);
 
 /* ---- test / measurement hooks (used by tests/ and bench.py, not by the sampling entry points) ---- */
 
-/* C[M,N] = A[M,K] * W[N,K]^T through the same tcgen05/TMA kernels the sampler uses (prec == HQ_PREC_BF16,
- * A and W bf16) or the fp32 CUDA-core kernel (HQ_PREC_FP32, A and W fp32); C fp32; device pointers.
+/* C[M,N] = A[M,K] * W[N,K]^T through the same tcgen05/TMA kernels the sampler uses (prec == HQ_PREC_BF16 / HQ_PREC_F16,
+ * A and W bf16 / fp16) or the fp32 CUDA-core kernel (HQ_PREC_FP32, A and W fp32); C fp32; device pointers.
  * tile: 0 = the engine's own choice; 32/64/96/128/192/256 = CTA-pair kernel with that tile width;
  * -64 / -128 = single-CTA kernel. */
 int hq_debug_gemm(int prec, const void* A, const void* W, float* C, int M, int N, int K, int tile, void* stream);
 
 /* Fused epilogue of one hq_debug_gemm_epi launch (the sampler's EpiParams).  Device pointers; q, kdst, vdst, vdup and out
- * in the precision's activation type (bf16 | fp32), bias, x and outf fp32. */
+ * in the precision's activation type (bf16 | fp16 | fp32), bias, x and outf fp32. */
 typedef struct hq_debug_epi {
   int32_t epi;          /* 0 QKV, 1 RESID, 2 GELU, 3 F32 (the sampler's EPI_* values) */
-  int32_t tile;         /* as hq_debug_gemm's `tile` (bf16 only; the fp32 engine has one kernel: 0) */
+  int32_t tile;         /* as hq_debug_gemm's `tile` (bf16 / fp16; the fp32 engine has one kernel: 0) */
   int32_t ks1;          /* 1: one 64-wide k-block per ring stage even where the engine would stage two */
   int32_t D, sec0, rpb, t_stride, t0;   /* QKV: column n is section sec0 + n / D (0 q, 1 k, 2 v); row m goes to q[m] and
                                            to cache row (m / rpb) * t_stride + t0 + m % rpb of kdst / vdst */
   int32_t w_row_off;    /* the product uses W rows w_row_off .. w_row_off + N - 1 */
-  int32_t ldo, splits;  /* F32: row stride of outf; K slices, slice s writes outf + s * split_stride (bf16 only) */
+  int32_t ldo, splits;  /* F32: row stride of outf; K slices, slice s writes outf + s * split_stride (bf16 / fp16 only) */
   int32_t reserved;
   uint64_t split_stride;
   const float* bias;    /* [N] or NULL; QKV / RESID / GELU */
@@ -243,7 +250,7 @@ int hq_debug_gemm_epi(int prec, const void* A, const void* W, int w_rows, int M,
                       void* stream);
 
 /* The sampler's LayerNorm launch: out[r * out_mul] = LN(x[(r / in_group) * in_mul + in_off + r % in_group]) * gamma + beta
- * (+ add), rows r < rows, out bf16 (prec_out == HQ_PREC_BF16) or fp32.  n_fold > 0: x row += fold_bias + the n_fold
+ * (+ add), rows r < rows, out bf16 (prec_out == HQ_PREC_BF16), fp16 (HQ_PREC_F16) or fp32.  n_fold > 0: x row += fold_bias + the n_fold
  * partial sums fold + s * fold_stride (same row index), written back before the normalisation.  fp32 device pointers. */
 int hq_debug_layernorm(int prec_out, float* x, const float* gamma, const float* beta, const float* add, void* out, int rows,
                        int D, int in_group, int in_mul, int in_off, int out_mul, const float* fold, int n_fold,
@@ -259,8 +266,8 @@ int hq_debug_sample(const float* logits, int R, int V, float temperature, int to
                     int64_t* out_codes, float* out_probs /* optional [R, V] */, void* stream);
 
 /* Single-query attention of B rows over `n_keys` cached keys through the kernels the sampler uses: q / out [B, D],
- * K / V [B, t_stride, D] with D = n_heads * 64, device pointers in the precision's activation type (bf16 / fp32).
- * variant: 0 = the engine's choice (bf16: persistent ldmatrix/mma kernel), 1 = the scalar bulk-staged kernel. */
+ * K / V [B, t_stride, D] with D = n_heads * 64, device pointers in the precision's activation type (bf16 / fp16 / fp32).
+ * variant: 0 = the engine's choice (bf16 / fp16: persistent ldmatrix/mma kernel), 1 = the scalar bulk-staged kernel. */
 int hq_debug_attention(int prec, const void* q, const void* K, const void* V, void* out, int B, int n_heads,
                        int t_stride, int n_keys, int variant, void* stream);
 
