@@ -6,11 +6,11 @@ import os
 
 PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(PKG_DIR, "libhqgraft.so")
-ABI_VERSION = 8
+ABI_VERSION = 9
 
 HQ_OK = 0
 HQ_COND_CLS, HQ_COND_TXT, HQ_COND_UNCOND = 0, 1, 2
-HQ_PREC_BF16, HQ_PREC_FP32, HQ_PREC_F16 = 0, 1, 2
+HQ_PREC_BF16, HQ_PREC_FP32, HQ_PREC_F16, HQ_PREC_TF32 = 0, 1, 2, 3
 HQ_PREC = {"bf16": HQ_PREC_BF16, "fp32": HQ_PREC_FP32, "fp16": HQ_PREC_F16}
 HQ_F32, HQ_BF16, HQ_F16 = 0, 1, 2
 HQ_MODEL = {"parallel": 0, "top2bot": 1, "bidirectional": 2}
@@ -51,7 +51,7 @@ class HQDebugEpi(C.Structure):
 class HQS1Config(C.Structure):
     _fields_ = [("embed_dim", C.c_int32), ("n_embed", C.c_int32), ("z_channels", C.c_int32), ("resolution", C.c_int32),
                 ("ch", C.c_int32), ("ch_mult", C.c_int32 * 8), ("n_levels", C.c_int32), ("num_res_blocks", C.c_int32),
-                ("attn_resolution", C.c_int32), ("out_ch", C.c_int32)]
+                ("attn_resolution", C.c_int32), ("out_ch", C.c_int32), ("precision", C.c_int32)]
 
 
 # every symbol include/hqgraft.h declares: name -> (restype, argtypes)
@@ -101,6 +101,8 @@ PROTOTYPES = {
     "hq_s1_params_complete": (C.c_int, [C.c_void_p]),
     "hq_s1_decode_codes": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "hq_s1_last_conv_flops": (C.c_double, [C.c_void_p]),
+    "hq_debug_s1_conv": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                                   C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
 }
 
 _lib = None

@@ -180,6 +180,15 @@ __host__ __device__ constexpr uint32_t umma_idesc(int M, int N) {
   static_assert(std::is_same<AT, bf16>::value || std::is_same<AT, f16>::value, "kind::f16 takes bf16 or fp16 operands");
   return std::is_same<AT, bf16>::value ? umma_idesc_bf16(M, N) : umma_idesc_f16(M, N);
 }
+// Instruction descriptor for kind::tf32: a_format = b_format = TF32 (2), both K-major, fp32 accumulate.  The operands are
+// fp32 in memory; the tensor core reads the sign, exponent and top 10 mantissa bits.
+__host__ __device__ constexpr uint32_t umma_idesc_tf32(int M, int N) {
+  return (1u << 4)                               // c_format = F32
+         | (2u << 7)                             // a_format = TF32
+         | (2u << 10)                            // b_format = TF32
+         | (static_cast<uint32_t>(N >> 3) << 17) // n_dim
+         | (static_cast<uint32_t>(M >> 4) << 24);// m_dim
+}
 
 // ------------------------------------------------------------------------------------------------
 // Kernel timeline tracing (hq_trace_run): every loop kernel takes a launch id as its first parameter; when it is
@@ -479,6 +488,18 @@ __device__ __forceinline__ void umma_bf16_2sm(uint32_t tmem_d, uint64_t desc_a, 
       ".reg .pred p;\n"
       "setp.ne.b32 p, %4, 0;\n"
       "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n"
+      "}\n" ::"r"(tmem_d),
+      "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+// The same with tf32 x tf32 -> fp32 (kind::tf32, K = 8 per instruction: 32 bytes of a K-major row, as K = 16 of bf16)
+__device__ __forceinline__ void umma_tf32_2sm(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
+                                              uint32_t accumulate) {
+  asm volatile(
+      "{\n"
+      ".reg .pred p;\n"
+      "setp.ne.b32 p, %4, 0;\n"
+      "tcgen05.mma.cta_group::2.kind::tf32 [%0], %1, %2, %3, p;\n"
       "}\n" ::"r"(tmem_d),
       "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
       : "memory");

@@ -620,6 +620,10 @@ static int reserve_alloc(hq_ctx* ctx, int max_batch) {
 
 static int create_impl(hq_ctx* ctx, const hq_config* cfg, int device, int max_batch) {
   int rc;
+  if (cfg->precision == HQ_PREC_TF32) {
+    set_err(ctx, "HQ_PREC_TF32 is a stage-1 decoder precision (hq_s1_config); the sampler runs in bf16, fp16 or fp32");
+    return HQ_ERR_INVALID;
+  }
   if ((rc = check_device(ctx, device))) return rc;
   HQ_CUDA(ctx, cudaSetDevice(device));
   ctx->cfg = *cfg;

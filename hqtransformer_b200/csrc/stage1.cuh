@@ -10,16 +10,43 @@
 // zero-filled by TMA - against the weight stored [Cout, 9 Cin] tap-major.  Outputs are computed for every padded position
 // and the epilogue keeps only interior pixels, so borders stay zero.  The residual stream is fp32 (as in the sampler);
 // GroupNorm (fp32 statistics, deterministic two-level reduction) writes the bf16 GEMM input.
+//
+// Operand type T.  The kernels that write or read convolution operands are templates over T:
+//   bf16  (the default): kind::f16 MMAs; every convolution input and weight rounded to bf16 (nearest-even); q / k / v bf16.
+//   float (precision tf32, what the reference computes: decode_code runs outside autocast and cuDNN runs its convolutions
+//         in TF32): kind::tf32 MMAs with fp32 accumulation in TMEM.  Every convolution input - the codebook gather and its
+//         PixelShuffle, the GroupNorm(+swish) output, the resample copy of x (nin_shortcut and upsample inputs), the
+//         attention output (proj_out input) - and every conv weight is stored as fp32 rounded to TF32 with round-to-nearest,
+//         ties away from zero (tf32_rna): the tensor core never sees low mantissa bits, so no result depends on how it treats
+//         them.  The fused q | k | v convolution writes UNROUNDED fp32 and the AttnBlock core runs in fp32 on CUDA cores
+//         (s1_attn_kernel<float>; PyTorch's default bmm does not use TF32).
+// A 128-byte swizzled k-block row holds 64 bf16 or 32 fp32: the shared-memory geometry, stage bytes, swizzle and the
+// descriptor advance per MMA (32 bytes: K = 16 bf16 or K = 8 tf32) are the same for both.
 #pragma once
 
 #include "chain.cuh"
 
 namespace hq {
 
+// fp32 -> TF32 (sign, 8-bit exponent, 10-bit mantissa) with round-to-nearest, ties away from zero; the low 13 bits are
+// cleared whatever the conversion leaves in them.
+__device__ __forceinline__ float tf32_rna(float v) {
+  uint32_t u;
+  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(u) : "f"(v));
+  return __uint_as_float(u & 0xffffe000u);
+}
+
+// One fp32 value as a convolution operand of type T (bf16: nearest-even; float: TF32, ties away)
+template <typename T> __device__ __forceinline__ T s1_round(float v);
+template <> __device__ __forceinline__ bf16 s1_round<bf16>(float v) { return __float2bfloat16_rn(v); }
+template <> __device__ __forceinline__ float s1_round<float>(float v) { return tf32_rna(v); }
+
 // ------------------------------------------------------------------------------------------------
 // implicit-GEMM convolution on CTA pairs (tcgen05, cta_group::2): 256 padded positions x bn output channels per tile
 // ------------------------------------------------------------------------------------------------
-enum { S1_OUT_F32 = 0, S1_OUT_BF16 = 1, S1_OUT_IMAGE = 2 };
+// S1_OUT_ACT: a T matrix - bf16 rounded to nearest-even, or UNROUNDED fp32 in the tf32 instantiation (its one user, the
+// q | k | v convolution, feeds the fp32 attention core)
+enum { S1_OUT_F32 = 0, S1_OUT_ACT = 1, S1_OUT_IMAGE = 2 };
 
 struct ConvParams {
   int R;            // padded positions in total (B * Hp * Wp) = rows of the A matrix
@@ -32,9 +59,11 @@ struct ConvParams {
   const float* bias;    // [CoutPad]
   const float* res;     // optional fp32 residual [R, ldo] (mode 0), may alias outf
   float* outf;          // mode 0: fp32 [R, ldo]; mode 2: image [B, cout, H, W] fp32
-  bf16* outb;           // mode 1: bf16 [R, ldo]
+  void* outb;           // mode 1: T [R, ldo]
 };
 
+// T = bf16 (kind::f16) or float (kind::tf32; operands already rounded to TF32)
+template <typename T>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(CH_THREADS, 1)
 conv_tc2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmW, ConvParams p) {
 #if defined(__CUDA_ARCH__)
@@ -56,7 +85,8 @@ conv_tc2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
   const int bn = p.bn;
   const int nt = p.CoutPad / bn, mt = (p.R + 255) / 256;
   const int total_tiles = nt * mt;
-  const int kpt = p.Cin / 64;                       // k-blocks per tap
+  constexpr int KB = 128 / static_cast<int>(sizeof(T));   // elements per 128-byte k-block row
+  const int kpt = p.Cin / KB;                       // k-blocks per tap
   const int num_kb = p.taps * kpt;
 
   if (warp == 0 && lane == 0) {
@@ -101,15 +131,15 @@ conv_tc2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
         mbar_wait(&empty_bar[s], ((g / CH_STAGES) & 1) ^ 1);
         if (elect_one()) {
           if (leader) mbar_arrive_expect_tx(&full_bar[s], stage_tx);
-          tma_load_2d_2sm(smem + s * CH_STAGE_BYTES, &tmA, &full_bar[s], kc * 64, m0 + off);
-          tma_load_2d_2sm(smem + s * CH_STAGE_BYTES + CH_A_BYTES, &tmW, &full_bar[s], kb * 64, wrow);
+          tma_load_2d_2sm(smem + s * CH_STAGE_BYTES, &tmA, &full_bar[s], kc * KB, m0 + off);
+          tma_load_2d_2sm(smem + s * CH_STAGE_BYTES + CH_A_BYTES, &tmW, &full_bar[s], kb * KB, wrow);
         }
       }
     }
   } else if (warp == 1) {
     if (leader) {
       // ---- MMA issuer (warp-uniform loop, the elected lane issues the MMAs and their commits) ----
-      const uint32_t idesc = umma_idesc_bf16(256, bn);
+      const uint32_t idesc = std::is_same<T, float>::value ? umma_idesc_tf32(256, bn) : umma_idesc_bf16(256, bn);
       const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);
       uint32_t g = 0, it = 0;
       for (int tile = pair; tile < total_tiles; tile += npairs, ++it) {
@@ -125,9 +155,14 @@ conv_tc2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
             const uint64_t da = umma_smem_desc_sw128(smem_u32(smem + s * CH_STAGE_BYTES));
             const uint64_t db = umma_smem_desc_sw128(smem_u32(smem + s * CH_STAGE_BYTES + CH_A_BYTES));
 #pragma unroll
-            for (int k = 0; k < 4; ++k)
-              umma_bf16_2sm(acc, da + static_cast<uint64_t>(2 * k), db + static_cast<uint64_t>(2 * k), idesc,
-                            (kb > 0 || k > 0) ? 1u : 0u);
+            for (int k = 0; k < 4; ++k) {
+              if constexpr (std::is_same<T, float>::value)
+                umma_tf32_2sm(acc, da + static_cast<uint64_t>(2 * k), db + static_cast<uint64_t>(2 * k), idesc,
+                              (kb > 0 || k > 0) ? 1u : 0u);
+              else
+                umma_bf16_2sm(acc, da + static_cast<uint64_t>(2 * k), db + static_cast<uint64_t>(2 * k), idesc,
+                              (kb > 0 || k > 0) ? 1u : 0u);
+            }
             umma_commit_2sm(&empty_bar[s], 0x3);
           }
         }
@@ -206,12 +241,16 @@ conv_tc2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
                 v.x += a.x; v.y += a.y; v.z += a.z; v.w += a.w;
               }
               *dst = v;
-            } else if (p.mode == S1_OUT_BF16) {
-              uint2 u;
-              __nv_bfloat162 h0 = __floats2bfloat162_rn(v.x, v.y), h1 = __floats2bfloat162_rn(v.z, v.w);
-              u.x = *reinterpret_cast<uint32_t*>(&h0);
-              u.y = *reinterpret_cast<uint32_t*>(&h1);
-              *reinterpret_cast<uint2*>(p.outb + row_off[r8] + col) = u;
+            } else if (p.mode == S1_OUT_ACT) {
+              if constexpr (std::is_same<T, float>::value) {
+                *reinterpret_cast<float4*>(static_cast<float*>(p.outb) + row_off[r8] + col) = v;
+              } else {
+                uint2 u;
+                __nv_bfloat162 h0 = __floats2bfloat162_rn(v.x, v.y), h1 = __floats2bfloat162_rn(v.z, v.w);
+                u.x = *reinterpret_cast<uint32_t*>(&h0);
+                u.y = *reinterpret_cast<uint32_t*>(&h1);
+                *reinterpret_cast<uint2*>(static_cast<bf16*>(p.outb) + row_off[r8] + col) = u;
+              }
             } else {
               const float vv[4] = {v.x, v.y, v.z, v.w};
               const size_t plane = static_cast<size_t>(H) * W;
@@ -244,13 +283,14 @@ conv_tc2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
 // ------------------------------------------------------------------------------------------------
 // codes -> input of post_quant_conv_b (generator.py:316-319): channels [0, E) = PixelShuffle(2) of the top entry (E*4 wide:
 // out[c, y, x] = in[4c + 2 (y % 2) + (x % 2), y / 2, x / 2]), channels [E, 2E) = the bottom entry.  One CTA per bottom pixel.
+template <typename T>
 __global__ void __launch_bounds__(256)
 s1_quant_kernel(const int64_t* __restrict__ code_t, const int64_t* __restrict__ code_b, const float* __restrict__ E_t,
-                const float* __restrict__ E_b, bf16* __restrict__ out, int E, int hb /*bottom grid side*/, int n_embed) {
+                const float* __restrict__ E_b, T* __restrict__ out, int E, int hb /*bottom grid side*/, int n_embed) {
   const int Wp = hb + 2;
   const int pp = blockIdx.x;                   // padded pixel: b * Wp * Wp + yp * Wp + xp
   const int b = pp / (Wp * Wp), q = pp % (Wp * Wp), y = q / Wp - 1, x = q % Wp - 1;
-  bf16* o = out + static_cast<size_t>(pp) * 2 * E;
+  T* o = out + static_cast<size_t>(pp) * 2 * E;
   const int ht = hb / 2;
   int64_t ct = -1, cb = -1;
   if (y >= 0 && y < hb && x >= 0 && x < hb) {
@@ -258,14 +298,14 @@ s1_quant_kernel(const int64_t* __restrict__ code_t, const int64_t* __restrict__ 
     cb = code_b[(static_cast<size_t>(b) * hb + y) * hb + x];
   }
   if (ct < 0 || ct >= n_embed || cb < 0 || cb >= n_embed) {      // border (or an out-of-range code: the host validates)
-    for (int c = threadIdx.x; c < 2 * E; c += blockDim.x) o[c] = __float2bfloat16_rn(0.f);
+    for (int c = threadIdx.x; c < 2 * E; c += blockDim.x) o[c] = s1_round<T>(0.f);
     return;
   }
   const float* et = E_t + static_cast<size_t>(ct) * 4 * E + 2 * (y & 1) + (x & 1);
   const float* eb = E_b + static_cast<size_t>(cb) * E;
   for (int c = threadIdx.x; c < E; c += blockDim.x) {
-    o[c] = __float2bfloat16_rn(et[4 * c]);
-    o[E + c] = __float2bfloat16_rn(eb[c]);
+    o[c] = s1_round<T>(et[4 * c]);
+    o[E + c] = s1_round<T>(eb[c]);
   }
 }
 
@@ -340,12 +380,13 @@ s1_gn_stats_kernel(const float* __restrict__ x, double* __restrict__ part, float
 // x * sigmoid(x) (layers.py:12-14) with the fast exponential / division: ~1e-6 relative, far below the bf16 rounding of the output
 __device__ __forceinline__ float swish_f(float v) { return __fdividef(v, 1.0f + __expf(-v)); }
 
-// y = GroupNorm(x) (optionally * sigmoid) as bf16; EVERY padded position is written, the border with zeros (the buffers are
+// y = GroupNorm(x) (optionally * sigmoid) as T; EVERY padded position is written, the border with zeros (the buffers are
 // reused at other resolutions: a 3x3 convolution must find zeros around its input).  One CTA per padded row (b, y), four
 // float4 loads in flight per thread.
+template <typename T>
 __global__ void __launch_bounds__(256)
 s1_gn_apply_kernel(const float* __restrict__ x, const float2* __restrict__ stat, const float* __restrict__ gamma,
-                   const float* __restrict__ beta, bf16* __restrict__ out, int Hp, int Wp, int C, int swish) {
+                   const float* __restrict__ beta, T* __restrict__ out, int Hp, int Wp, int C, int swish) {
   const int b = blockIdx.y, y = blockIdx.x;
   const int H = Hp - 2, W = Wp - 2, cg = C / 32;
   __shared__ float s_mean[32], s_rstd[32];
@@ -373,6 +414,7 @@ s1_gn_apply_kernel(const float* __restrict__ x, const float2* __restrict__ stat,
     for (int k = 0; k < 4; ++k) {
       if (off[k] < 0) continue;
       uint2 u = make_uint2(0u, 0u);
+      float4 f = make_float4(0.f, 0.f, 0.f, 0.f);
       if (in[k]) {
         const int c = (i0 + k * 256) % c4 * 4;
         const float4 ga = *reinterpret_cast<const float4*>(gamma + c);
@@ -382,43 +424,56 @@ s1_gn_apply_kernel(const float* __restrict__ x, const float2* __restrict__ stat,
         float o0 = (v[k].x - s_mean[g0]) * s_rstd[g0] * ga.x + be.x, o1 = (v[k].y - s_mean[g1]) * s_rstd[g1] * ga.y + be.y;
         float o2 = (v[k].z - s_mean[g2]) * s_rstd[g2] * ga.z + be.z, o3 = (v[k].w - s_mean[g3]) * s_rstd[g3] * ga.w + be.w;
         if (swish) { o0 = swish_f(o0); o1 = swish_f(o1); o2 = swish_f(o2); o3 = swish_f(o3); }
-        __nv_bfloat162 h0 = __floats2bfloat162_rn(o0, o1), h1 = __floats2bfloat162_rn(o2, o3);
-        u.x = *reinterpret_cast<uint32_t*>(&h0);
-        u.y = *reinterpret_cast<uint32_t*>(&h1);
+        if constexpr (std::is_same<T, float>::value) {
+          f = make_float4(tf32_rna(o0), tf32_rna(o1), tf32_rna(o2), tf32_rna(o3));
+        } else {
+          __nv_bfloat162 h0 = __floats2bfloat162_rn(o0, o1), h1 = __floats2bfloat162_rn(o2, o3);
+          u.x = *reinterpret_cast<uint32_t*>(&h0);
+          u.y = *reinterpret_cast<uint32_t*>(&h1);
+        }
       }
-      *reinterpret_cast<uint2*>(out + base + off[k]) = u;
+      if constexpr (std::is_same<T, float>::value) *reinterpret_cast<float4*>(out + base + off[k]) = f;
+      else *reinterpret_cast<uint2*>(out + base + off[k]) = u;
     }
   }
 }
 
-// nearest-neighbour 2x upsampling (Upsample, layers.py:49-52) fp32 [B, H+2, W+2, C] -> bf16 [B, 2H+2, 2W+2, C]: the input
-// of the level's upsample convolution.  up = 1: plain fp32 -> bf16 copy of the interior (input of a nin_shortcut 1x1 conv).
+// nearest-neighbour 2x upsampling (Upsample, layers.py:49-52) fp32 [B, H+2, W+2, C] -> T [B, 2H+2, 2W+2, C]: the input
+// of the level's upsample convolution.  up = 1: plain fp32 -> T copy of the interior (input of a nin_shortcut 1x1 conv).
+template <typename T>
 __global__ void __launch_bounds__(256)
-s1_resample_kernel(const float* __restrict__ x, bf16* __restrict__ out, int H, int W, int C, int up) {
+s1_resample_kernel(const float* __restrict__ x, T* __restrict__ out, int H, int W, int C, int up) {
   const int b = blockIdx.y, yp = blockIdx.x;           // output padded row 0 .. up*H+1
   const int Ho = up * H, Wo = up * W, c4 = C / 4;
-  bf16* dst = out + ((static_cast<size_t>(b) * (Ho + 2) + yp) * (Wo + 2)) * C;
+  T* dst = out + ((static_cast<size_t>(b) * (Ho + 2) + yp) * (Wo + 2)) * C;
   const bool row_in = yp >= 1 && yp <= Ho;
   const float* src = x + ((static_cast<size_t>(b) * (H + 2) + (row_in ? (yp - 1) / up + 1 : 0)) * (W + 2)) * C;
   for (int i = threadIdx.x; i < (Wo + 2) * c4; i += blockDim.x) {
     const int xp = i / c4, c = (i % c4) * 4;
     uint2 u = make_uint2(0u, 0u);
+    float4 f = make_float4(0.f, 0.f, 0.f, 0.f);
     if (row_in && xp >= 1 && xp <= Wo) {
       const float4 v = *reinterpret_cast<const float4*>(src + static_cast<size_t>((xp - 1) / up + 1) * C + c);
-      __nv_bfloat162 h0 = __floats2bfloat162_rn(v.x, v.y), h1 = __floats2bfloat162_rn(v.z, v.w);
-      u.x = *reinterpret_cast<uint32_t*>(&h0);
-      u.y = *reinterpret_cast<uint32_t*>(&h1);
+      if constexpr (std::is_same<T, float>::value) {
+        f = make_float4(tf32_rna(v.x), tf32_rna(v.y), tf32_rna(v.z), tf32_rna(v.w));
+      } else {
+        __nv_bfloat162 h0 = __floats2bfloat162_rn(v.x, v.y), h1 = __floats2bfloat162_rn(v.z, v.w);
+        u.x = *reinterpret_cast<uint32_t*>(&h0);
+        u.y = *reinterpret_cast<uint32_t*>(&h1);
+      }
     }
-    *reinterpret_cast<uint2*>(dst + static_cast<size_t>(xp) * C + c) = u;
+    if constexpr (std::is_same<T, float>::value) *reinterpret_cast<float4*>(dst + static_cast<size_t>(xp) * C + c) = f;
+    else *reinterpret_cast<uint2*>(dst + static_cast<size_t>(xp) * C + c) = u;
   }
 }
 
 // AttnBlock core (layers.py:170-183): single-head attention over the N = H W pixels of an image, C channels, scale C^-1/2.
-// qkv: bf16 padded [B, Hp, Wp, 3C] (q | k | v along channels); out: bf16 padded [B, Hp, Wp, C] (interior only).
-// One CTA (256 threads) per (image, tile of S1_ATT_Q queries): scores in shared memory, full softmax, then P V.
+// qkv: T padded [B, Hp, Wp, 3C] (q | k | v along channels); out: T padded [B, Hp, Wp, C] (interior only), a proj_out input
+// (s1_round).  One CTA (256 threads) per (image, tile of S1_ATT_Q queries): scores in shared memory, full softmax, then P V.
 constexpr int S1_ATT_Q = 8;
+template <typename T>
 __global__ void __launch_bounds__(256)
-s1_attn_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ out, int H, int W, int C) {
+s1_attn_kernel(const T* __restrict__ qkv, T* __restrict__ out, int H, int W, int C) {
   extern __shared__ float s1_att_smem[];
   const int N = H * W, Wp = W + 2;
   float* sq = s1_att_smem;                     // [S1_ATT_Q][C]
@@ -430,12 +485,12 @@ s1_attn_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ out, int H, int 
   auto prow = [&](int n) { return img + static_cast<size_t>(n / W + 1) * Wp + (n % W + 1); };
   for (int i = tid; i < S1_ATT_Q * C; i += blockDim.x) {
     const int qi = i / C, c = i % C, n = q0 + qi;
-    sq[i] = n < N ? __bfloat162float(qkv[prow(n) * 3 * C + c]) : 0.f;
+    sq[i] = n < N ? ActT<T>::to_f(qkv[prow(n) * 3 * C + c]) : 0.f;
   }
   __syncthreads();
   const float scale = rsqrtf(static_cast<float>(C));
   for (int j = tid; j < N; j += blockDim.x) {
-    const bf16* kr = qkv + prow(j) * 3 * C + C;
+    const T* kr = qkv + prow(j) * 3 * C + C;
     float acc[S1_ATT_Q];
 #pragma unroll
     for (int qi = 0; qi < S1_ATT_Q; ++qi) acc[qi] = 0.f;
@@ -471,8 +526,13 @@ s1_attn_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ out, int H, int 
 #pragma unroll
     for (int qi = 0; qi < S1_ATT_Q; ++qi) a0[qi] = a1[qi] = 0.f;
     for (int j = 0; j < N; ++j) {
-      const __nv_bfloat162 v2 = *reinterpret_cast<const __nv_bfloat162*>(qkv + prow(j) * 3 * C + 2 * C + c);
-      const float2 vf = __bfloat1622float2(v2);
+      float2 vf;
+      if constexpr (std::is_same<T, float>::value) {
+        vf = *reinterpret_cast<const float2*>(qkv + prow(j) * 3 * C + 2 * C + c);
+      } else {
+        const __nv_bfloat162 v2 = *reinterpret_cast<const __nv_bfloat162*>(qkv + prow(j) * 3 * C + 2 * C + c);
+        vf = __bfloat1622float2(v2);
+      }
 #pragma unroll
       for (int qi = 0; qi < S1_ATT_Q; ++qi) {
         const float w = sp[qi * N + j];
@@ -485,7 +545,10 @@ s1_attn_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ out, int H, int 
       const int n = q0 + qi;
       if (n < N) {
         const float inv = red[qi][0];
-        *reinterpret_cast<__nv_bfloat162*>(out + prow(n) * C + c) = __floats2bfloat162_rn(a0[qi] * inv, a1[qi] * inv);
+        if constexpr (std::is_same<T, float>::value)
+          *reinterpret_cast<float2*>(out + prow(n) * C + c) = make_float2(tf32_rna(a0[qi] * inv), tf32_rna(a1[qi] * inv));
+        else
+          *reinterpret_cast<__nv_bfloat162*>(out + prow(n) * C + c) = __floats2bfloat162_rn(a0[qi] * inv, a1[qi] * inv);
       }
     }
   }
@@ -686,14 +749,16 @@ s1_attn_mma_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ out, int H, 
 #endif
 }
 
-// conv weight [Cout, Cin, k, k] (fp32 / bf16 / fp16 source already converted to fp32) -> bf16 [CoutPad, k*k*Cin] tap-major
-__global__ void s1_pack_weight_kernel(const float* __restrict__ w, bf16* __restrict__ out, int Cout, int Cin, int taps) {
+// conv weight [Cout, Cin, k, k] (fp32 / bf16 / fp16 source already converted to fp32) -> T [CoutPad, k*k*Cin] tap-major
+// (bf16, or fp32 rounded to TF32)
+template <typename T>
+__global__ void s1_pack_weight_kernel(const float* __restrict__ w, T* __restrict__ out, int Cout, int Cin, int taps) {
   const size_t n = static_cast<size_t>(Cout) * Cin * taps;
   for (size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x; i < n; i += static_cast<size_t>(gridDim.x) * blockDim.x) {
     const int t = static_cast<int>(i % taps);
     const int ci = static_cast<int>((i / taps) % Cin);
     const int co = static_cast<int>(i / (static_cast<size_t>(taps) * Cin));
-    out[(static_cast<size_t>(co) * taps + t) * Cin + ci] = __float2bfloat16_rn(w[i]);
+    out[(static_cast<size_t>(co) * taps + t) * Cin + ci] = s1_round<T>(w[i]);
   }
 }
 

@@ -45,6 +45,7 @@ class Experiment:                      # measure_throughput/__main__.py:34-48
     stage1: int = 1                    # extension: 1 = build and time the stage-1 decoder too
     decode_chunks: int = 1             # extension: chunks the batch is decoded in (batch_size = the reference's protocol)
     precision: str = "bf16"            # extension: engine of use_fp16=True - "bf16", or "fp16" (the reference's autocast type)
+    stage1_precision: str = "bf16"     # extension: stage-1 decoder format - "bf16", or "tf32" (the reference's decode format)
 
 
 def parse_cli(argv) -> Experiment:
@@ -66,11 +67,11 @@ def parse_cli(argv) -> Experiment:
 
 
 def load_model(result_path: str, device="cuda", max_batch: int = 50, with_stage1: bool = True,
-               precision: str = "bf16") -> ImageGPT2:
+               precision: str = "bf16", stage1_precision: str = "bf16") -> ImageGPT2:
     """:25-31 - config only, no checkpoint: random-init weights of the named architecture."""
     dev = torch.device(device)
     return ImageGPT2.from_config(result_path, device=dev.index or 0, precision=precision, max_batch=max_batch,
-                                 with_stage1=with_stage1, stage1_max_batch=min(max_batch, 32))
+                                 with_stage1=with_stage1, stage1_max_batch=min(max_batch, 32), stage1_precision=stage1_precision)
 
 
 def main(args: Experiment):
@@ -80,8 +81,11 @@ def main(args: Experiment):
     device = torch.device("cuda")
     if args.precision not in ("bf16", "fp16"):
         raise SystemExit(f"precision={args.precision!r}: bf16 or fp16 (the engines use_fp16=True selects)")
+    if args.stage1_precision not in ("bf16", "tf32"):
+        raise SystemExit(f"stage1_precision={args.stage1_precision!r}: bf16 or tf32")
     model_ar = load_model(args.model_path, device, args.batch_size,
-                          with_stage1=bool(args.stage1) and args.code_levels == 2, precision=args.precision).to(device).eval()
+                          with_stage1=bool(args.stage1) and args.code_levels == 2, precision=args.precision,
+                          stage1_precision=args.stage1_precision).to(device).eval()
     if (args.code_levels == 3) != hasattr(model_ar.stage2, "code_level"):
         raise SystemExit(f"code_levels={args.code_levels} does not match the model type of {args.model_path}")
     title = f"bs{args.batch_size}, sampling loops {args.warmup + 1}-{args.n_loop}"

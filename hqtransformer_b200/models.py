@@ -287,9 +287,13 @@ class iHQGPT:
 class ImageGPT2:
     """The object the scripts build from a config (hqvae/models/__init__.py:92-174): `.stage2` is the sampler.
     Stage 1 (HQ-VAE decoder) is outside this path; attach any module with the reference's
-    `decode_code(code_t [B,8,8], code_b [B,16,16])` as `.stage1` to get pixels out of `sample()`."""
+    `decode_code(code_t [B,8,8], code_b [B,16,16])` as `.stage1` to get pixels out of `sample()`.
+    `stage1_precision` ("bf16" | "tf32") selects the format of the stage-1 decoder built with `with_stage1=True`."""
 
-    def __init__(self, config, with_stage1: bool = False, stage1_max_batch: int = 16, **engine_opts) -> None:
+    def __init__(self, config, with_stage1: bool = False, stage1_max_batch: int = 16, stage1_precision: str = "bf16",
+                 **engine_opts) -> None:
+        from .stage1 import check_s1_precision
+        check_s1_precision(stage1_precision)
         self.config = config
         self.stage1 = None
         if "multilevel-hq" in config.stage2.type:               # hqvae/models/__init__.py:138-145
@@ -304,7 +308,8 @@ class ImageGPT2:
             s1 = getattr(config, "stage1", None)
             if s1 is None:
                 raise KeyError("with_stage1=True needs a `stage1` section in the config")
-            self.stage1 = HQVAEDecoder.from_stage1_config(s1, max_batch=stage1_max_batch, device=self.stage2.device)
+            self.stage1 = HQVAEDecoder.from_stage1_config(s1, max_batch=stage1_max_batch, device=self.stage2.device,
+                                                          precision=stage1_precision)
         self.use_cls_cond = config.stage2.use_cls_cond
         self.use_txt_cond = config.stage2.use_txt_cond
         self.type = config.stage2.type

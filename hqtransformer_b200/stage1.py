@@ -19,14 +19,26 @@ from . import _lib
 from ._lib import HQS1Config, check_s1
 
 _TORCH2HQ = {torch.float32: _lib.HQ_F32, torch.bfloat16: _lib.HQ_BF16, torch.float16: _lib.HQ_F16}
+# operand format of the convolutions: "bf16" (default), or "tf32" - the reference's own (decode_code runs in fp32 outside
+# autocast and cuDNN runs its convolutions in TF32); see HQ_PREC_TF32 in include/hqgraft.h
+S1_PRECISIONS = {"bf16": _lib.HQ_PREC_BF16, "tf32": _lib.HQ_PREC_TF32}
+
+
+def check_s1_precision(precision: str) -> int:
+    if precision not in S1_PRECISIONS:
+        raise ValueError(f"stage-1 precision {precision!r}: one of {sorted(S1_PRECISIONS)}")
+    return S1_PRECISIONS[precision]
 
 
 class HQVAEDecoder:
-    """`stage1` of an `ImageGPT2`: only what `decode_code` needs (codebooks, post_quant_conv_b, Decoder)."""
+    """`stage1` of an `ImageGPT2`: only what `decode_code` needs (codebooks, post_quant_conv_b, Decoder).
+    precision: "bf16" (default) or "tf32" (the reference's format: TF32 convolutions, fp32 attention and residual stream)."""
 
     def __init__(self, *, embed_dim: int = 256, n_embed: int = 8192, z_channels: int = 256, resolution: int = 256,
                  ch: int = 128, ch_mult=(1, 2, 4, 4), num_res_blocks: int = 2, attn_resolutions=(16,), out_ch: int = 3,
-                 max_batch: int = 16, device: Union[int, str, torch.device] = 0):
+                 max_batch: int = 16, device: Union[int, str, torch.device] = 0, precision: str = "bf16"):
+        prec = check_s1_precision(precision)
+        self.precision = precision
         self._lib = _lib.load()
         self._ctx = C.c_void_p()
         dev = torch.device(device) if not isinstance(device, int) else torch.device("cuda", device)
@@ -43,13 +55,13 @@ class HQVAEDecoder:
         mult = (C.c_int32 * 8)(*(list(self.ch_mult) + [0] * (8 - len(self.ch_mult))))
         cfg = HQS1Config(embed_dim=embed_dim, n_embed=n_embed, z_channels=z_channels, resolution=resolution, ch=ch,
                          ch_mult=mult, n_levels=len(self.ch_mult), num_res_blocks=num_res_blocks,
-                         attn_resolution=self.attn_resolution, out_ch=out_ch)
+                         attn_resolution=self.attn_resolution, out_ch=out_ch, precision=prec)
         check_s1(self._lib.hq_s1_create(C.byref(cfg), self.device.index, self.max_batch, C.byref(self._ctx)), None,
                  self._lib, "hq_s1_create")
 
     @classmethod
     def from_stage1_config(cls, s1, **kw) -> "HQVAEDecoder":
-        """From the `stage1` section of a reference YAML (namespace or dict)."""
+        """From the `stage1` section of a reference YAML (namespace or dict); `kw` (max_batch, device, precision) pass through."""
         get = (lambda o, k, d=None: o.get(k, d)) if isinstance(s1, dict) else (lambda o, k, d=None: getattr(o, k, d))
         if get(s1, "type") not in (None, "simrqgan2"):
             raise NotImplementedError(f"stage1.type={get(s1, 'type')!r}: only 'simrqgan2' (2-level HQ-VAE) is implemented")
@@ -195,3 +207,23 @@ class HQVAEDecoder:
             check_s1(self._lib.hq_s1_decode_codes(self._ctx, ct[lo:hi].data_ptr(), cb[lo:hi].data_ptr(), out[lo:hi].data_ptr(),
                                                   hi - lo, C.c_void_p(st)), self._ctx, self._lib, "hq_s1_decode_codes")
         return out
+
+
+def debug_s1_conv(A: torch.Tensor, weight: torch.Tensor, bias: torch.Tensor, out: torch.Tensor, mode: int, *,
+                  resid: Optional[torch.Tensor] = None, tile: int = 0) -> None:
+    """One decoder convolution through hq_debug_s1_conv (weight packing, tile planner and conv kernel of the decoder),
+    in place, synchronous.  A: padded NHWC [B, res+2, res+2, Cin], bf16 (precision bf16) or fp32 (tf32: already rounded);
+    weight fp32 [Cout, Cin, k, k]; bias fp32 [Cout].  mode 0: out fp32 [B, res+2, res+2, Cout] (+= resid, which may be out);
+    1: out in A's dtype, same layout; 2: out fp32 [B, Cout, res, res].  tile 0: the planner's width."""
+    lib = _lib.load()
+    prec = {torch.bfloat16: _lib.HQ_PREC_BF16, torch.float32: _lib.HQ_PREC_TF32}[A.dtype]
+    B, Hp, _, Cin = A.shape
+    Cout, _, k, _ = weight.shape
+    for t in (A, weight, bias, out) + ((resid,) if resid is not None else ()):
+        assert t.is_cuda and t.is_contiguous() and t.device == A.device
+    assert weight.dtype == bias.dtype == torch.float32 and out.dtype == (A.dtype if mode == 1 else torch.float32)
+    with torch.cuda.device(A.device):
+        st = torch.cuda.current_stream(A.device).cuda_stream
+        rc = lib.hq_debug_s1_conv(prec, A.data_ptr(), weight.data_ptr(), bias.data_ptr(), B, Hp - 2, Cin, Cout, k, mode,
+                                  tile, resid.data_ptr() if resid is not None else None, out.data_ptr(), C.c_void_p(st))
+        check_s1(rc, None, lib, "hq_debug_s1_conv")

@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define HQ_ABI_VERSION 8
+#define HQ_ABI_VERSION 9
 
 enum hq_status {
   HQ_OK = 0,
@@ -49,8 +49,15 @@ enum hq_cond_kind { HQ_COND_CLS = 0, HQ_COND_TXT = 1, HQ_COND_UNCOND = 2 };
  *               and the sampler (the same kernels and rounding points as HQ_PREC_BF16).  No saturation or overflow
  *               detection: an activation beyond the fp16 range (|x| > 65504) becomes inf, as under the reference's
  *               autocast.  use_chain is ignored (no persistent chain kernel); fuse_head_sampler applies.  Libraries
- *               older than this value reject it in hq_create (HQ_ERR_INVALID). */
-enum hq_precision { HQ_PREC_BF16 = 0, HQ_PREC_FP32 = 1, HQ_PREC_F16 = 2 };
+ *               older than this value reject it in hq_create (HQ_ERR_INVALID).
+ * HQ_PREC_TF32: stage-1 decoder only (hq_s1_config.precision; hq_create rejects it with HQ_ERR_INVALID) - what the
+ *               reference's decode_code computes (fp32 outside autocast, cuDNN convolutions in TF32).  Convolutions on
+ *               tcgen05 kind::tf32 with fp32 accumulation.  Rounded to TF32 (round-to-nearest, ties away from zero; stored
+ *               as fp32 with the low 13 bits zero): every convolution input - codebook gather + PixelShuffle, GroupNorm(+swish)
+ *               outputs, the copies of x that feed nin_shortcut and the upsample convolutions, attention outputs - and the
+ *               conv weights.  fp32: q / k / v (unrounded), the AttnBlock core (CUDA cores), the residual stream, GroupNorm
+ *               statistics, biases and the output image.  fp32 range throughout (no overflow at fp16's 65504). */
+enum hq_precision { HQ_PREC_BF16 = 0, HQ_PREC_FP32 = 1, HQ_PREC_F16 = 2, HQ_PREC_TF32 = 3 };
 
 enum hq_dtype { HQ_F32 = 0, HQ_BF16 = 1, HQ_F16 = 2 };
 
@@ -327,6 +334,7 @@ typedef struct hq_s1_config {
   int32_t num_res_blocks;   /* hparams.num_res_blocks */
   int32_t attn_resolution;  /* hparams.attn_resolutions[0] */
   int32_t out_ch;           /* hparams.out_ch (3) */
+  int32_t precision;        /* HQ_PREC_BF16 (0, the default: bf16 convolution inputs and weights) or HQ_PREC_TF32 */
 } hq_s1_config;
 
 typedef struct hq_s1_ctx hq_s1_ctx;
@@ -338,8 +346,8 @@ size_t hq_s1_device_bytes(const hq_s1_ctx* ctx);
 
 /* `name`: key of the reference generator's state_dict without the 'stage1.' prefix, e.g. "quantize_t.embedding",
  * "post_quant_conv_b.weight", "decoder.up.2.block.1.conv1.weight", "decoder.mid.attn_1.q.bias" (generator.py:243-250,
- * stage1/modules/layers.py:77-186, 300-383).  Only the keys decode_code reads exist; conv weights are repacked to bf16
- * [Cout, kh kw Cin].  hq_s1_params_complete: HQ_OK once all of them were loaded. */
+ * stage1/modules/layers.py:77-186, 300-383).  Only the keys decode_code reads exist; conv weights (fp32, bf16 or fp16
+ * sources) are repacked to [Cout, kh kw Cin] bf16, or fp32 rounded to TF32 under HQ_PREC_TF32.  hq_s1_params_complete: HQ_OK once all of them were loaded. */
 int hq_s1_load_param(hq_s1_ctx* ctx, const char* name, const void* data, int dtype, const int64_t* shape, int ndim,
                      int is_device);
 int hq_s1_params_complete(hq_s1_ctx* ctx);
@@ -350,6 +358,16 @@ int hq_s1_decode_codes(hq_s1_ctx* ctx, const int64_t* code_t, const int64_t* cod
 
 /* 2 * MACs of the convolutions of the last hq_s1_decode_codes call (interior pixels only): the roofline numerator. */
 double hq_s1_last_conv_flops(const hq_s1_ctx* ctx);
+
+/* Test hook: one stage-1 convolution through the decoder's own path (weight packing, tile planner, conv kernel), synchronous
+ * on `stream`, device pointers.  prec: HQ_PREC_BF16 or HQ_PREC_TF32.  A: padded NHWC input [B, res+2, res+2, Cin] in the
+ * operand type (bf16 | fp32; under HQ_PREC_TF32 the kernel reads it as TF32, so pass values already rounded), border zero;
+ * weight fp32 [Cout, Cin, k, k] (k = 1 or 3; packed and rounded as hq_s1_load_param does); bias fp32 [Cout]; Cin a
+ * multiple of 64.  mode 0: out fp32 [B, res+2, res+2, Cout], interior written, += resid (fp32, same layout, may equal
+ * out) when resid != NULL; 1: out in the operand type (fp32 unrounded under HQ_PREC_TF32), interior written; 2: out fp32
+ * image [B, Cout, res, res].  tile: 0 = the planner's width, else a multiple of 32 in [32, 256]. */
+int hq_debug_s1_conv(int prec, const void* A, const float* weight, const float* bias, int B, int res, int Cin, int Cout,
+                     int k, int mode, int tile, const float* resid, void* out, void* stream);
 
 #ifdef __cplusplus
 }
