@@ -19,11 +19,11 @@ from .config import load_config, merge_config  # noqa: E402
 from .engine import Engine, SamplingParams  # noqa: E402
 from .models import ImageGPT2, iHQGPT  # noqa: E402
 from .sampling import (codes_to_grids, cutoff_topk_logits, cutoff_topp_probs, encode_prompts,  # noqa: E402
-                       get_positional_encoding, sampling_ihqgpt, step_logits)
+                       get_positional_encoding, grids_to_codes, sampling_ihqgpt, step_logits)
 from .distributed import sampling_ihqgpt_sharded, shard_range  # noqa: E402
 from .stage1 import HQVAEDecoder  # noqa: E402
 from .hqtransformer3 import HQTransformer, sampling_hqtransformer, step_logits3  # noqa: E402
 
 __all__ = ["HQError", "Engine", "SamplingParams", "ImageGPT2", "iHQGPT", "load_config", "merge_config",
            "sampling_ihqgpt", "step_logits", "cutoff_topk_logits", "cutoff_topp_probs", "get_positional_encoding",
-           "codes_to_grids", "encode_prompts", "sampling_ihqgpt_sharded", "shard_range", "HQVAEDecoder", "HQTransformer", "sampling_hqtransformer", "step_logits3"]
+           "codes_to_grids", "grids_to_codes", "encode_prompts", "sampling_ihqgpt_sharded", "shard_range", "HQVAEDecoder", "HQTransformer", "sampling_hqtransformer", "step_logits3"]

@@ -38,7 +38,7 @@ class HQRunArgs(C.Structure):
                 ("cond", C.c_void_p), ("sos", C.c_void_p), ("given_top", C.c_void_p), ("given_bot", C.c_void_p),
                 ("codes_top", C.c_void_p), ("codes_bot", C.c_void_p), ("logits", C.c_void_p),
                 ("sampling", HQSamplingParams), ("codes_mid", C.c_void_p), ("given_mid", C.c_void_p),
-                ("shared_prefix", C.c_int32), ("reserved", C.c_int32)]
+                ("shared_prefix", C.c_int32), ("prefix_len", C.c_int32)]
 
 
 class HQDebugEpi(C.Structure):
@@ -81,6 +81,8 @@ PROTOTYPES = {
                                   C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "hq_debug_attention": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                      C.c_int, C.c_int, C.c_void_p]),
+    "hq_debug_attention_prefix": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                            C.c_int, C.c_int, C.c_void_p]),
     "hq_debug_attention_phases": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_uint64), C.c_int,
                                             C.POINTER(C.c_int), C.c_void_p]),
     "hq_debug_chain_phases": (C.c_int, [C.c_void_p, C.POINTER(HQRunArgs), C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_uint64),

@@ -139,10 +139,10 @@ static DebugSwitches read_debug_switches() {
 }
 
 struct GraphKey {
-  int B, S, p0, p1, forced_top, forced_bot, sos_override, tracing;
+  int B, S, p0, p1, forced_top, forced_bot, sos_override, tracing, prefix_len;
   bool operator<(const GraphKey& o) const {
-    return std::tie(B, S, p0, p1, forced_top, forced_bot, sos_override, tracing) <
-           std::tie(o.B, o.S, o.p0, o.p1, o.forced_top, o.forced_bot, o.sos_override, o.tracing);
+    return std::tie(B, S, p0, p1, forced_top, forced_bot, sos_override, tracing, prefix_len) <
+           std::tie(o.B, o.S, o.p0, o.p1, o.forced_top, o.forced_bot, o.sos_override, o.tracing, o.prefix_len);
   }
 };
 
@@ -158,8 +158,9 @@ struct hq_ctx {
   std::string err;
   std::vector<void*> allocs;       // parameters (live as long as the ctx)
   std::vector<void*> act_allocs;   // batch-sized state (re-made by hq_reserve_batch)
-  bool alloc_act = false;
-  size_t device_bytes = 0, act_bytes = 0;
+  std::vector<void*> pre_allocs;   // image-completion workspace (grown on demand by runs with a prefix, freed with act_allocs)
+  bool alloc_act = false, alloc_pre = false;
+  size_t device_bytes = 0, act_bytes = 0, pre_bytes = 0;
   std::map<std::string, ParamSlot> params;
   PFN_encodeTiled encode = nullptr;
 
@@ -191,6 +192,13 @@ struct hq_ctx {
   bool kv_maps = false;
   int num_sms = 0;
   int ws_rows = 0;
+  // image completion: the causal prefix pass runs on its own activation buffers of pre_rows rows (B x (T0 + P - 1) tokens;
+  // swapped in for h / att / mlp / q while it runs), so that a run without a prefix allocates nothing
+  ABuf pre_h, pre_att, pre_mlp;
+  void* pre_q = nullptr;
+  float* pre_x = nullptr;
+  int pre_rows = 0;
+  bool prefix_pass = false;        // attention(): causal multi-token calls take attention_prefix_kernel (2-byte engines)
   void *kc = nullptr, *vc = nullptr, *kd = nullptr, *vd = nullptr;
   int64_t *cond = nullptr, *codes_top = nullptr, *codes_bot = nullptr;
   float* sos_override = nullptr;
@@ -249,7 +257,10 @@ static int dev_alloc(hq_ctx* ctx, void** p, size_t bytes) {
   bytes = (bytes + 255) & ~static_cast<size_t>(255);
   HQ_CUDA(ctx, cudaMalloc(p, bytes));
   HQ_CUDA(ctx, cudaMemset(*p, 0, bytes));
-  if (ctx->alloc_act) {
+  if (ctx->alloc_pre) {
+    ctx->pre_allocs.push_back(*p);
+    ctx->pre_bytes += bytes;
+  } else if (ctx->alloc_act) {
     ctx->act_allocs.push_back(*p);
     ctx->act_bytes += bytes;
   } else {
@@ -504,9 +515,19 @@ extern "C" int hq_destroy(hq_ctx* ctx) {
   return HQ_OK;
 }
 
+static void free_prefix_ws(hq_ctx* ctx) {
+  for (void* p : ctx->pre_allocs) cudaFree(p);
+  ctx->pre_allocs.clear();
+  ctx->pre_bytes = 0;
+  ctx->pre_rows = 0;
+  ctx->pre_h = ABuf(); ctx->pre_att = ABuf(); ctx->pre_mlp = ABuf();
+  ctx->pre_q = nullptr; ctx->pre_x = nullptr;
+}
+
 static void free_activations(hq_ctx* ctx) {
   for (auto& kv : ctx->graphs) cudaGraphExecDestroy(kv.second.exec);
   ctx->graphs.clear();
+  free_prefix_ws(ctx);
   for (void* p : ctx->act_allocs) cudaFree(p);
   ctx->act_allocs.clear();
   ctx->act_bytes = 0;
@@ -932,7 +953,7 @@ extern "C" int hq_max_batch(const hq_ctx* ctx) { return ctx ? ctx->max_batch : 0
 
 extern "C" int64_t hq_last_launch_count(const hq_ctx* ctx) { return ctx ? ctx->last_launches : 0; }
 extern "C" int64_t hq_chain_launch_count(const hq_ctx* ctx) { return ctx ? ctx->chain_launches : 0; }
-extern "C" size_t hq_device_bytes(const hq_ctx* ctx) { return ctx ? ctx->device_bytes + ctx->act_bytes : 0; }
+extern "C" size_t hq_device_bytes(const hq_ctx* ctx) { return ctx ? ctx->device_bytes + ctx->act_bytes + ctx->pre_bytes : 0; }
 
 // ------------------------------------------------------------------------------------------------
 // launch helpers
@@ -1329,6 +1350,14 @@ static void attention(hq_ctx* ctx, cudaStream_t st, const AT* q, const AT* K, co
   if (resume) chain_flush(ctx, st);
   struct Resume { hq_ctx* c; bool on; ~Resume() { c->recording = on; } } resume_guard{ctx, resume};
   ctx->recording = false;
+  if constexpr (sizeof(AT) == 2) {
+    if (ctx->prefix_pass && causal && kbase == 0 && Tq <= ATT_MAX_KEYS) {
+      // image-completion prefix pass: one CTA per (image, head), K / V staged once, tensor-core QK^T and PV
+      launch_k(ctx, st, "attention_prefix", attention_prefix_kernel<AT>, dim3((M / Tq) * ctx->nh), dim3(256), 0, q, K, V, out,
+               ctx->nh, ctx->D, Tq, t_stride);
+      return;
+    }
+  }
   if (Tq == 1 && !causal && !ctx->dbg.attn_generic && attn_decode_plan<AT>(ctx, &CH, &hpc, &groups, &smem)) {
     // spatial decode: (image, head group) work items, K/V streamed through shared memory by bulk async copies
     if (ctx->tracing) ctx->tag_suffix = ":t" + std::to_string(kbase) + ":B" + std::to_string(M);
@@ -1450,7 +1479,9 @@ template <typename AT>
 static void gemm_resid(hq_ctx* ctx, cudaStream_t st, const ABuf& A, const Weight& W, const float* bias, float* x, int M,
                        int N, int K, int rows_per_image, Fold* fold) {
   const Fc2Plan plan = pick_resid_plan(ctx, M, N, K, rows_per_image);
-  if (plan.splits > 1 && M <= ctx->ws_rows) {
+  // The image-completion prefix pass never splits: whether M fits the split-K workspace depends on the batch, and a row's
+  // rounding must not (its M = B x (T0 + P - 1) GEMMs have tiles enough without slices).
+  if (plan.splits > 1 && M <= ctx->ws_rows && !ctx->prefix_pass) {
     gemm_fc2_split(ctx, st, A, W, M, N, K, plan.splits, plan.bn, static_cast<AT*>(nullptr));
     fold->partial = ctx->splitk_ws;
     fold->n = plan.splits;
@@ -1498,6 +1529,8 @@ static void run_block(hq_ctx* ctx, cudaStream_t st, const BlockW& w, float* x, i
 struct RunFlags {
   int forced_top, forced_bot, sos_override, forced_mid;
   int shared_prefix;    // text models: every row has the same prompt - prefill image 0 only, broadcast its cache rows
+  int prefix_len;       // image completion: positions < prefix_len are given; run_prefix fills their cache slots
+  int prefix_shared;    // ... and every row has the same condition and prefix: the prefix pass runs for image 0 only
   int fuse_mask;        // bit filt_sel (0 top, 1 bottom, 2 middle): that filter pair is (None, None) -> head GEMM draws in its epilogue
   float* logits_out;
 };
@@ -1737,10 +1770,67 @@ static void run_position3(hq_ctx* ctx, cudaStream_t st, int B, int S, int pos, c
   draw(ctx, st, sa, head_gemm<AT>(ctx, st, ctx->head_bot, 16 * B, ctx->Vb, sa, f));
 }
 
+// Image completion (hq_run_args.prefix_len = P): the spatial KV cache of the given positions 0 .. P - 2 (cache slots
+// 0 .. T0 + P - 2) in ONE causal pass over the T0 + P - 1 tokens of every image - the text prefill's shape, large-M GEMMs -
+// instead of P steps of the loop.  It depends on the given codes only: no depth pass, ln_f, head or draw.  run_position(P)
+// then embeds stack P - 1 into slot T0 + P - 1 as usual and samples on.  The last block stops after its QKV GEMM (its
+// attention output and MLP feed nothing).  No chain kernel here, as for the text prefill.  Shared prefix: image 0 only, then
+// its cache rows (every layer) are broadcast; the depth start token is computed per row by step P.
+template <typename AT>
+static void run_prefix(hq_ctx* ctx, cudaStream_t st, int B, int S, const RunFlags& f) {
+  const int D = ctx->D, T0 = ctx->T0, Tc = ctx->Tc, L = ctx->L;
+  const int N = T0 + f.prefix_len - 1;                 // tokens per image
+  const bool shared = f.prefix_shared && B > 1;
+  const int M = (shared ? 1 : B) * N;
+  AT* kc = static_cast<AT*>(ctx->kc);
+  AT* vc = static_cast<AT*>(ctx->vc);
+  const size_t lstride = static_cast<size_t>(ctx->max_batch) * Tc * D;
+  const int eb = (D / 4 + 31) / 32 * 32 > 1024 ? 1024 : (D / 4 + 31) / 32 * 32;
+  // the prefix workspace stands in for the step activations while the pass runs
+  std::swap(ctx->h, ctx->pre_h); std::swap(ctx->att, ctx->pre_att); std::swap(ctx->mlp, ctx->pre_mlp); std::swap(ctx->q, ctx->pre_q);
+  ctx->full_dependency_next = true;                    // as every position's first kernel (see run_position)
+  if (ctx->levels == 3) {
+    Embed3Args ea;
+    ea.x = ctx->pre_x; ea.sos_table = ctx->sos_table; ea.sos_override = f.sos_override ? ctx->sos_override : nullptr;
+    ea.cond = ctx->cond; ea.E0 = ctx->E_top; ea.E1 = ctx->E_mid; ea.E2 = ctx->E_bot; ea.P_top = ctx->P_top; ea.P_emb = ctx->P_emb;
+    ea.codes_top = ctx->codes_top; ea.codes_mid = ctx->codes_mid; ea.codes_bot = ctx->codes_bot;
+    ea.D = D; ea.S = S; ea.pos = 0; ea.cond_kind = ctx->cfg.cond_kind;
+    launch_k(ctx, st, "embed_prefix", embed3_prefix_kernel, dim3(M), dim3(eb), 0, ea, N);
+  } else {
+    EmbedArgs ea;
+    ea.x = ctx->pre_x; ea.sos_table = ctx->sos_table; ea.sos_override = f.sos_override ? ctx->sos_override : nullptr;
+    ea.cond = ctx->cond; ea.E_top = ctx->E_top; ea.E_bot = ctx->E_bot; ea.P_top = ctx->P_top; ea.P_emb = ctx->P_emb;
+    ea.codes_top = ctx->codes_top; ea.codes_bot = ctx->codes_bot; ea.D = D; ea.S = S; ea.pos = 0;
+    ea.cond_kind = ctx->cfg.cond_kind;
+    ea.emb_kind = ctx->cfg.embedding_kind; ea.P_top_h = ctx->P_top_h; ea.P_top_w = ctx->P_top_w; ea.Hpos = ctx->Hpos;
+    launch_k(ctx, st, "embed_prefix", embed_prefix_kernel, dim3(M), dim3(eb), 0, ea, static_cast<const float*>(ctx->E_txt),
+             static_cast<const float*>(ctx->P_txt), T0, N);
+  }
+  ctx->prefix_pass = true;
+  Fold fold;
+  for (int l = 0; l + 1 < L; ++l)
+    run_block<AT>(ctx, st, ctx->blocks[l], ctx->pre_x, M, 0, kc + l * lstride, vc + l * lstride, N, Tc, 0, 0, 1, &fold);
+  {
+    const BlockW& w = ctx->blocks[L - 1];
+    layernorm_act<AT>(ctx, st, ctx->pre_x, w.ln1g, w.ln1b, static_cast<AT*>(ctx->h.ptr), M, &fold);
+    EpiParams<AT> ep;
+    memset(&ep, 0, sizeof(ep));
+    ep.q = static_cast<AT*>(ctx->q); ep.kdst = kc + (L - 1) * lstride; ep.vdst = vc + (L - 1) * lstride; ep.D = D; ep.rpb = N;
+    ep.t_stride = Tc; ep.t0 = 0; ep.bias = w.bqkv; ep.sec0 = 0; ep.vdup = nullptr;
+    gemm_any<EPI_QKV>(ctx, st, ctx->h, w.qkv, 0, M, 3 * D, D, ep);
+  }
+  ctx->prefix_pass = false;
+  std::swap(ctx->h, ctx->pre_h); std::swap(ctx->att, ctx->pre_att); std::swap(ctx->mlp, ctx->pre_mlp); std::swap(ctx->q, ctx->pre_q);
+  if (shared)    // image 0's N cache rows of every layer -> images 1..B-1 (the kernel's copy of yd row 0 is rewritten by step P)
+    launch_k(ctx, st, "broadcast_prefix", broadcast_prefix_kernel<AT>, dim3(N, L, B - 1), dim3(256), 0, kc, vc, ctx->yd,
+             ctx->max_batch, Tc, D);
+}
+
 static void run_range(hq_ctx* ctx, cudaStream_t st, int B, int S, int p0, int p1, const RunFlags& f) {
   with_act(ctx->prec, [&](auto tag) {
     using AT = decltype(tag);
-    for (int pos = p0; pos < p1; ++pos) {
+    if (f.prefix_len > 0) run_prefix<AT>(ctx, st, B, S, f);
+    for (int pos = p0 + f.prefix_len; pos < p1; ++pos) {
       if (ctx->levels == 3) run_position3<AT>(ctx, st, B, S, pos, f);
       else run_position<AT>(ctx, st, B, S, pos, f);
     }
@@ -1767,6 +1857,25 @@ static int validate_run(hq_ctx* ctx, const hq_run_args* a) {
     set_err(ctx, "conditional model: `cond` (or `sos`) is required at pos_begin == 0");
     return HQ_ERR_INVALID;
   }
+  if (a->prefix_len < 0) {
+    set_err(ctx, "prefix_len must be >= 0 (got %d)", a->prefix_len);
+    return HQ_ERR_INVALID;
+  }
+  if (a->prefix_len > 0) {
+    if (a->pos_begin != 0) {
+      set_err(ctx, "prefix_len %d needs pos_begin == 0 (got %d): a completion starts a new batch", a->prefix_len, a->pos_begin);
+      return HQ_ERR_INVALID;
+    }
+    if (a->prefix_len >= a->pos_end) {
+      set_err(ctx, "prefix_len %d must be below pos_end %d (at least one position is sampled)", a->prefix_len, a->pos_end);
+      return HQ_ERR_INVALID;
+    }
+    if (ctx->T0 + a->prefix_len - 1 > ATT_MAX_KEYS) {
+      set_err(ctx, "prefix_len %d: %d prefix tokens exceed the %d keys of the attention kernels", a->prefix_len,
+              ctx->T0 + a->prefix_len - 1, ATT_MAX_KEYS);
+      return HQ_ERR_INVALID;
+    }
+  }
   const hq_sampling_params& s = a->sampling;
   if (!(s.temperature_top > 0.f) || !(s.temperature_bot > 0.f)) {
     set_err(ctx, "softmax temperatures must be > 0 (got %g, %g)", s.temperature_top, s.temperature_bot);
@@ -1775,12 +1884,46 @@ static int validate_run(hq_ctx* ctx, const hq_run_args* a) {
   return HQ_OK;
 }
 
+// The image-completion workspace for `rows` prefix tokens (grown, never shrunk, until hq_reserve_batch).  Graphs captured
+// with a prefix point into the buffers being replaced: they go too.  Runs without a prefix never come here.
+static int ensure_prefix_ws(hq_ctx* ctx, int rows) {
+  if (rows <= ctx->pre_rows) return HQ_OK;
+  HQ_CUDA(ctx, cudaDeviceSynchronize());
+  for (auto it = ctx->graphs.begin(); it != ctx->graphs.end();) {
+    if (it->first.prefix_len > 0) {
+      cudaGraphExecDestroy(it->second.exec);
+      it = ctx->graphs.erase(it);
+    } else {
+      ++it;
+    }
+  }
+  free_prefix_ws(ctx);
+  ctx->alloc_pre = true;
+  struct Guard { hq_ctx* c; ~Guard() { c->alloc_pre = false; } } guard{ctx};
+  const int D = ctx->D;
+  int rc;
+  if ((rc = alloc_abuf(ctx, &ctx->pre_h, rows, D)) || (rc = alloc_abuf(ctx, &ctx->pre_att, rows, D)) ||
+      (rc = alloc_abuf(ctx, &ctx->pre_mlp, rows, 4 * D)) ||
+      (rc = dev_alloc(ctx, &ctx->pre_q, static_cast<size_t>(rows) * D * ctx->wsize)) ||
+      (rc = alloc_f32(ctx, &ctx->pre_x, static_cast<size_t>(rows) * D))) {
+    const std::string why = ctx->err;
+    cudaGetLastError();
+    free_prefix_ws(ctx);
+    set_err(ctx, "image-completion workspace of %d rows: %s", rows, why.c_str());
+    return rc;
+  }
+  ctx->pre_rows = rows;
+  return HQ_OK;
+}
+
 static int run_impl(hq_ctx* ctx, const hq_run_args* a, cudaStream_t st, cudaMemcpyKind in_kind, cudaMemcpyKind out_kind) {
   int rc = validate_run(ctx, a);
   if (rc) return rc;
   HQ_CUDA(ctx, cudaSetDevice(ctx->device));
-  const int B = a->batch, S = a->seq_len, D = ctx->D, T0 = ctx->T0;
+  const int B = a->batch, S = a->seq_len, D = ctx->D, T0 = ctx->T0, P = a->prefix_len;
   const size_t nt = static_cast<size_t>(B) * S * 8, nb = nt * (ctx->levels == 3 ? 16 : 4), nm = nt * 4;
+  const int prefix_shared = P > 0 && a->shared_prefix != 0 && a->sos == nullptr;
+  if (P > 0 && (rc = ensure_prefix_ws(ctx, (prefix_shared && B > 1 ? 1 : B) * (T0 + P - 1)))) return rc;
 
   // ---- stage inputs into ctx-owned buffers (what the captured graph reads) ----
   // pageable source: the runtime stages it before returning, so back-to-back calls cannot race on it
@@ -1790,21 +1933,35 @@ static int run_impl(hq_ctx* ctx, const hq_run_args* a, cudaStream_t st, cudaMemc
       HQ_CUDA(ctx, cudaMemcpyAsync(ctx->cond, a->cond, static_cast<size_t>(B) * T0 * 8, in_kind, st));
     if (a->sos)
       HQ_CUDA(ctx, cudaMemcpyAsync(ctx->sos_override, a->sos, static_cast<size_t>(B) * T0 * D * 4, in_kind, st));
-  } else {
+  }
+  if (a->pos_begin > 0 || P > 0) {     // the codes of the earlier positions (a continued batch, or a completion's prefix)
     HQ_CUDA(ctx, cudaMemcpyAsync(ctx->codes_top, a->codes_top, nt, in_kind, st));
     HQ_CUDA(ctx, cudaMemcpyAsync(ctx->codes_bot, a->codes_bot, nb, in_kind, st));
     if (ctx->levels == 3) HQ_CUDA(ctx, cudaMemcpyAsync(ctx->codes_mid, a->codes_mid, nm, in_kind, st));
   }
-  if (a->given_top) HQ_CUDA(ctx, cudaMemcpyAsync(ctx->codes_top, a->given_top, nt, in_kind, st));
-  if (a->given_bot) HQ_CUDA(ctx, cudaMemcpyAsync(ctx->codes_bot, a->given_bot, nb, in_kind, st));
-  if (ctx->levels == 3 && a->given_mid) HQ_CUDA(ctx, cudaMemcpyAsync(ctx->codes_mid, a->given_mid, nm, in_kind, st));
+  if (P == 0) {
+    if (a->given_top) HQ_CUDA(ctx, cudaMemcpyAsync(ctx->codes_top, a->given_top, nt, in_kind, st));
+    if (a->given_bot) HQ_CUDA(ctx, cudaMemcpyAsync(ctx->codes_bot, a->given_bot, nb, in_kind, st));
+    if (ctx->levels == 3 && a->given_mid) HQ_CUDA(ctx, cudaMemcpyAsync(ctx->codes_mid, a->given_mid, nm, in_kind, st));
+  } else {
+    // forced codes apply at positions >= P only: the prefix keeps the codes just copied in
+    auto given_tail = [&](int64_t* dst, const int64_t* src, size_t per_pos) {
+      const size_t pitch = static_cast<size_t>(S) * per_pos * 8, off = static_cast<size_t>(P) * per_pos;
+      return cudaMemcpy2DAsync(dst + off, pitch, src + off, pitch, pitch - off * 8, B, in_kind, st);
+    };
+    if (a->given_top) HQ_CUDA(ctx, given_tail(ctx->codes_top, a->given_top, 1));
+    if (a->given_bot) HQ_CUDA(ctx, given_tail(ctx->codes_bot, a->given_bot, ctx->levels == 3 ? 16 : 4));
+    if (ctx->levels == 3 && a->given_mid) HQ_CUDA(ctx, given_tail(ctx->codes_mid, a->given_mid, 4));
+  }
 
   RunFlags f;
   f.forced_top = a->given_top != nullptr;
   f.forced_bot = a->given_bot != nullptr;
   f.forced_mid = ctx->levels == 3 && a->given_mid != nullptr;
-  f.shared_prefix = a->shared_prefix != 0 && ctx->cfg.cond_kind == HQ_COND_TXT && a->sos == nullptr &&
+  f.shared_prefix = P == 0 && a->shared_prefix != 0 && ctx->cfg.cond_kind == HQ_COND_TXT && a->sos == nullptr &&
                     ctx->cfg.model_type != HQ_MODEL_BIDIRECTIONAL;
+  f.prefix_len = P;
+  f.prefix_shared = prefix_shared;
   f.sos_override = a->sos != nullptr;
   f.fuse_mask = 0;
   if (ctx->cfg.fuse_head_sampler && ctx->half) {
@@ -1863,8 +2020,9 @@ static int run_impl(hq_ctx* ctx, const hq_run_args* a, cudaStream_t st, cudaMemc
     ctx->launches = 0;
   };
   if (use_graph) {
-    GraphKey key{B, S, a->pos_begin, a->pos_end, f.forced_top, f.forced_bot | (f.forced_mid << 1) | (f.shared_prefix << 2) | (f.fuse_mask << 3), f.sos_override,
-                 ctx->tracing ? 1 : 0};
+    GraphKey key{B, S, a->pos_begin, a->pos_end, f.forced_top,
+                 f.forced_bot | (f.forced_mid << 1) | (f.shared_prefix << 2) | (f.fuse_mask << 3) | (f.prefix_shared << 6), f.sos_override,
+                 ctx->tracing ? 1 : 0, P};
     auto it = ctx->graphs.find(key);
     if (it == ctx->graphs.end()) {
       plan_chains();
@@ -1917,7 +2075,13 @@ static int run_impl(hq_ctx* ctx, const hq_run_args* a, cudaStream_t st, cudaMemc
   HQ_CUDA(ctx, cudaMemcpyAsync(a->codes_bot, ctx->codes_bot, nb, out_kind, st));
   if (ctx->levels == 3) HQ_CUDA(ctx, cudaMemcpyAsync(a->codes_mid, ctx->codes_mid, nm, out_kind, st));
   if (dev_logits) {
-    HQ_CUDA(ctx, cudaMemcpyAsync(a->logits, dev_logits, nlog, cudaMemcpyDeviceToHost, st));
+    if (P > 0) {    // positions >= P only: the caller's prefix rows stay untouched
+      const size_t row = nlog / B, off = row / S * P;
+      HQ_CUDA(ctx, cudaMemcpy2DAsync(reinterpret_cast<char*>(a->logits) + off, row, reinterpret_cast<const char*>(dev_logits) + off,
+                                     row, row - off, B, cudaMemcpyDeviceToHost, st));
+    } else {
+      HQ_CUDA(ctx, cudaMemcpyAsync(a->logits, dev_logits, nlog, cudaMemcpyDeviceToHost, st));
+    }
     HQ_CUDA(ctx, cudaStreamSynchronize(st));
     cudaFree(dev_logits);
   }
@@ -1984,6 +2148,37 @@ extern "C" int hq_debug_attention(int prec, const void* q, const void* K, const 
   if (e == cudaSuccess) e = tmp.launch_err;
   if (e != cudaSuccess) {
     set_err(nullptr, "hq_debug_attention: %s", cudaGetErrorString(e));
+    return HQ_ERR_CUDA;
+  }
+  return HQ_OK;
+}
+
+extern "C" int hq_debug_attention_prefix(int prec, const void* q, const void* K, const void* V, void* out, int B, int n_heads,
+                                         int t_stride, int n_q, int variant, void* stream) {
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (B < 1 || n_heads < 1 || n_q < 1 || n_q > t_stride || n_q > ATT_MAX_KEYS || !q || !K || !V || !out) {
+    set_err(nullptr, "hq_debug_attention_prefix: bad argument");
+    return HQ_ERR_INVALID;
+  }
+  hq_ctx tmp;   // launch bookkeeping + the fields attention() reads
+  int dev = 0;
+  HQ_CUDA(nullptr, cudaGetDevice(&dev));
+  int rc = check_device(&tmp, dev);
+  if (rc) return rc;
+  tmp.prec = (prec == HQ_PREC_BF16 || prec == HQ_PREC_F16) ? prec : HQ_PREC_FP32;
+  tmp.half = tmp.prec != HQ_PREC_FP32;
+  tmp.D = n_heads * 64;
+  tmp.nh = n_heads;
+  tmp.prefix_pass = variant != 1;
+  with_act(tmp.prec, [&](auto tag) {
+    using AT = decltype(tag);
+    attention<AT>(&tmp, st, static_cast<const AT*>(q), static_cast<const AT*>(K), static_cast<const AT*>(V), static_cast<AT*>(out),
+                  B * n_q, n_q, t_stride, 0, 1);
+  });
+  cudaError_t e = cudaStreamSynchronize(st);
+  if (e == cudaSuccess) e = tmp.launch_err;
+  if (e != cudaSuccess) {
+    set_err(nullptr, "hq_debug_attention_prefix: %s", cudaGetErrorString(e));
     return HQ_ERR_CUDA;
   }
   return HQ_OK;

@@ -243,6 +243,128 @@ broadcast_prefix_kernel(int trace_id, AT* K, AT* V, float* yd, int Bmax, int Tc,
       *reinterpret_cast<float4*>(yd + static_cast<size_t>(b) * D + i) = *reinterpret_cast<const float4*>(yd + i);
 }
 
+// Image completion (hq_run_args.prefix_len = P): the spatial input tokens of the given prefix, all of them in one launch.
+//   row r = b * N + t, N = T0 + P - 1 tokens per image:
+//   t <  T0 : the conditioning row - `sos` override, E_txt[ids[b, t]] + P_txt[t] (text), sos table (class / unconditional)
+//   t >= T0 : the stack of position p = t - T0 (0 .. P - 2), what embed_kernel writes at pos = p + 1
+// Every float operation is the one of embed_kernel / embed_txt_kernel, in the same order, so each token is bit-identical
+// to the one the step path embeds (the arithmetic is restated here so that those kernels stay exactly as they are).
+// One CTA per row.
+__global__ void __launch_bounds__(1024)
+embed_prefix_kernel(int trace_id, EmbedArgs a, const float* __restrict__ E_txt, const float* __restrict__ P_txt, int T0, int N) {
+  TraceScope trace_scope(trace_id);
+  pdl_launch_dependents();
+  pdl_wait();
+  const int row = blockIdx.x;
+  const int b = row / N, t = row % N;
+  float4* xo = reinterpret_cast<float4*>(a.x + static_cast<size_t>(row) * a.D);
+  const int n4 = a.D / 4;
+  if (t < T0) {
+    const float* src;
+    if (a.sos_override != nullptr) {
+      src = a.sos_override + (static_cast<size_t>(b) * T0 + t) * a.D;
+    } else if (a.cond_kind == HQ_COND_TXT) {
+      const float4* e = reinterpret_cast<const float4*>(E_txt + static_cast<size_t>(a.cond[static_cast<size_t>(b) * T0 + t]) * a.D);
+      const float4* p = reinterpret_cast<const float4*>(P_txt + static_cast<size_t>(t) * a.D);
+      for (int i = threadIdx.x; i < n4; i += blockDim.x) {
+        float4 u = e[i], c = p[i];
+        xo[i] = make_float4(u.x + c.x, u.y + c.y, u.z + c.z, u.w + c.w);
+      }
+      return;
+    } else if (a.cond_kind == HQ_COND_CLS) {
+      src = a.sos_table + static_cast<size_t>(a.cond[b]) * a.D;
+    } else {
+      src = a.sos_table;
+    }
+    const float4* s4 = reinterpret_cast<const float4*>(src);
+    for (int i = threadIdx.x; i < n4; i += blockDim.x) xo[i] = s4[i];
+    return;
+  }
+  const int p = t - T0;
+  const int64_t ct = a.codes_top[static_cast<size_t>(b) * a.S + p];
+  const int64_t* cbp = a.codes_bot + (static_cast<size_t>(b) * a.S + p) * 4;
+  const float4* et = reinterpret_cast<const float4*>(a.E_top + static_cast<size_t>(ct) * a.D);
+  const bool pos2d = a.P_top_h != nullptr;
+  const float4* pt = reinterpret_cast<const float4*>(pos2d ? a.P_top_h + static_cast<size_t>(p / a.Hpos) * a.D
+                                                           : a.P_top + static_cast<size_t>(p) * a.D);
+  const float4* pw = pos2d ? reinterpret_cast<const float4*>(a.P_top_w + static_cast<size_t>(p % a.Hpos) * a.D) : nullptr;
+  if (a.emb_kind == 1) {
+    const int Dq = a.D / 4;
+    const float* ebq[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) ebq[j] = a.E_bot + static_cast<size_t>(cbp[j]) * Dq;
+    for (int i = threadIdx.x; i < n4; i += blockDim.x) {
+      const float4 u = et[i];
+      float4 q = pt[i];
+      if (pos2d) { const float4 w = pw[i]; q.x += w.x; q.y += w.y; q.z += w.z; q.w += w.w; }
+      xo[i] = make_float4((u.x + q.x) + ebq[0][i], (u.y + q.y) + ebq[1][i], (u.z + q.z) + ebq[2][i], (u.w + q.w) + ebq[3][i]);
+    }
+    return;
+  }
+  const float4* eb[4];
+#pragma unroll
+  for (int j = 0; j < 4; ++j) eb[j] = reinterpret_cast<const float4*>(a.E_bot + static_cast<size_t>(cbp[j]) * a.D);
+  const float4* pe = reinterpret_cast<const float4*>(a.P_emb);
+  for (int i = threadIdx.x; i < n4; i += blockDim.x) {
+    float4 u = et[i], q = pt[i], e0 = pe[i];
+    if (pos2d) { const float4 w = pw[i]; q.x += w.x; q.y += w.y; q.z += w.z; q.w += w.w; }
+    float4 acc;
+    acc.x = (u.x + q.x) + e0.x; acc.y = (u.y + q.y) + e0.y; acc.z = (u.z + q.z) + e0.z; acc.w = (u.w + q.w) + e0.w;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      float4 e = eb[j][i], pj = pe[(j + 1) * n4 + i];
+      acc.x += e.x + pj.x; acc.y += e.y + pj.y; acc.z += e.z + pj.z; acc.w += e.w + pj.w;
+    }
+    acc.x /= 5.0f; acc.y /= 5.0f; acc.z /= 5.0f; acc.w /= 5.0f;
+    xo[i] = acc;
+  }
+}
+
+// The same for the 3-level HQTransformer (T0 = 1): row b * N + t is the sos row (t = 0) or the 21-token stack mean of
+// position t - 1, with embed3_kernel's operations and order.
+__global__ void __launch_bounds__(1024) embed3_prefix_kernel(int trace_id, Embed3Args a, int N) {
+  TraceScope trace_scope(trace_id);
+  pdl_launch_dependents();
+  pdl_wait();
+  const int row = blockIdx.x;
+  const int b = row / N, t = row % N;
+  float4* xo = reinterpret_cast<float4*>(a.x + static_cast<size_t>(row) * a.D);
+  const int n4 = a.D / 4;
+  if (t == 0) {
+    const float* src;
+    if (a.sos_override != nullptr) src = a.sos_override + static_cast<size_t>(b) * a.D;
+    else if (a.cond_kind == HQ_COND_CLS) src = a.sos_table + static_cast<size_t>(a.cond[b]) * a.D;
+    else src = a.sos_table;
+    const float4* s4 = reinterpret_cast<const float4*>(src);
+    for (int i = threadIdx.x; i < n4; i += blockDim.x) xo[i] = s4[i];
+    return;
+  }
+  const int p = t - 1;
+  __shared__ const float* rows[21];
+  if (threadIdx.x < 21) {
+    const size_t bp = static_cast<size_t>(b) * a.S + p;
+    const int j = threadIdx.x;
+    rows[j] = j == 0 ? a.E0 + static_cast<size_t>(a.codes_top[bp]) * a.D
+            : j < 5 ? a.E1 + static_cast<size_t>(a.codes_mid[bp * 4 + (j - 1)]) * a.D
+                    : a.E2 + static_cast<size_t>(a.codes_bot[bp * 16 + (j - 5)]) * a.D;
+  }
+  __syncthreads();
+  const float4* pt = reinterpret_cast<const float4*>(a.P_top + static_cast<size_t>(p) * a.D);
+  const float4* pe = reinterpret_cast<const float4*>(a.P_emb);
+  for (int i = threadIdx.x; i < n4; i += blockDim.x) {
+    const float4 u = reinterpret_cast<const float4*>(rows[0])[i], q = pt[i], e0 = pe[i];
+    float4 acc;
+    acc.x = (u.x + q.x) + e0.x; acc.y = (u.y + q.y) + e0.y; acc.z = (u.z + q.z) + e0.z; acc.w = (u.w + q.w) + e0.w;
+#pragma unroll 4
+    for (int j = 1; j < 21; ++j) {
+      const float4 e = reinterpret_cast<const float4*>(rows[j])[i], pj = pe[j * n4 + i];
+      acc.x += e.x + pj.x; acc.y += e.y + pj.y; acc.z += e.z + pj.z; acc.w += e.w + pj.w;
+    }
+    acc.x /= 21.0f; acc.y /= 21.0f; acc.z /= 21.0f; acc.w /= 21.0f;
+    xo[i] = acc;
+  }
+}
+
 // model_type 'top2bot' (hierarchical_ar.py:596-601): input of depth pass c >= 1:
 //   y[b] = E[code[b]] + P_depth[c - 1], E = tok_emb_top_depth with the top code (c == 1), tok_emb_bot_depth with bottom
 //   code c - 2 otherwise.  `codes` points at the first code (element stride `cstride` int64 between images).
@@ -1166,6 +1288,148 @@ attention_decode_mma_kernel(int trace_id, const __grid_constant__ CUtensorMap tm
     if (it == 0 && threadIdx.x == 0) phase_mark(6);
   }
   if (threadIdx.x == 0) phase_mark(7);
+#endif
+}
+
+// ------------------------------------------------------------------------------------------------
+// Causal attention of the image-completion prefix pass (2-byte engines): the Tq = T0 + P - 1 <= 128 prefix tokens of an
+// image, query i over cache slots 0 .. i - attention_kernel with causal = 1, kbase = 0.  attention_kernel gives every
+// (query, head) a warp of its own, which re-reads the image's keys and values from L2 once per query; here one CTA per
+// (image, head) stages them in shared memory once.  Warp w owns queries 16w .. 16w + 15:
+//   S = q K^T on mma.sync m16n8k16 (fp32 accumulation), scaled by 2^-3;
+//   fp32 causal softmax in registers (row max / sum over the four lanes of a fragment row);
+//   O = P V on mma.sync m16n8k16 with P split into a 2-byte head and tail (attention_decode_mma_kernel's split: P carried
+//   to ~2^-17 relative, not the 2-byte type's 2^-8 / 2^-11), then O / sum rounded to the 2-byte type.
+// q / out: row b * Tq + i of [*, D]; K / V: row b * t_stride + t of [*, D] (one layer's cache).  Grid: B * n_heads CTAs.
+// ------------------------------------------------------------------------------------------------
+constexpr int ATTP_PITCH = 72;    // shared row pitch of K / V (elements): 144-byte rows keep fragment loads conflict-free
+
+template <typename AT>
+__global__ void __launch_bounds__(256)
+attention_prefix_kernel(int trace_id, const AT* __restrict__ q, const AT* __restrict__ K, const AT* __restrict__ V,
+                        AT* __restrict__ out, int n_heads, int D, int Tq, int t_stride) {
+#if defined(__CUDA_ARCH__)
+  TraceScope trace_scope(trace_id);
+  pdl_launch_dependents();
+  pdl_wait();
+  __shared__ __align__(16) AT ks[ATT_MAX_KEYS * ATTP_PITCH];
+  __shared__ __align__(16) AT vs[ATT_MAX_KEYS * ATTP_PITCH];
+  const int b = blockIdx.x / n_heads, h = blockIdx.x % n_heads;
+  // keys staged: Tq rounded up to the 16-key step of the value MMA; rows past Tq are zero (0 * garbage must not reach O)
+  const int nrows = (Tq + 15) & ~15;
+  const AT* Kb = K + static_cast<size_t>(b) * t_stride * D + h * 64;
+  const AT* Vb = V + static_cast<size_t>(b) * t_stride * D + h * 64;
+  for (int i = threadIdx.x; i < nrows * 8; i += blockDim.x) {
+    const int t = i >> 3, c = (i & 7) * 8;
+    uint4 kv = make_uint4(0u, 0u, 0u, 0u), vv = kv;
+    if (t < Tq) {
+      kv = *reinterpret_cast<const uint4*>(Kb + static_cast<size_t>(t) * D + c);
+      vv = *reinterpret_cast<const uint4*>(Vb + static_cast<size_t>(t) * D + c);
+    }
+    *reinterpret_cast<uint4*>(ks + t * ATTP_PITCH + c) = kv;
+    *reinterpret_cast<uint4*>(vs + t * ATTP_PITCH + c) = vv;
+  }
+  __syncthreads();
+  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int r0 = w * 16;
+  if (r0 >= Tq) return;
+  const int gq = lane >> 2, tq = lane & 3;          // fragment row / column pair
+  const int ra = r0 + gq, rb = ra + 8;              // the two query rows of this lane
+  const int nks = ((r0 + 16 < Tq ? r0 + 16 : Tq) + 15) >> 4;   // 16-key steps holding keys <= the warp's last query
+
+  // q as the A operand (a0 / a2: row ra, a1 / a3: row rb; dims 2tq, 2tq + 1 and + 8 of each 16-dim step)
+  uint32_t qa[4][4];
+  {
+    const uint32_t* qra = reinterpret_cast<const uint32_t*>(q + (static_cast<size_t>(b) * Tq + (ra < Tq ? ra : 0)) * D + h * 64);
+    const uint32_t* qrb = reinterpret_cast<const uint32_t*>(q + (static_cast<size_t>(b) * Tq + (rb < Tq ? rb : 0)) * D + h * 64);
+#pragma unroll
+    for (int kk = 0; kk < 4; ++kk) {
+      qa[kk][0] = ra < Tq ? qra[kk * 8 + tq] : 0u;
+      qa[kk][1] = rb < Tq ? qrb[kk * 8 + tq] : 0u;
+      qa[kk][2] = ra < Tq ? qra[kk * 8 + 4 + tq] : 0u;
+      qa[kk][3] = rb < Tq ? qrb[kk * 8 + 4 + tq] : 0u;
+    }
+  }
+  // ---- scores: tile j = keys 8j .. 8j + 7; lane holds (ra | rb, keys 8j + 2tq, 8j + 2tq + 1) ----
+  float s[16][4];
+#pragma unroll
+  for (int j = 0; j < 16; ++j) {
+#pragma unroll
+    for (int e = 0; e < 4; ++e) s[j][e] = 0.f;
+    if (j < 2 * nks) {
+      const uint32_t* krow = reinterpret_cast<const uint32_t*>(ks + (j * 8 + gq) * ATTP_PITCH);
+#pragma unroll
+      for (int kk = 0; kk < 4; ++kk)
+        mma_16816<AT>(s[j], qa[kk][0], qa[kk][1], qa[kk][2], qa[kk][3], krow[kk * 8 + tq], krow[kk * 8 + 4 + tq]);
+    }
+  }
+  // ---- causal softmax, fp32 ----
+  float mx_a = -INFINITY, mx_b = -INFINITY;
+#pragma unroll
+  for (int j = 0; j < 16; ++j)
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+      const int key = j * 8 + 2 * tq + (e & 1);
+      const int row = e < 2 ? ra : rb;
+      const float v = (j < 2 * nks && key <= row) ? s[j][e] * 0.125f : -INFINITY;
+      s[j][e] = v;
+      if (e < 2) mx_a = fmaxf(mx_a, v);
+      else mx_b = fmaxf(mx_b, v);
+    }
+  mx_a = fmaxf(mx_a, __shfl_xor_sync(0xffffffffu, mx_a, 1));
+  mx_a = fmaxf(mx_a, __shfl_xor_sync(0xffffffffu, mx_a, 2));
+  mx_b = fmaxf(mx_b, __shfl_xor_sync(0xffffffffu, mx_b, 1));
+  mx_b = fmaxf(mx_b, __shfl_xor_sync(0xffffffffu, mx_b, 2));
+  float sum_a = 0.f, sum_b = 0.f;
+#pragma unroll
+  for (int j = 0; j < 16; ++j)
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+      const float p = expf(s[j][e] - (e < 2 ? mx_a : mx_b));    // masked keys: exp(-inf) = 0
+      s[j][e] = p;
+      if (e < 2) sum_a += p;
+      else sum_b += p;
+    }
+  sum_a += __shfl_xor_sync(0xffffffffu, sum_a, 1);
+  sum_a += __shfl_xor_sync(0xffffffffu, sum_a, 2);
+  sum_b += __shfl_xor_sync(0xffffffffu, sum_b, 1);
+  sum_b += __shfl_xor_sync(0xffffffffu, sum_b, 2);
+  // ---- O = P V: A = P (rows ra | rb, keys 16kk ..), head then tail; B = V rows by ldmatrix.trans ----
+  float o[8][4];
+#pragma unroll
+  for (int nt = 0; nt < 8; ++nt)
+#pragma unroll
+    for (int e = 0; e < 4; ++e) o[nt][e] = 0.f;
+  const uint32_t vrow = smem_u32(vs) + static_cast<uint32_t>((lane & 15) * ATTP_PITCH * 2);
+#pragma unroll
+  for (int kk = 0; kk < 8; ++kk) {
+    if (kk < nks) {
+      // a0: (ra, keys 16kk + 2tq ..), a1: (rb, same keys), a2 / a3: keys + 8 - C fragments of tiles 2kk and 2kk + 1
+      uint32_t hd[4], tl[4];
+#pragma unroll
+      for (int r = 0; r < 4; ++r) {
+        const int j = 2 * kk + (r >> 1), e = (r & 1) * 2;
+        hd[r] = pack2_rn<AT>(s[j][e], s[j][e + 1]);
+        const float2 f = unpack2<AT>(hd[r]);
+        tl[r] = pack2_rn<AT>(s[j][e] - f.x, s[j][e + 1] - f.y);
+      }
+#pragma unroll
+      for (int nt = 0; nt < 8; ++nt) {
+        uint32_t b0, b1;
+        ldmatrix_x2_trans(vrow + static_cast<uint32_t>((kk * 16 * ATTP_PITCH + nt * 8) * 2), b0, b1);
+        mma_16816<AT>(o[nt], hd[0], hd[1], hd[2], hd[3], b0, b1);
+        mma_16816<AT>(o[nt], tl[0], tl[1], tl[2], tl[3], b0, b1);
+      }
+    }
+  }
+  const float inv_a = 1.0f / sum_a, inv_b = 1.0f / sum_b;
+  AT* oa = out + (static_cast<size_t>(b) * Tq + ra) * D + h * 64 + 2 * tq;
+  AT* ob = out + (static_cast<size_t>(b) * Tq + rb) * D + h * 64 + 2 * tq;
+#pragma unroll
+  for (int nt = 0; nt < 8; ++nt) {
+    if (ra < Tq) *reinterpret_cast<uint32_t*>(oa + nt * 8) = pack2_rn<AT>(o[nt][0] * inv_a, o[nt][1] * inv_a);
+    if (rb < Tq) *reinterpret_cast<uint32_t*>(ob + nt * 8) = pack2_rn<AT>(o[nt][2] * inv_b, o[nt][3] * inv_b);
+  }
 #endif
 }
 

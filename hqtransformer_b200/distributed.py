@@ -58,6 +58,10 @@ def sampling_ihqgpt_sharded(model, num_candidates: int, cond, *, gather: bool = 
     lo, hi = shard_range(B, rank, world)
     local_cond = cond[lo:hi] if torch.is_tensor(cond) and cond.numel() > 1 else cond
     kw = dict(kw)
+    for name in ("prefix_code_top", "prefix_code_bot"):     # image completion: per-row prefixes follow the rows, as cond does
+        t = kw.get(name)
+        if t is not None and torch.is_tensor(t) and t.shape[0] > 1:
+            kw[name] = t[lo:hi]
     if kw.get("seed") is None:
         # one Philox key for the whole global batch: rank 0 draws it from its default generator, everyone uses it
         box = [fresh_seed() if rank == 0 else None]

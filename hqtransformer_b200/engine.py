@@ -156,8 +156,10 @@ class Engine:
             codes_top: torch.Tensor = None, codes_bot: torch.Tensor = None,
             logits: Optional[torch.Tensor] = None, host: bool = False, stream: Optional[int] = None,
             codes_mid: Optional[torch.Tensor] = None, given_mid: Optional[torch.Tensor] = None,
-            shared_prefix: bool = False) -> None:
-        """hq_run (device tensors, async on the current torch stream) or hq_run_host (CPU tensors, synchronous)."""
+            shared_prefix: bool = False, prefix_len: int = 0) -> None:
+        """hq_run (device tensors, async on the current torch stream) or hq_run_host (CPU tensors, synchronous).
+        prefix_len > 0 (with pos_begin 0): image completion - codes_top / codes_bot (/ codes_mid) hold the given codes of
+        positions < prefix_len, which come back unchanged; the rest is sampled after them."""
         tensors = dict(cond=cond, sos=sos, given_top=given_top, given_bot=given_bot, codes_top=codes_top,
                        codes_bot=codes_bot, logits=logits, codes_mid=codes_mid, given_mid=given_mid)
         for k, t in tensors.items():
@@ -172,7 +174,7 @@ class Engine:
                          cond=_ptr(cond), sos=_ptr(sos), given_top=_ptr(given_top), given_bot=_ptr(given_bot),
                          codes_top=_ptr(codes_top), codes_bot=_ptr(codes_bot), logits=_ptr(logits),
                          sampling=sampling.to_c(), codes_mid=_ptr(codes_mid), given_mid=_ptr(given_mid),
-                         shared_prefix=1 if shared_prefix else 0, reserved=0)
+                         shared_prefix=1 if shared_prefix else 0, prefix_len=int(prefix_len))
         if host:
             check(self._lib.hq_run_host(self._ctx, C.byref(args)), self._ctx, "hq_run_host")
         else:
@@ -346,6 +348,24 @@ def debug_attention(q: torch.Tensor, K: torch.Tensor, V: torch.Tensor, n_keys: i
         st = torch.cuda.current_stream(q.device).cuda_stream
         check(lib.hq_debug_attention(prec, q.data_ptr(), K.data_ptr(), V.data_ptr(), out.data_ptr(), B, D // 64, T, n_keys,
                                      variant, C.c_void_p(st)), None, "hq_debug_attention")
+    return out
+
+
+def debug_attention_prefix(q: torch.Tensor, K: torch.Tensor, V: torch.Tensor, variant: int = 0) -> torch.Tensor:
+    """Causal attention of the image-completion prefix pass: query i of q [B, n_q, D] over keys 0 .. i of K / V [B, T, D]
+    (head size 64, T >= n_q) through the engine's kernel for that pass (bf16 / fp16: the tensor-core prefix kernel, fp32:
+    the fp32 engine's per-query kernel); variant 1: the per-query kernel at every precision (the text prefill's)."""
+    lib = _lib.load()
+    assert q.is_cuda and q.dtype == K.dtype == V.dtype and q.dtype in _ACT2PREC
+    assert q.is_contiguous() and K.is_contiguous() and V.is_contiguous() and K.shape == V.shape
+    B, n_q, D = q.shape
+    T = K.shape[1]
+    assert K.shape == (B, T, D) and D % 64 == 0 and 1 <= n_q <= T
+    out = torch.empty_like(q)
+    with torch.cuda.device(q.device):
+        st = torch.cuda.current_stream(q.device).cuda_stream
+        check(lib.hq_debug_attention_prefix(_ACT2PREC[q.dtype], q.data_ptr(), K.data_ptr(), V.data_ptr(), out.data_ptr(), B,
+                                            D // 64, T, n_q, int(variant), C.c_void_p(st)), None, "hq_debug_attention_prefix")
     return out
 
 

@@ -172,9 +172,13 @@ def _triple(v, name):
 def sampling_hqtransformer(model: HQTransformer, num_candidates: int, cond, top_k: Optional[List[float]] = None,
                            top_p: Optional[List[float]] = None, softmax_temperature: List[float] = [1.0, 1.0, 1.0],
                            is_tqdm: bool = True, use_fp16: bool = True, max_seq_len: int = 256, model_stage1=None, *,
-                           seed: Optional[int] = None, row_offset: int = 0) -> List[torch.Tensor]:
+                           seed: Optional[int] = None, row_offset: int = 0, prefix_codes: Optional[Sequence] = None,
+                           shared_prefix: Optional[bool] = None) -> List[torch.Tensor]:
     """utils/sampling.py:240-307: returns [codes_top [B,S], codes_mid [B,S,4], codes_bot [B,S,16]] (int64).  `top_k`,
-    `top_p`, `softmax_temperature`: one entry per level (hqtransformer.py:626-631).  `cond` may be a per-row class tensor."""
+    `top_p`, `softmax_temperature`: one entry per level (hqtransformer.py:626-631).  `cond` may be a per-row class tensor.
+    prefix_codes = (top [B or 1, P], mid [B or 1, P, 4], bot [B or 1, P, 16]): image completion, as `sampling_ihqgpt`'s
+    prefix_code_top / prefix_code_bot - positions < P given and returned unchanged, the rest sampled after them.
+    shared_prefix: every row has the same condition and prefix (None = detect; results are identical either way)."""
     if max_seq_len > model.max_seq_len:
         raise ValueError(f"max_seq_len={max_seq_len} exceeds the engine's {model.max_seq_len} top positions")
     k, p, t = _triple(top_k, "top_k"), _triple(top_p, "top_p"), _triple(softmax_temperature, "softmax_temperature")
@@ -188,8 +192,21 @@ def sampling_hqtransformer(model: HQTransformer, num_candidates: int, cond, top_
     ct = torch.empty(B, max_seq_len, dtype=torch.int64, device=dev)
     cm = torch.empty(B, max_seq_len, 4, dtype=torch.int64, device=dev)
     cb = torch.empty(B, max_seq_len, 16, dtype=torch.int64, device=dev)
+    P = 0
+    if prefix_codes is not None:
+        from .sampling import _rows_equal, prefix_rows
+        if len(prefix_codes) != 3:
+            raise ValueError(f"prefix_codes must be (top, mid, bot), got {len(prefix_codes)} tensors")
+        V = model.vocab_sizes
+        parts = prefix_rows([(prefix_codes[0], "prefix_codes[0]", V[0], ()), (prefix_codes[1], "prefix_codes[1]", V[1], (4,)),
+                             (prefix_codes[2], "prefix_codes[2]", V[2], (16,))], B, max_seq_len, dev)
+        P = parts[0].shape[1]
+        for dst, src in zip((ct, cm, cb), parts):
+            dst[:, :P] = src
+        if shared_prefix is None:
+            shared_prefix = B > 1 and _rows_equal(cond_t) and all(_rows_equal(t) for t in parts)
     eng.run(batch=B, seq_len=max_seq_len, pos_begin=0, pos_end=max_seq_len, sampling=sp, cond=cond_t, codes_top=ct,
-            codes_mid=cm, codes_bot=cb)
+            codes_mid=cm, codes_bot=cb, prefix_len=P, shared_prefix=bool(shared_prefix) and P > 0)
     return [ct, cm, cb]
 
 

@@ -20,7 +20,9 @@ def sampling_ihqgpt(model, num_candidates: int, cond, top_k_top: Optional[float]
                     top_p_bot: Optional[float] = None, softmax_temperature: List[float] = [1.0, 1.0],
                     is_tqdm: bool = True, use_fp16: bool = True, max_seq_len: int = 256, model_stage1=None,
                     given_top_code: Optional[torch.Tensor] = None, *, seed: Optional[int] = None,
-                    row_offset: int = 0, shared_prefix: Optional[bool] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+                    row_offset: int = 0, shared_prefix: Optional[bool] = None,
+                    prefix_code_top: Optional[torch.Tensor] = None,
+                    prefix_code_bot: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
     """utils/sampling.py:164-237.
 
     cond: class id (int, broadcast to the batch as in the reference :183-186, or an int64 [B] tensor for per-row
@@ -33,7 +35,13 @@ def sampling_ihqgpt(model, num_candidates: int, cond, top_k_top: Optional[float]
     (utils/utils.py:6-10) reproduces the whole run.
     shared_prefix (text models): one prompt sampled B times (the reference notebook repeats a prompt 8x) - the 64-token
     prefill runs once and its KV-cache rows are broadcast.  None = detect (all rows of `cond` equal); results are
-    identical either way."""
+    identical either way.
+    prefix_code_top [B or 1, P] / prefix_code_bot [B or 1, P, 4] (together, raster layout of the returned grids; a [1, ...]
+    row is broadcast over the batch): image completion - positions < P are given and returned unchanged, positions >= P
+    are sampled as the loop samples them after those codes (the same Philox counters: completing a grid's own prefix with
+    its seed re-draws the same stream).  The prefix goes through the spatial transformer in one causal pass.
+    `given_top_code` applies at positions >= P.  shared_prefix then means: every row has the same condition and the same
+    prefix (None = detect)."""
     if max_seq_len > model.max_seq_len:
         raise ValueError(f"max_seq_len={max_seq_len} exceeds the engine's {model.max_seq_len} top positions "
                          "(the scripts pass 64 for 8x8 top codes)")
@@ -56,11 +64,51 @@ def sampling_ihqgpt(model, num_candidates: int, cond, top_k_top: Optional[float]
             raise ValueError(f"given_top_code must be [B, >= {max_seq_len}], got {tuple(given_top_code.shape)}")
         if int(given.min()) < 0 or int(given.max()) >= model.vocab_size_top:
             raise IndexError(f"given_top_code out of range [0, {model.vocab_size_top})")
+    P = 0
+    if prefix_code_top is not None or prefix_code_bot is not None:
+        if prefix_code_top is None or prefix_code_bot is None:
+            raise ValueError("prefix_code_top and prefix_code_bot go together")
+        pt, pb = prefix_rows([(prefix_code_top, "prefix_code_top", model.vocab_size_top, ()),
+                              (prefix_code_bot, "prefix_code_bot", model.vocab_size_bot, (4,))], B, max_seq_len, dev)
+        P = pt.shape[1]
+        codes_top[:, :P] = pt
+        codes_bot[:, :P] = pb
+        if shared_prefix is None:
+            shared_prefix = B > 1 and _rows_equal(cond_t) and _rows_equal(pt) and _rows_equal(pb)
     if shared_prefix is None:
         shared_prefix = bool(model.use_txt_cond and cond_t is not None and B > 1 and bool((cond_t == cond_t[:1]).all()))
     eng.run(batch=B, seq_len=max_seq_len, pos_begin=0, pos_end=max_seq_len, sampling=sp, cond=cond_t,
-            given_top=given, codes_top=codes_top, codes_bot=codes_bot, shared_prefix=bool(shared_prefix))
+            given_top=given, codes_top=codes_top, codes_bot=codes_bot, shared_prefix=bool(shared_prefix), prefix_len=P)
     return codes_top, codes_bot
+
+
+def _rows_equal(t: Optional[torch.Tensor]) -> bool:
+    return t is None or bool((t == t[:1]).all())
+
+
+def prefix_rows(parts, B: int, max_seq_len: int, dev) -> List[torch.Tensor]:
+    """Checks the prefix code tensors of an image completion and returns them as int64 [B, P, ...] on `dev`.
+    parts: (tensor [B or 1, P, *tail], name, vocabulary size, tail) per code level; every level must have the same P, with
+    1 <= P < max_seq_len.  A [1, ...] tensor is broadcast over the batch."""
+    out, P = [], None
+    for t, name, vocab, tail in parts:
+        t = torch.as_tensor(t)
+        want = "[B or 1, P" + "".join(f", {w}" for w in tail) + "]"
+        if t.dim() != 2 + len(tail) or tuple(t.shape[2:]) != tuple(tail) or t.shape[0] not in (1, B):
+            raise ValueError(f"{name} must be {want} with B = {B}, got {tuple(t.shape)}")
+        if t.dtype.is_floating_point or t.dtype.is_complex or t.dtype == torch.bool:
+            raise ValueError(f"{name} must hold integer codes, got {t.dtype}")
+        if P is None:
+            P = t.shape[1]
+            if not 1 <= P < max_seq_len:
+                raise ValueError(f"prefix length {P} outside [1, max_seq_len={max_seq_len})")
+        elif t.shape[1] != P:
+            raise ValueError(f"{name} covers {t.shape[1]} positions, the other prefix tensors {P}")
+        t = t.to(device=dev, dtype=torch.int64)
+        if int(t.min()) < 0 or int(t.max()) >= vocab:
+            raise IndexError(f"{name} out of range [0, {vocab})")
+        out.append(t.expand(B, *t.shape[1:]).contiguous())
+    return out
 
 
 def encode_prompts(tokenizer, texts, context_length: int = 64) -> torch.Tensor:
@@ -120,6 +168,20 @@ def get_positional_encoding(inputs: torch.Tensor, mode: str = "1d") -> torch.Ten
         raise ValueError("%s positional encoding invalid" % mode)
     B, N = inputs.shape
     return torch.arange(N, device=inputs.device).repeat((B, 1))
+
+
+def grids_to_codes(codes_t: torch.Tensor, codes_b: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+    """The exact inverse of `codes_to_grids`: code grids as the reference's `stage1.get_codes` returns them, top [B, H, W]
+    and bottom [B, 2H, 2W], -> the sampler's raster layout codes_top [B, H*W], codes_bot [B, H*W, 4] (within-stack order
+    kh*2 + kw) - e.g. the prefix of an image completion."""
+    if codes_t.dim() != 3 or codes_b.dim() != 3 or codes_b.shape[0] != codes_t.shape[0] or \
+            tuple(codes_b.shape[1:]) != (2 * codes_t.shape[1], 2 * codes_t.shape[2]):
+        raise ValueError(f"grids must be top [B, H, W] and bottom [B, 2H, 2W], got {tuple(codes_t.shape)} and "
+                         f"{tuple(codes_b.shape)}")
+    B, H, W = codes_t.shape
+    top = codes_t.reshape(B, H * W)
+    bot = codes_b.reshape(B, H, 2, W, 2).permute(0, 1, 3, 2, 4).reshape(B, H * W, 4)
+    return top, bot
 
 
 def codes_to_grids(codes_top: torch.Tensor, codes_bot: torch.Tensor, H: int = 8) -> Tuple[torch.Tensor, torch.Tensor]:

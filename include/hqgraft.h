@@ -162,8 +162,15 @@ typedef struct hq_run_args {
   const int64_t* given_mid;  /* code_levels == 3 only: optional forced middle codes (teacher forcing, parity only) */
   int32_t shared_prefix;     /* text models, pos_begin == 0: 1 = every row of `cond` is the SAME prompt (one prompt sampled B
                                 times, as the reference notebook does): the 64-token prefill runs for row 0 only and its
-                                cached keys / values are broadcast to the other rows.  Results are identical to 0. */
-  int32_t reserved;
+                                cached keys / values are broadcast to the other rows.  Results are identical to 0.
+                                With prefix_len > 0 (any model, `sos` NULL): 1 = every row has the same `cond` AND the same
+                                prefix codes; the prefix pass runs for row 0 only and its cache rows are broadcast. */
+  int32_t prefix_len;        /* image completion: 0 = off.  P in [1, pos_end) with pos_begin == 0: the codes of positions < P are
+                                GIVEN - read from codes_top / codes_bot (/ codes_mid) and returned unchanged - and positions
+                                [P, pos_end) are sampled exactly as the loop samples them after those codes (same Philox
+                                counters).  The spatial KV cache of the prefix is computed in one causal pass over its
+                                T0 + P - 1 tokens (no depth pass, head or draw there).  given_top / given_bot / given_mid apply
+                                at positions >= P; logits are written for positions >= P only. */
 } hq_run_args;
 
 typedef struct hq_ctx hq_ctx;
@@ -217,7 +224,8 @@ int64_t hq_last_launch_count(const hq_ctx* ctx);
  * ran as a kernel of its own (batch <= 128, fp32 or fp16 engine, use_chain == 0). */
 int64_t hq_chain_launch_count(const hq_ctx* ctx);
 
-/* Bytes of device memory owned by the ctx (weights + KV cache + workspaces). */
+/* Bytes of device memory owned by the ctx (weights + KV cache + workspaces, including the image-completion workspace that
+ * the first run with a longer prefix (or a larger batch under one) grows; hq_reserve_batch frees it). */
 size_t hq_device_bytes(const hq_ctx* ctx);
 
 /* ---- test / measurement hooks (used by tests/ and bench.py, not by the sampling entry points) ---- */
@@ -277,6 +285,14 @@ int hq_debug_sample(const float* logits, int R, int V, float temperature, int to
  * variant: 0 = the engine's choice (bf16 / fp16: persistent ldmatrix/mma kernel), 1 = the scalar bulk-staged kernel. */
 int hq_debug_attention(int prec, const void* q, const void* K, const void* V, void* out, int B, int n_heads,
                        int t_stride, int n_keys, int variant, void* stream);
+
+/* Causal attention of the image-completion prefix pass: query i of image b (q / out [B, n_q, D]) over keys 0 .. i of its
+ * cache rows (K / V [B, t_stride, D]), D = n_heads * 64, device pointers in the precision's activation type.
+ * variant 0: the kernel of the prefix pass - bf16 / fp16: the tensor-core prefix kernel, fp32: the per-(query, head) warp
+ * kernel the fp32 engine runs there; variant 1: the per-(query, head) warp kernel at every precision (what the text prefill
+ * runs).  1 <= n_q <= min(t_stride, 128). */
+int hq_debug_attention_prefix(int prec, const void* q, const void* K, const void* V, void* out, int B, int n_heads,
+                              int t_stride, int n_q, int variant, void* stream);
 
 /* Times the single-query KV-cache attention kernel alone at cache length `n_keys` for batch B on the
  * ctx's cache (events on `stream`); returns mean microseconds over `iters` launches in *usec. */
