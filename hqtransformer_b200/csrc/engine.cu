@@ -1564,26 +1564,42 @@ static void draw(hq_ctx* ctx, cudaStream_t st, const SampleArgs& sa, bool fused)
     launch_sample(ctx, st, sa);
 }
 
-// One top position (SURVEY.md 8a-spec): spatial step, depth pass 0, draw top, depth pass 1, draw 4 bottoms.
+// Threads of the row-wise embedding kernels: one float4 per thread, so every gather of a row is in flight at once (a single
+// memory round trip after the codes).
+static int embed_threads(int D) {
+  const int n = (D / 4 + 31) / 32 * 32;
+  return n > 1024 ? 1024 : n;
+}
+
+// Spatial input tokens (kernels.cuh K1): row r of x gets the token of image r / N in cache slot t_begin + r % N.
+static void embed_tokens(hq_ctx* ctx, cudaStream_t st, const RunFlags& f, float* x, int S, int t_begin, int N, int rows,
+                         const char* tag) {
+  EmbedArgs ea;
+  ea.x = x; ea.sos_table = ctx->sos_table; ea.sos_override = f.sos_override ? ctx->sos_override : nullptr;
+  ea.cond = ctx->cond; ea.E_txt = ctx->E_txt; ea.P_txt = ctx->P_txt;
+  ea.E_top = ctx->E_top; ea.E_mid = ctx->E_mid; ea.E_bot = ctx->E_bot; ea.P_top = ctx->P_top; ea.P_emb = ctx->P_emb;
+  ea.codes_top = ctx->codes_top; ea.codes_mid = ctx->codes_mid; ea.codes_bot = ctx->codes_bot;
+  ea.D = ctx->D; ea.S = S; ea.T0 = ctx->T0; ea.cond_kind = ctx->cfg.cond_kind;
+  ea.emb_kind = ctx->cfg.embedding_kind; ea.P_top_h = ctx->P_top_h; ea.P_top_w = ctx->P_top_w; ea.Hpos = ctx->Hpos;
+  launch_k(ctx, st, tag, ctx->levels == 3 ? embed3_kernel : embed_kernel, dim3(rows), dim3(embed_threads(ctx->D)), 0, ea,
+           t_begin, N);
+}
+
+// Spatial step of one top position, either hierarchy: input token(s), L blocks over the KV cache, hs = ln_f(x) and the depth
+// start token y = hs + sos_depth.  Returns whether the persistent chain kernel is recording (the caller ends the chain).
 template <typename AT>
-static void run_position(hq_ctx* ctx, cudaStream_t st, int B, int S, int pos, const RunFlags& f) {
+static bool spatial_step(hq_ctx* ctx, cudaStream_t st, int B, int S, int pos, const RunFlags& f) {
   const int D = ctx->D, T0 = ctx->T0, Tc = ctx->Tc;
-  const bool txt = ctx->cfg.cond_kind == HQ_COND_TXT;
-  const bool prefill = txt && pos == 0;
+  const bool prefill = ctx->cfg.cond_kind == HQ_COND_TXT && pos == 0;
   const bool shared = prefill && f.shared_prefix && B > 1;
   const int Bp = shared ? 1 : B;                      // images the prefill runs for
   const int M = prefill ? Bp * T0 : B;
   AT* kc = static_cast<AT*>(ctx->kc);
   AT* vc = static_cast<AT*>(ctx->vc);
-  AT* kd = static_cast<AT*>(ctx->kd);
-  AT* vd = static_cast<AT*>(ctx->vd);
-  AT* h = static_cast<AT*>(ctx->h.ptr);
   const size_t lstride = static_cast<size_t>(ctx->max_batch) * Tc * D;
-  const size_t dstride = static_cast<size_t>(ctx->max_batch) * 5 * D;
+  Fold fold_x;   // split-K partial sums pending on the spatial residual stream
+  const int tok = (pos == 0) ? 0 : T0 + pos - 1;     // cache slot of this position's (first) token
 
-  // one float4 per thread: every gather of a row is in flight at once (a single memory round trip after the codes)
-  const int eb = (D / 4 + 31) / 32 * 32 > 1024 ? 1024 : (D / 4 + 31) / 32 * 32;
-  Fold fold_x, fold_y;   // split-K partial sums pending on the spatial / depth residual stream
   // ---- K1: input token(s) ----
   // The first kernel of a position is NOT a programmatic dependent: it starts only when the previous position has
   // completed.  Programmatic launches cascade - kernel N+1 may become resident as soon as N has started, N+2 as soon as
@@ -1592,21 +1608,10 @@ static void run_position(hq_ctx* ctx, cudaStream_t st, int B, int S, int pos, co
   // griddepcontrol.wait; a barrier per position is what makes "earlier positions are complete" true.  (Found by the
   // asymmetric golden: without it a second run read the previous run's keys, graph + PDL only.)  Cost: ~1 us per position.
   ctx->full_dependency_next = true;
-  if (prefill) {
-    launch_k(ctx, st, "embed_txt", embed_txt_kernel, dim3(M), dim3(eb), 0, ctx->x, f.sos_override ? ctx->sos_override : nullptr,
-             ctx->cond, ctx->E_txt, ctx->P_txt, T0, D);
-  } else {
-    EmbedArgs ea;
-    ea.x = ctx->x; ea.sos_table = ctx->sos_table; ea.sos_override = f.sos_override ? ctx->sos_override : nullptr;
-    ea.cond = ctx->cond; ea.E_top = ctx->E_top; ea.E_bot = ctx->E_bot; ea.P_top = ctx->P_top; ea.P_emb = ctx->P_emb;
-    ea.codes_top = ctx->codes_top; ea.codes_bot = ctx->codes_bot; ea.D = D; ea.S = S; ea.pos = pos;
-    ea.cond_kind = ctx->cfg.cond_kind;
-    ea.emb_kind = ctx->cfg.embedding_kind; ea.P_top_h = ctx->P_top_h; ea.P_top_w = ctx->P_top_w; ea.Hpos = ctx->Hpos;
-    launch_k(ctx, st, "embed", embed_kernel, dim3(B), dim3(eb), 0, ea);
-  }
+  if (prefill) embed_tokens(ctx, st, f, ctx->x, S, 0, T0, M, "embed_txt");
+  else embed_tokens(ctx, st, f, ctx->x, S, tok, 1, B, "embed");
 
   // ---- spatial transformer: L blocks over the KV cache ----
-  const int tok = (pos == 0) ? 0 : T0 + pos - 1;     // cache slot of this position's (first) token
   // persistent chain kernel: every run of ops between two cache attentions (and the whole depth transformer) is one launch
   const bool chain = std::is_same<AT, bf16>::value && !prefill && chain_enabled(ctx, B);
   if (chain) chain_begin(ctx, tok, pos, S);
@@ -1627,10 +1632,23 @@ static void run_position(hq_ctx* ctx, cudaStream_t st, int B, int S, int pos, co
              ctx->sos_depth, ctx->yd, prefill ? Bp : B, D, prefill ? T0 : 1, prefill ? T0 - 1 : 0, fold_x.partial, fold_x.n, fold_x.stride,
              fold_x.bias, 1, ctx->cfg.model_type == HQ_MODEL_BIDIRECTIONAL ? 5 : 1);
   }
-  fold_x = Fold();
   if (shared)    // one prompt, B samples: image 0's prefix cache rows (all layers) and depth start token -> images 1..B-1
     launch_k(ctx, st, "broadcast_prefix", broadcast_prefix_kernel<AT>, dim3(T0, ctx->L, B - 1), dim3(256), 0, kc, vc, ctx->yd,
              ctx->max_batch, Tc, D);
+  return chain;
+}
+
+// One top position (SURVEY.md 8a-spec): spatial step, depth pass 0, draw top, depth pass 1, draw 4 bottoms.
+template <typename AT>
+static void run_position(hq_ctx* ctx, cudaStream_t st, int B, int S, int pos, const RunFlags& f) {
+  const int D = ctx->D;
+  AT* kd = static_cast<AT*>(ctx->kd);
+  AT* vd = static_cast<AT*>(ctx->vd);
+  AT* h = static_cast<AT*>(ctx->h.ptr);
+  const size_t dstride = static_cast<size_t>(ctx->max_batch) * 5 * D;
+  const int eb = embed_threads(D);
+  Fold fold_y;   // split-K partial sums pending on the depth residual stream
+  const bool chain = spatial_step<AT>(ctx, st, B, S, pos, f);
 
   SampleArgs sa;
   memset(&sa, 0, sizeof(sa));
@@ -1689,7 +1707,7 @@ static void run_position(hq_ctx* ctx, cudaStream_t st, int B, int S, int pos, co
 
   // ---- depth pass 1 -> 4 bottom logits ----
   if (chain) {
-    chain_begin(ctx, tok, pos, S);
+    chain_begin(ctx, ctx->T0 + pos - 1, pos, S);   // the spatial step's cache slot (the chain never runs the text prefill)
     ChainOp* op = chain_push(ctx, CH_OP_EMBED_DEPTH, "embed_depth");
     op->y = ctx->yd; op->E = ctx->E_top_depth; op->P = ctx->P_depth; op->codes_top = ctx->codes_top; op->B = B; op->D = D;
   } else {
@@ -1714,30 +1732,14 @@ static void run_position(hq_ctx* ctx, cudaStream_t st, int B, int S, int pos, co
 // and one set of (temperature, top-k, top-p) per level, 21 draws (Philox slots 0..20).
 template <typename AT>
 static void run_position3(hq_ctx* ctx, cudaStream_t st, int B, int S, int pos, const RunFlags& f) {
-  const int D = ctx->D, Tc = ctx->Tc;
-  AT* kc = static_cast<AT*>(ctx->kc);
-  AT* vc = static_cast<AT*>(ctx->vc);
+  const int D = ctx->D;
   AT* kd = static_cast<AT*>(ctx->kd);
   AT* vd = static_cast<AT*>(ctx->vd);
   AT* h = static_cast<AT*>(ctx->h.ptr);
-  const size_t lstride = static_cast<size_t>(ctx->max_batch) * Tc * D;
   const size_t dstride = static_cast<size_t>(ctx->max_batch) * 21 * D;
-  const int eb = (D / 4 + 31) / 32 * 32 > 1024 ? 1024 : (D / 4 + 31) / 32 * 32;
-  Fold fold_x, fold_y;
-  ctx->full_dependency_next = true;             // one full dependency per position (see run_position)
-  Embed3Args ea;
-  ea.x = ctx->x; ea.sos_table = ctx->sos_table; ea.sos_override = f.sos_override ? ctx->sos_override : nullptr;
-  ea.cond = ctx->cond; ea.E0 = ctx->E_top; ea.E1 = ctx->E_mid; ea.E2 = ctx->E_bot; ea.P_top = ctx->P_top; ea.P_emb = ctx->P_emb;
-  ea.codes_top = ctx->codes_top; ea.codes_mid = ctx->codes_mid; ea.codes_bot = ctx->codes_bot;
-  ea.D = D; ea.S = S; ea.pos = pos; ea.cond_kind = ctx->cfg.cond_kind;
-  launch_k(ctx, st, "embed", embed3_kernel, dim3(B), dim3(eb), 0, ea);
-  const int tok = pos;                          // cache slot (no text prefix)
-  for (int l = 0; l < ctx->L; ++l)
-    run_block<AT>(ctx, st, ctx->blocks[l], ctx->x, B, 0, kc + l * lstride, vc + l * lstride, 1, Tc, tok, tok + 1, 0, &fold_x);
-  launch_k(ctx, st, "layernorm_f", fold_x.n > 3 ? layernorm_kernel<float, LN_MAXFOLD> : layernorm_kernel<float, 3>, dim3(B),
-           dim3(LN_THREADS), 0, ctx->x, ctx->lnf_g, ctx->lnf_b, ctx->sos_depth, ctx->yd, B, D, 1, 0, fold_x.partial, fold_x.n,
-           fold_x.stride, fold_x.bias, 1, 1);
-  fold_x = Fold();
+  const int eb = embed_threads(D);
+  Fold fold_y;
+  spatial_step<AT>(ctx, st, B, S, pos, f);     // never the chain kernel: it runs the 2-level model only
 
   SampleArgs sa;
   memset(&sa, 0, sizeof(sa));
@@ -1785,27 +1787,10 @@ static void run_prefix(hq_ctx* ctx, cudaStream_t st, int B, int S, const RunFlag
   AT* kc = static_cast<AT*>(ctx->kc);
   AT* vc = static_cast<AT*>(ctx->vc);
   const size_t lstride = static_cast<size_t>(ctx->max_batch) * Tc * D;
-  const int eb = (D / 4 + 31) / 32 * 32 > 1024 ? 1024 : (D / 4 + 31) / 32 * 32;
   // the prefix workspace stands in for the step activations while the pass runs
   std::swap(ctx->h, ctx->pre_h); std::swap(ctx->att, ctx->pre_att); std::swap(ctx->mlp, ctx->pre_mlp); std::swap(ctx->q, ctx->pre_q);
   ctx->full_dependency_next = true;                    // as every position's first kernel (see run_position)
-  if (ctx->levels == 3) {
-    Embed3Args ea;
-    ea.x = ctx->pre_x; ea.sos_table = ctx->sos_table; ea.sos_override = f.sos_override ? ctx->sos_override : nullptr;
-    ea.cond = ctx->cond; ea.E0 = ctx->E_top; ea.E1 = ctx->E_mid; ea.E2 = ctx->E_bot; ea.P_top = ctx->P_top; ea.P_emb = ctx->P_emb;
-    ea.codes_top = ctx->codes_top; ea.codes_mid = ctx->codes_mid; ea.codes_bot = ctx->codes_bot;
-    ea.D = D; ea.S = S; ea.pos = 0; ea.cond_kind = ctx->cfg.cond_kind;
-    launch_k(ctx, st, "embed_prefix", embed3_prefix_kernel, dim3(M), dim3(eb), 0, ea, N);
-  } else {
-    EmbedArgs ea;
-    ea.x = ctx->pre_x; ea.sos_table = ctx->sos_table; ea.sos_override = f.sos_override ? ctx->sos_override : nullptr;
-    ea.cond = ctx->cond; ea.E_top = ctx->E_top; ea.E_bot = ctx->E_bot; ea.P_top = ctx->P_top; ea.P_emb = ctx->P_emb;
-    ea.codes_top = ctx->codes_top; ea.codes_bot = ctx->codes_bot; ea.D = D; ea.S = S; ea.pos = 0;
-    ea.cond_kind = ctx->cfg.cond_kind;
-    ea.emb_kind = ctx->cfg.embedding_kind; ea.P_top_h = ctx->P_top_h; ea.P_top_w = ctx->P_top_w; ea.Hpos = ctx->Hpos;
-    launch_k(ctx, st, "embed_prefix", embed_prefix_kernel, dim3(M), dim3(eb), 0, ea, static_cast<const float*>(ctx->E_txt),
-             static_cast<const float*>(ctx->P_txt), T0, N);
-  }
+  embed_tokens(ctx, st, f, ctx->pre_x, S, 0, N, M, "embed_prefix");
   ctx->prefix_pass = true;
   Fold fold;
   for (int l = 0; l + 1 < L; ++l)

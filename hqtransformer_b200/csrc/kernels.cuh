@@ -8,44 +8,71 @@
 namespace hq {
 
 // ------------------------------------------------------------------------------------------------
-// K1: spatial-transformer input token (hierarchical_ar.py:493-499, 506-544 with emb_blocks empty):
-//   pos == 0 : x[b] = sos row (class embedding / learned sos / caller-provided override)
-//   pos  > 0 : x[b] = mean_5( {E_top[c_t] + P_top[pos-1], E_bot[c_b0..3]} + P_emb[0..4] ), codes of pos-1
-// One CTA per batch row.
+// K1: spatial-transformer input tokens (hierarchical_ar.py:493-499, 506-544 with emb_blocks empty; 3 levels:
+// hqtransformer.py:453-487).  Row r of a launch (a, t_begin, N) writes the token of image b = r / N that sits in cache
+// slot t = t_begin + r % N:
+//   t <  T0 : the conditioning row (embed_cond_row)
+//   t >= T0 : the code stack of position p = t - T0
+//     embed_kernel  (2 levels): mean_5( {E_top[c_t] + P_top[p], E_bot[c_b0..3]} + P_emb[0..4] )
+//     embed3_kernel (3 levels): mean_21( {E_top[c_top] + P_top[p], E_mid[c_mid 0..3], E_bot[c_bot 0..15]} + P_emb[0..20] )
+// The step (t_begin = its slot, N = 1), the text prefill (0, T0) and the completion prefix (0, T0 + P - 1) all embed here,
+// so a token of the prefix pass is bit-identical to the one the step path writes for the same slot.  One CTA per row.
 // ------------------------------------------------------------------------------------------------
 struct EmbedArgs {
-  float* x;                 // [B, D]
+  float* x;                 // [rows, D]
   const float* sos_table;   // cls: [n_classes, D]; uncond: [D]
-  const float* sos_override;// optional [B, D]
-  const int64_t* cond;      // cls: [B]
-  const float* E_top; const float* E_bot; const float* P_top; const float* P_emb;
+  const float* sos_override;// optional [B, T0, D]
+  const int64_t* cond;      // cls: [B]; text: [B, T0] token ids
+  const float* E_txt; const float* P_txt;   // text: [vocab_txt, D], [T0, D]
+  const float* E_top; const float* E_mid; const float* E_bot; const float* P_top; const float* P_emb;
   const int64_t* codes_top; // [B, S]
-  const int64_t* codes_bot; // [B, S, 4]
-  int D, S, pos, cond_kind;
-  // variants (SURVEY.md 8f-3)
+  const int64_t* codes_mid; // [B, S, 4]  (3 levels)
+  const int64_t* codes_bot; // [B, S, 4]; 3 levels: [B, S, 16]
+  int D, S, T0, cond_kind;
+  // variants of the 2-level model (SURVEY.md 8f-3)
   int emb_kind;             // 0: 'transformer1' (mean of the 5 stack tokens + pos_emb_emb); 1: 'reduce' (hierarchical_ar.py:522-526)
   const float* P_top_h;     // position_embedding == '2d' (:508-514): P_top_h[p / Hpos] + P_top_w[p % Hpos]; else nullptr
   const float* P_top_w;
   int Hpos;
 };
 
-__global__ void __launch_bounds__(1024) embed_kernel(int trace_id, EmbedArgs a) {
+// Conditioning row t < T0 of image b: row b * T0 + t of the `sos` override, E_txt[ids[b, t]] + P_txt[t] (text,
+// sampling.py:187-190), the class embedding of cond[b], or the learned sos.
+__device__ __forceinline__ void embed_cond_row(const EmbedArgs& a, float4* xo, int b, int t) {
+  const int n4 = a.D / 4;
+  const float* src;
+  if (a.sos_override != nullptr) {
+    src = a.sos_override + (static_cast<size_t>(b) * a.T0 + t) * a.D;
+  } else if (a.cond_kind == HQ_COND_TXT) {
+    const float4* e = reinterpret_cast<const float4*>(a.E_txt + static_cast<size_t>(a.cond[static_cast<size_t>(b) * a.T0 + t]) * a.D);
+    const float4* p = reinterpret_cast<const float4*>(a.P_txt + static_cast<size_t>(t) * a.D);
+    for (int i = threadIdx.x; i < n4; i += blockDim.x) {
+      float4 u = e[i], c = p[i];
+      xo[i] = make_float4(u.x + c.x, u.y + c.y, u.z + c.z, u.w + c.w);
+    }
+    return;
+  } else if (a.cond_kind == HQ_COND_CLS) {
+    src = a.sos_table + static_cast<size_t>(a.cond[b]) * a.D;
+  } else {
+    src = a.sos_table;
+  }
+  const float4* s4 = reinterpret_cast<const float4*>(src);
+  for (int i = threadIdx.x; i < n4; i += blockDim.x) xo[i] = s4[i];
+}
+
+__global__ void __launch_bounds__(1024) embed_kernel(int trace_id, EmbedArgs a, int t_begin, int N) {
   TraceScope trace_scope(trace_id);
   pdl_launch_dependents();   // programmatic dependent launch: let the next kernel get resident ...
   pdl_wait();                // ... and wait for the previous kernel's results (no-ops without the launch attribute)
-  const int b = blockIdx.x;
-  float4* xo = reinterpret_cast<float4*>(a.x + static_cast<size_t>(b) * a.D);
-  const int n4 = a.D / 4;
-  if (a.pos == 0) {
-    const float* src;
-    if (a.sos_override != nullptr) src = a.sos_override + static_cast<size_t>(b) * a.D;
-    else if (a.cond_kind == HQ_COND_CLS) src = a.sos_table + static_cast<size_t>(a.cond[b]) * a.D;
-    else src = a.sos_table;
-    const float4* s4 = reinterpret_cast<const float4*>(src);
-    for (int i = threadIdx.x; i < n4; i += blockDim.x) xo[i] = s4[i];
+  const int row = blockIdx.x;
+  const int b = row / N, t = t_begin + row % N;
+  float4* xo = reinterpret_cast<float4*>(a.x + static_cast<size_t>(row) * a.D);
+  if (t < a.T0) {
+    embed_cond_row(a, xo, b, t);
     return;
   }
-  const int p = a.pos - 1;
+  const int n4 = a.D / 4;
+  const int p = t - a.T0;
   const int64_t ct = a.codes_top[static_cast<size_t>(b) * a.S + p];
   const int64_t* cbp = a.codes_bot + (static_cast<size_t>(b) * a.S + p) * 4;
   const float4* et = reinterpret_cast<const float4*>(a.E_top + static_cast<size_t>(ct) * a.D);
@@ -61,11 +88,11 @@ __global__ void __launch_bounds__(1024) embed_kernel(int trace_id, EmbedArgs a) 
 #pragma unroll
     for (int j = 0; j < 4; ++j) ebq[j] = a.E_bot + static_cast<size_t>(cbp[j]) * Dq;
     for (int i = threadIdx.x; i < n4; i += blockDim.x) {
-      const float4 t = et[i];
+      const float4 u = et[i];
       float4 q = pt[i];
       if (pos2d) { const float4 w = pw[i]; q.x += w.x; q.y += w.y; q.z += w.z; q.w += w.w; }
       // elements 4i .. 4i+3 -> bottom code 0..3, element i of its narrow embedding
-      xo[i] = make_float4((t.x + q.x) + ebq[0][i], (t.y + q.y) + ebq[1][i], (t.z + q.z) + ebq[2][i], (t.w + q.w) + ebq[3][i]);
+      xo[i] = make_float4((u.x + q.x) + ebq[0][i], (u.y + q.y) + ebq[1][i], (u.z + q.z) + ebq[2][i], (u.w + q.w) + ebq[3][i]);
     }
     return;
   }
@@ -74,10 +101,10 @@ __global__ void __launch_bounds__(1024) embed_kernel(int trace_id, EmbedArgs a) 
   for (int j = 0; j < 4; ++j) eb[j] = reinterpret_cast<const float4*>(a.E_bot + static_cast<size_t>(cbp[j]) * a.D);
   const float4* pe = reinterpret_cast<const float4*>(a.P_emb);
   for (int i = threadIdx.x; i < n4; i += blockDim.x) {
-    float4 t = et[i], q = pt[i], e0 = pe[i];
+    float4 u = et[i], q = pt[i], e0 = pe[i];
     if (pos2d) { const float4 w = pw[i]; q.x += w.x; q.y += w.y; q.z += w.z; q.w += w.w; }
     float4 acc;
-    acc.x = (t.x + q.x) + e0.x; acc.y = (t.y + q.y) + e0.y; acc.z = (t.z + q.z) + e0.z; acc.w = (t.w + q.w) + e0.w;
+    acc.x = (u.x + q.x) + e0.x; acc.y = (u.y + q.y) + e0.y; acc.z = (u.z + q.z) + e0.z; acc.w = (u.w + q.w) + e0.w;
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
       float4 e = eb[j][i], pj = pe[(j + 1) * n4 + i];
@@ -88,27 +115,43 @@ __global__ void __launch_bounds__(1024) embed_kernel(int trace_id, EmbedArgs a) 
   }
 }
 
-// text prefix embedding (sampling.py:187-190): x[b*T + t] = E_txt[ids[b, t]] + P_txt[t]
-__global__ void __launch_bounds__(1024)
-embed_txt_kernel(int trace_id, float* x, const float* sos_override, const int64_t* ids, const float* E_txt, const float* P_txt,
-                 int T, int D) {
+// 3-level HQTransformer (SURVEY.md 8f-2; class / unconditional only, so T0 = 1)
+__global__ void __launch_bounds__(1024) embed3_kernel(int trace_id, EmbedArgs a, int t_begin, int N) {
   TraceScope trace_scope(trace_id);
-  pdl_launch_dependents();   // programmatic dependent launch: let the next kernel get resident ...
-  pdl_wait();                // ... and wait for the previous kernel's results (no-ops without the launch attribute)
-  const int row = blockIdx.x;  // b*T + t
-  const int t = row % T;
-  float4* xo = reinterpret_cast<float4*>(x + static_cast<size_t>(row) * D);
-  const int n4 = D / 4;
-  if (sos_override != nullptr) {
-    const float4* s4 = reinterpret_cast<const float4*>(sos_override + static_cast<size_t>(row) * D);
-    for (int i = threadIdx.x; i < n4; i += blockDim.x) xo[i] = s4[i];
+  pdl_launch_dependents();
+  pdl_wait();
+  const int row = blockIdx.x;
+  const int b = row / N, t = t_begin + row % N;
+  float4* xo = reinterpret_cast<float4*>(a.x + static_cast<size_t>(row) * a.D);
+  if (t < a.T0) {
+    embed_cond_row(a, xo, b, t);
     return;
   }
-  const float4* e = reinterpret_cast<const float4*>(E_txt + static_cast<size_t>(ids[row]) * D);
-  const float4* p = reinterpret_cast<const float4*>(P_txt + static_cast<size_t>(t) * D);
+  const int n4 = a.D / 4;
+  const int p = t - a.T0;
+  __shared__ const float* rows[21];
+  if (threadIdx.x < 21) {
+    const size_t bp = static_cast<size_t>(b) * a.S + p;
+    const int j = threadIdx.x;
+    rows[j] = j == 0 ? a.E_top + static_cast<size_t>(a.codes_top[bp]) * a.D
+            : j < 5 ? a.E_mid + static_cast<size_t>(a.codes_mid[bp * 4 + (j - 1)]) * a.D
+                    : a.E_bot + static_cast<size_t>(a.codes_bot[bp * 16 + (j - 5)]) * a.D;
+  }
+  __syncthreads();   // block-uniform: t is the same for the whole CTA
+  const float4* pt = reinterpret_cast<const float4*>(a.P_top + static_cast<size_t>(p) * a.D);
+  const float4* pe = reinterpret_cast<const float4*>(a.P_emb);
   for (int i = threadIdx.x; i < n4; i += blockDim.x) {
-    float4 a = e[i], c = p[i];
-    xo[i] = make_float4(a.x + c.x, a.y + c.y, a.z + c.z, a.w + c.w);
+    // the order of the reference: cat([e0 + pos, e1.., e2..]) + pos_emb_emb, then mean over the 21 tokens (sequential sum)
+    const float4 u = reinterpret_cast<const float4*>(rows[0])[i], q = pt[i], e0 = pe[i];
+    float4 acc;
+    acc.x = (u.x + q.x) + e0.x; acc.y = (u.y + q.y) + e0.y; acc.z = (u.z + q.z) + e0.z; acc.w = (u.w + q.w) + e0.w;
+#pragma unroll 4
+    for (int j = 1; j < 21; ++j) {
+      const float4 e = reinterpret_cast<const float4*>(rows[j])[i], pj = pe[j * n4 + i];
+      acc.x += e.x + pj.x; acc.y += e.y + pj.y; acc.z += e.z + pj.z; acc.w += e.w + pj.w;
+    }
+    acc.x /= 21.0f; acc.y /= 21.0f; acc.z /= 21.0f; acc.w /= 21.0f;
+    xo[i] = acc;
   }
 }
 
@@ -132,60 +175,6 @@ embed_depth_kernel(int trace_id, float* y, const float* E_top_depth, const float
       reinterpret_cast<float4*>(y + (static_cast<size_t>(b) * 4 + j) * D)[i] =
           make_float4(a.x + c.x, a.y + c.y, a.z + c.z, a.w + c.w);
     }
-  }
-}
-
-// 3-level HQTransformer (SURVEY.md 8f-2), spatial input token (hqtransformer.py:453-487, emb_blocks empty):
-//   pos == 0 : x[b] = sos row;  pos > 0 : x[b] = mean_21( {E0[c_top] + P_top[pos-1], E1[c_mid 0..3], E2[c_bot 0..15]} + P_emb[0..20] )
-struct Embed3Args {
-  float* x;
-  const float* sos_table; const float* sos_override; const int64_t* cond;
-  const float* E0; const float* E1; const float* E2; const float* P_top; const float* P_emb;
-  const int64_t* codes_top;   // [B, S]
-  const int64_t* codes_mid;   // [B, S, 4]
-  const int64_t* codes_bot;   // [B, S, 16]
-  int D, S, pos, cond_kind;
-};
-__global__ void __launch_bounds__(1024) embed3_kernel(int trace_id, Embed3Args a) {
-  TraceScope trace_scope(trace_id);
-  pdl_launch_dependents();
-  pdl_wait();
-  const int b = blockIdx.x;
-  float4* xo = reinterpret_cast<float4*>(a.x + static_cast<size_t>(b) * a.D);
-  const int n4 = a.D / 4;
-  if (a.pos == 0) {
-    const float* src;
-    if (a.sos_override != nullptr) src = a.sos_override + static_cast<size_t>(b) * a.D;
-    else if (a.cond_kind == HQ_COND_CLS) src = a.sos_table + static_cast<size_t>(a.cond[b]) * a.D;
-    else src = a.sos_table;
-    const float4* s4 = reinterpret_cast<const float4*>(src);
-    for (int i = threadIdx.x; i < n4; i += blockDim.x) xo[i] = s4[i];
-    return;
-  }
-  const int p = a.pos - 1;
-  __shared__ const float* rows[21];
-  if (threadIdx.x < 21) {
-    const size_t bp = static_cast<size_t>(b) * a.S + p;
-    const int j = threadIdx.x;
-    rows[j] = j == 0 ? a.E0 + static_cast<size_t>(a.codes_top[bp]) * a.D
-            : j < 5 ? a.E1 + static_cast<size_t>(a.codes_mid[bp * 4 + (j - 1)]) * a.D
-                    : a.E2 + static_cast<size_t>(a.codes_bot[bp * 16 + (j - 5)]) * a.D;
-  }
-  __syncthreads();
-  const float4* pt = reinterpret_cast<const float4*>(a.P_top + static_cast<size_t>(p) * a.D);
-  const float4* pe = reinterpret_cast<const float4*>(a.P_emb);
-  for (int i = threadIdx.x; i < n4; i += blockDim.x) {
-    // the order of the reference: cat([e0 + pos, e1.., e2..]) + pos_emb_emb, then mean over the 21 tokens (sequential sum)
-    const float4 t = reinterpret_cast<const float4*>(rows[0])[i], q = pt[i], e0 = pe[i];
-    float4 acc;
-    acc.x = (t.x + q.x) + e0.x; acc.y = (t.y + q.y) + e0.y; acc.z = (t.z + q.z) + e0.z; acc.w = (t.w + q.w) + e0.w;
-#pragma unroll 4
-    for (int j = 1; j < 21; ++j) {
-      const float4 e = reinterpret_cast<const float4*>(rows[j])[i], pj = pe[j * n4 + i];
-      acc.x += e.x + pj.x; acc.y += e.y + pj.y; acc.z += e.z + pj.z; acc.w += e.w + pj.w;
-    }
-    acc.x /= 21.0f; acc.y /= 21.0f; acc.z /= 21.0f; acc.w /= 21.0f;
-    xo[i] = acc;
   }
 }
 
@@ -241,128 +230,6 @@ broadcast_prefix_kernel(int trace_id, AT* K, AT* V, float* yd, int Bmax, int Tc,
   if (t == 0 && l == 0)
     for (int i = threadIdx.x * 4; i < D; i += blockDim.x * 4)
       *reinterpret_cast<float4*>(yd + static_cast<size_t>(b) * D + i) = *reinterpret_cast<const float4*>(yd + i);
-}
-
-// Image completion (hq_run_args.prefix_len = P): the spatial input tokens of the given prefix, all of them in one launch.
-//   row r = b * N + t, N = T0 + P - 1 tokens per image:
-//   t <  T0 : the conditioning row - `sos` override, E_txt[ids[b, t]] + P_txt[t] (text), sos table (class / unconditional)
-//   t >= T0 : the stack of position p = t - T0 (0 .. P - 2), what embed_kernel writes at pos = p + 1
-// Every float operation is the one of embed_kernel / embed_txt_kernel, in the same order, so each token is bit-identical
-// to the one the step path embeds (the arithmetic is restated here so that those kernels stay exactly as they are).
-// One CTA per row.
-__global__ void __launch_bounds__(1024)
-embed_prefix_kernel(int trace_id, EmbedArgs a, const float* __restrict__ E_txt, const float* __restrict__ P_txt, int T0, int N) {
-  TraceScope trace_scope(trace_id);
-  pdl_launch_dependents();
-  pdl_wait();
-  const int row = blockIdx.x;
-  const int b = row / N, t = row % N;
-  float4* xo = reinterpret_cast<float4*>(a.x + static_cast<size_t>(row) * a.D);
-  const int n4 = a.D / 4;
-  if (t < T0) {
-    const float* src;
-    if (a.sos_override != nullptr) {
-      src = a.sos_override + (static_cast<size_t>(b) * T0 + t) * a.D;
-    } else if (a.cond_kind == HQ_COND_TXT) {
-      const float4* e = reinterpret_cast<const float4*>(E_txt + static_cast<size_t>(a.cond[static_cast<size_t>(b) * T0 + t]) * a.D);
-      const float4* p = reinterpret_cast<const float4*>(P_txt + static_cast<size_t>(t) * a.D);
-      for (int i = threadIdx.x; i < n4; i += blockDim.x) {
-        float4 u = e[i], c = p[i];
-        xo[i] = make_float4(u.x + c.x, u.y + c.y, u.z + c.z, u.w + c.w);
-      }
-      return;
-    } else if (a.cond_kind == HQ_COND_CLS) {
-      src = a.sos_table + static_cast<size_t>(a.cond[b]) * a.D;
-    } else {
-      src = a.sos_table;
-    }
-    const float4* s4 = reinterpret_cast<const float4*>(src);
-    for (int i = threadIdx.x; i < n4; i += blockDim.x) xo[i] = s4[i];
-    return;
-  }
-  const int p = t - T0;
-  const int64_t ct = a.codes_top[static_cast<size_t>(b) * a.S + p];
-  const int64_t* cbp = a.codes_bot + (static_cast<size_t>(b) * a.S + p) * 4;
-  const float4* et = reinterpret_cast<const float4*>(a.E_top + static_cast<size_t>(ct) * a.D);
-  const bool pos2d = a.P_top_h != nullptr;
-  const float4* pt = reinterpret_cast<const float4*>(pos2d ? a.P_top_h + static_cast<size_t>(p / a.Hpos) * a.D
-                                                           : a.P_top + static_cast<size_t>(p) * a.D);
-  const float4* pw = pos2d ? reinterpret_cast<const float4*>(a.P_top_w + static_cast<size_t>(p % a.Hpos) * a.D) : nullptr;
-  if (a.emb_kind == 1) {
-    const int Dq = a.D / 4;
-    const float* ebq[4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) ebq[j] = a.E_bot + static_cast<size_t>(cbp[j]) * Dq;
-    for (int i = threadIdx.x; i < n4; i += blockDim.x) {
-      const float4 u = et[i];
-      float4 q = pt[i];
-      if (pos2d) { const float4 w = pw[i]; q.x += w.x; q.y += w.y; q.z += w.z; q.w += w.w; }
-      xo[i] = make_float4((u.x + q.x) + ebq[0][i], (u.y + q.y) + ebq[1][i], (u.z + q.z) + ebq[2][i], (u.w + q.w) + ebq[3][i]);
-    }
-    return;
-  }
-  const float4* eb[4];
-#pragma unroll
-  for (int j = 0; j < 4; ++j) eb[j] = reinterpret_cast<const float4*>(a.E_bot + static_cast<size_t>(cbp[j]) * a.D);
-  const float4* pe = reinterpret_cast<const float4*>(a.P_emb);
-  for (int i = threadIdx.x; i < n4; i += blockDim.x) {
-    float4 u = et[i], q = pt[i], e0 = pe[i];
-    if (pos2d) { const float4 w = pw[i]; q.x += w.x; q.y += w.y; q.z += w.z; q.w += w.w; }
-    float4 acc;
-    acc.x = (u.x + q.x) + e0.x; acc.y = (u.y + q.y) + e0.y; acc.z = (u.z + q.z) + e0.z; acc.w = (u.w + q.w) + e0.w;
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      float4 e = eb[j][i], pj = pe[(j + 1) * n4 + i];
-      acc.x += e.x + pj.x; acc.y += e.y + pj.y; acc.z += e.z + pj.z; acc.w += e.w + pj.w;
-    }
-    acc.x /= 5.0f; acc.y /= 5.0f; acc.z /= 5.0f; acc.w /= 5.0f;
-    xo[i] = acc;
-  }
-}
-
-// The same for the 3-level HQTransformer (T0 = 1): row b * N + t is the sos row (t = 0) or the 21-token stack mean of
-// position t - 1, with embed3_kernel's operations and order.
-__global__ void __launch_bounds__(1024) embed3_prefix_kernel(int trace_id, Embed3Args a, int N) {
-  TraceScope trace_scope(trace_id);
-  pdl_launch_dependents();
-  pdl_wait();
-  const int row = blockIdx.x;
-  const int b = row / N, t = row % N;
-  float4* xo = reinterpret_cast<float4*>(a.x + static_cast<size_t>(row) * a.D);
-  const int n4 = a.D / 4;
-  if (t == 0) {
-    const float* src;
-    if (a.sos_override != nullptr) src = a.sos_override + static_cast<size_t>(b) * a.D;
-    else if (a.cond_kind == HQ_COND_CLS) src = a.sos_table + static_cast<size_t>(a.cond[b]) * a.D;
-    else src = a.sos_table;
-    const float4* s4 = reinterpret_cast<const float4*>(src);
-    for (int i = threadIdx.x; i < n4; i += blockDim.x) xo[i] = s4[i];
-    return;
-  }
-  const int p = t - 1;
-  __shared__ const float* rows[21];
-  if (threadIdx.x < 21) {
-    const size_t bp = static_cast<size_t>(b) * a.S + p;
-    const int j = threadIdx.x;
-    rows[j] = j == 0 ? a.E0 + static_cast<size_t>(a.codes_top[bp]) * a.D
-            : j < 5 ? a.E1 + static_cast<size_t>(a.codes_mid[bp * 4 + (j - 1)]) * a.D
-                    : a.E2 + static_cast<size_t>(a.codes_bot[bp * 16 + (j - 5)]) * a.D;
-  }
-  __syncthreads();
-  const float4* pt = reinterpret_cast<const float4*>(a.P_top + static_cast<size_t>(p) * a.D);
-  const float4* pe = reinterpret_cast<const float4*>(a.P_emb);
-  for (int i = threadIdx.x; i < n4; i += blockDim.x) {
-    const float4 u = reinterpret_cast<const float4*>(rows[0])[i], q = pt[i], e0 = pe[i];
-    float4 acc;
-    acc.x = (u.x + q.x) + e0.x; acc.y = (u.y + q.y) + e0.y; acc.z = (u.z + q.z) + e0.z; acc.w = (u.w + q.w) + e0.w;
-#pragma unroll 4
-    for (int j = 1; j < 21; ++j) {
-      const float4 e = reinterpret_cast<const float4*>(rows[j])[i], pj = pe[j * n4 + i];
-      acc.x += e.x + pj.x; acc.y += e.y + pj.y; acc.z += e.z + pj.z; acc.w += e.w + pj.w;
-    }
-    acc.x /= 21.0f; acc.y /= 21.0f; acc.z /= 21.0f; acc.w /= 21.0f;
-    xo[i] = acc;
-  }
 }
 
 // model_type 'top2bot' (hierarchical_ar.py:596-601): input of depth pass c >= 1:
