@@ -105,6 +105,12 @@ PROTOTYPES = {
     "hq_s1_last_conv_flops": (C.c_double, [C.c_void_p]),
     "hq_debug_s1_conv": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                    C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "hq_debug_s1_groupnorm": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                        C.c_int, C.c_void_p, C.c_void_p]),
+    "hq_debug_s1_resample": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "hq_debug_s1_quant": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
+                                    C.c_int, C.c_int, C.c_void_p]),
+    "hq_debug_s1_attention": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
 }
 
 _lib = None

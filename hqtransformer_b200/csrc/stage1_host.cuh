@@ -163,6 +163,8 @@ static int s1_make_attn(hq_s1_ctx* ctx, S1Attn* a, const std::string& p, int c) 
   return s1_make_conv(ctx, &a->proj, {p + ".proj_out"}, c, c, 1);
 }
 
+static constexpr int S1_ATT_SMEM_MAX = 96 * 1024;       // dynamic shared memory s1_attn_kernel may use: 8 (C + N) fp32
+
 // device, tensor-map encoder and kernel attributes of a ctx whose precision is set
 static int s1_open(hq_s1_ctx* ctx, int device) {
   int rc;
@@ -181,8 +183,8 @@ static int s1_open(hq_s1_ctx* ctx, int device) {
   S1_CUDA(ctx, cudaDeviceGetAttribute(&ctx->num_sms, cudaDevAttrMultiProcessorCount, device));
   S1_CUDA(ctx, cudaFuncSetAttribute(conv_tc2_kernel<bf16>, cudaFuncAttributeMaxDynamicSharedMemorySize, CH_SMEM_BYTES));
   S1_CUDA(ctx, cudaFuncSetAttribute(conv_tc2_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, CH_SMEM_BYTES));
-  S1_CUDA(ctx, cudaFuncSetAttribute(s1_attn_kernel<bf16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
-  S1_CUDA(ctx, cudaFuncSetAttribute(s1_attn_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
+  S1_CUDA(ctx, cudaFuncSetAttribute(s1_attn_kernel<bf16>, cudaFuncAttributeMaxDynamicSharedMemorySize, S1_ATT_SMEM_MAX));
+  S1_CUDA(ctx, cudaFuncSetAttribute(s1_attn_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, S1_ATT_SMEM_MAX));
   S1_CUDA(ctx, cudaFuncSetAttribute(s1_attn_mma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
   return HQ_OK;
 }
@@ -409,6 +411,14 @@ static void s1_resample(hq_s1_ctx* ctx, cudaStream_t st, const float* x, void* o
   s1_check(ctx);
 }
 
+// codes -> the padded input of post_quant_conv_b (PixelShuffle(2) of the top entries | bottom entries), border zero
+template <typename T>
+static void s1_quant(hq_s1_ctx* ctx, cudaStream_t st, const int64_t* code_t, const int64_t* code_b, const float* E_t,
+                     const float* E_b, void* out, int B, int E, int hb, int n_embed) {
+  s1_quant_kernel<T><<<B * (hb + 2) * (hb + 2), 256, 0, st>>>(code_t, code_b, E_t, E_b, static_cast<T*>(out), E, hb, n_embed);
+  s1_check(ctx);
+}
+
 // x (ctx->X) -> ResnetBlock (layers.py:118-135); result in ctx->X
 template <typename T>
 static void s1_resblock(hq_s1_ctx* ctx, cudaStream_t st, const S1Res& r, int B, int res) {
@@ -425,25 +435,36 @@ static void s1_resblock(hq_s1_ctx* ctx, cudaStream_t st, const S1Res& r, int B, 
   }
 }
 
-// AttnBlock (layers.py:163-186); result in ctx->X.  bf16: tensor-core core where the shape allows; float: the fp32 core.
+// whether the AttnBlock core over N tokens of C channels runs on the tensor cores (s1_attn_mma_kernel, bf16 only)
 template <typename T>
-static void s1_attnblock(hq_s1_ctx* ctx, cudaStream_t st, const S1Attn& a, int B, int res) {
-  const int C = a.n.C;
-  s1_gn<T>(ctx, st, a.n, ctx->X, ctx->H, B, res, 0);
-  s1_conv<T>(ctx, st, a.qkv, ctx->H, B, res, S1_OUT_ACT, nullptr, ctx->QKV, nullptr);
+static bool s1_attn_uses_mma(int N, int C) {
+  return std::is_same<T, bf16>::value && N % 16 == 0 && N <= S1A_NMAX && C % S1A_CB == 0 && C <= S1A_CMAX;
+}
+
+// AttnBlock core: qkv (padded [B, res+2, res+2, 3C]) -> out (padded [B, res+2, res+2, C], interior only).  bf16: the
+// tensor-core kernel where the shape allows (force_simt: the CUDA-core kernel regardless); float: the fp32 core.
+template <typename T>
+static void s1_attn_core(hq_s1_ctx* ctx, cudaStream_t st, const void* qkv, void* out, int B, int res, int C, bool force_simt) {
   const int N = res * res;
-  static const bool no_mma = getenv("HQ_DEBUG") != nullptr && getenv("HQ_S1_ATTN_SIMT") != nullptr;
-  if (std::is_same<T, bf16>::value && !no_mma && N % 16 == 0 && N <= S1A_NMAX && C % S1A_CB == 0 && C <= S1A_CMAX) {
+  if (!force_simt && s1_attn_uses_mma<T>(N, C)) {
     // tensor-core path: 64 queries per CTA
     const size_t smem = static_cast<size_t>(s1a_smem_bytes(C));
-    s1_attn_mma_kernel<<<dim3((N + S1A_Q - 1) / S1A_Q, B), 128, smem, st>>>(static_cast<const bf16*>(ctx->QKV),
-                                                                             static_cast<bf16*>(ctx->H2), res, res, C);
+    s1_attn_mma_kernel<<<dim3((N + S1A_Q - 1) / S1A_Q, B), 128, smem, st>>>(static_cast<const bf16*>(qkv),
+                                                                             static_cast<bf16*>(out), res, res, C);
   } else {
     const size_t smem = static_cast<size_t>(S1_ATT_Q) * (C + N) * 4;
-    s1_attn_kernel<T><<<dim3((N + S1_ATT_Q - 1) / S1_ATT_Q, B), 256, smem, st>>>(static_cast<const T*>(ctx->QKV),
-                                                                                 static_cast<T*>(ctx->H2), res, res, C);
+    s1_attn_kernel<T><<<dim3((N + S1_ATT_Q - 1) / S1_ATT_Q, B), 256, smem, st>>>(static_cast<const T*>(qkv),
+                                                                                 static_cast<T*>(out), res, res, C);
   }
   s1_check(ctx);
+}
+
+// AttnBlock (layers.py:163-186); result in ctx->X
+template <typename T>
+static void s1_attnblock(hq_s1_ctx* ctx, cudaStream_t st, const S1Attn& a, int B, int res) {
+  s1_gn<T>(ctx, st, a.n, ctx->X, ctx->H, B, res, 0);
+  s1_conv<T>(ctx, st, a.qkv, ctx->H, B, res, S1_OUT_ACT, nullptr, ctx->QKV, nullptr);
+  s1_attn_core<T>(ctx, st, ctx->QKV, ctx->H2, B, res, a.n.C, false);
   s1_conv<T>(ctx, st, a.proj, ctx->H2, B, res, S1_OUT_F32, ctx->X, nullptr, ctx->X);
 }
 
@@ -453,9 +474,7 @@ static void s1_decode(hq_s1_ctx* ctx, cudaStream_t st, const int64_t* code_t, co
   const hq_s1_config& cfg = ctx->cfg;
   const int lat = cfg.resolution >> cfg.n_levels;
   // codes -> [quant_t (pixel-shuffled) | quant_b] -> post_quant_conv_b -> conv_in
-  s1_quant_kernel<T><<<B * (lat + 2) * (lat + 2), 256, 0, st>>>(code_t, code_b, ctx->E_t, ctx->E_b, static_cast<T*>(ctx->H),
-                                                                 cfg.embed_dim, lat, cfg.n_embed);
-  s1_check(ctx);
+  s1_quant<T>(ctx, st, code_t, code_b, ctx->E_t, ctx->E_b, ctx->H, B, cfg.embed_dim, lat, cfg.n_embed);
   s1_conv<T>(ctx, st, ctx->post_quant, ctx->H, B, lat, S1_OUT_F32, ctx->X, nullptr, nullptr);
   s1_resample<T>(ctx, st, ctx->X, ctx->H, B, lat, cfg.z_channels, 1);
   s1_conv<T>(ctx, st, ctx->conv_in, ctx->H, B, lat, S1_OUT_F32, ctx->T, nullptr, nullptr);
@@ -500,37 +519,125 @@ extern "C" int hq_s1_decode_codes(hq_s1_ctx* ctx, const int64_t* code_t, const i
   return HQ_OK;
 }
 
-// One convolution through s1_make_conv / hq_s1_load_param / s1_conv on a throw-away ctx (include/hqgraft.h).
+// ---- test hooks (include/hqgraft.h): one decoder layer through the host function the decode calls, on a throw-away ctx ----
+static int s1_debug_open(hq_s1_ctx* ctx, int prec) {
+  ctx->prec = prec;
+  int device = 0;
+  S1_CUDA(ctx, cudaGetDevice(&device));
+  return s1_open(ctx, device);
+}
+
+// the launch error or stream fault of a hook's launches (if rc is still HQ_OK), then the ctx's buffers are freed
+static int s1_debug_finish(hq_s1_ctx* ctx, cudaStream_t st, int rc, const char* what) {
+  if (!rc) {
+    cudaError_t e = ctx->launch_err != cudaSuccess ? ctx->launch_err : cudaStreamSynchronize(st);
+    if (e != cudaSuccess) {
+      s1_err(ctx, "%s: %s", what, cudaGetErrorString(e));
+      rc = HQ_ERR_CUDA;
+    }
+  }
+  for (void* p : ctx->allocs) cudaFree(p);
+  if (rc) g_last_error = ctx->err;
+  return rc;
+}
+
 extern "C" int hq_debug_s1_conv(int prec, const void* A, const float* weight, const float* bias, int B, int res, int Cin,
                                 int Cout, int k, int mode, int tile, const float* resid, void* out, void* stream) {
+  // modes 0 / 1 store 4-wide vectors at row * Cout + col: Cout % 4 keeps every row's vectors aligned
   if (!A || !weight || !bias || !out || B < 1 || res < 1 || Cout < 1 || (k != 1 && k != 3) || mode < S1_OUT_F32 ||
-      mode > S1_OUT_IMAGE || (resid && mode != S1_OUT_F32) || (tile != 0 && (tile % 32 != 0 || tile < 32 || tile > 256))) {
+      mode > S1_OUT_IMAGE || (mode != S1_OUT_IMAGE && Cout % 4 != 0) || (resid && mode != S1_OUT_F32) ||
+      (tile != 0 && (tile % 32 != 0 || tile < 32 || tile > 256))) {
     s1_err(nullptr, "hq_debug_s1_conv: bad argument");
     return HQ_ERR_INVALID;
   }
   hq_s1_ctx ctx;
-  ctx.prec = prec;
-  int device = 0;
-  S1_CUDA(&ctx, cudaGetDevice(&device));
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
   S1Conv c;
-  int rc = s1_open(&ctx, device);
+  int rc = s1_debug_open(&ctx, prec);
   if (!rc) rc = s1_make_conv(&ctx, &c, {"conv"}, Cin, Cout, k, tile);
   const int64_t wshape[4] = {Cout, Cin, k, k}, bshape[1] = {Cout};
   if (!rc) rc = hq_s1_load_param(&ctx, "conv.weight", weight, HQ_F32, wshape, 4, 1);
   if (!rc) rc = hq_s1_load_param(&ctx, "conv.bias", bias, HQ_F32, bshape, 1, 1);
   if (!rc) {
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
     float* outf = mode == S1_OUT_ACT ? nullptr : static_cast<float*>(out);
     void* outb = mode == S1_OUT_ACT ? out : nullptr;
     if (prec == HQ_PREC_TF32) s1_conv<float>(&ctx, st, c, A, B, res, mode, outf, outb, resid);
     else s1_conv<bf16>(&ctx, st, c, A, B, res, mode, outf, outb, resid);
-    cudaError_t e = ctx.launch_err != cudaSuccess ? ctx.launch_err : cudaStreamSynchronize(st);
-    if (e != cudaSuccess) {
-      s1_err(&ctx, "hq_debug_s1_conv: %s", cudaGetErrorString(e));
-      rc = HQ_ERR_CUDA;
-    }
   }
-  for (void* p : ctx.allocs) cudaFree(p);
-  if (rc) g_last_error = ctx.err;
-  return rc;
+  return s1_debug_finish(&ctx, st, rc, "hq_debug_s1_conv");
+}
+
+extern "C" int hq_debug_s1_groupnorm(int prec, const float* x, const float* gamma, const float* beta, void* out, int B, int res,
+                                     int C, int swish, float* stat_out, void* stream) {
+  if (!x || !gamma || !beta || !out || B < 1 || res < 1 || C < 32 || C % 32 != 0 || C > 1024 || (swish != 0 && swish != 1)) {
+    s1_err(nullptr, "hq_debug_s1_groupnorm: bad argument");
+    return HQ_ERR_INVALID;
+  }
+  hq_s1_ctx ctx;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  int rc = s1_debug_open(&ctx, prec);
+  if (!rc) rc = s1_alloc(&ctx, reinterpret_cast<void**>(&ctx.gn_part), static_cast<size_t>(B) * 32 * 64 * 2 * 8);
+  if (!rc) rc = s1_alloc(&ctx, reinterpret_cast<void**>(&ctx.gn_stat), static_cast<size_t>(B) * 32 * 8);
+  if (!rc) rc = s1_alloc(&ctx, reinterpret_cast<void**>(&ctx.gn_cnt), static_cast<size_t>(B) * 4);
+  if (!rc) {
+    S1Norm n;
+    n.C = C;
+    n.g = const_cast<float*>(gamma);
+    n.b = const_cast<float*>(beta);
+    if (prec == HQ_PREC_TF32) s1_gn<float>(&ctx, st, n, x, out, B, res, swish);
+    else s1_gn<bf16>(&ctx, st, n, x, out, B, res, swish);
+    cudaError_t e = stat_out ? cudaMemcpyAsync(stat_out, ctx.gn_stat, static_cast<size_t>(B) * 32 * 8, cudaMemcpyDeviceToDevice, st)
+                             : cudaSuccess;
+    if (e != cudaSuccess && ctx.launch_err == cudaSuccess) ctx.launch_err = e;
+  }
+  return s1_debug_finish(&ctx, st, rc, "hq_debug_s1_groupnorm");
+}
+
+extern "C" int hq_debug_s1_resample(int prec, const float* x, void* out, int B, int res, int C, int up, void* stream) {
+  if (!x || !out || B < 1 || res < 1 || C < 4 || C % 4 != 0 || (up != 1 && up != 2)) {
+    s1_err(nullptr, "hq_debug_s1_resample: bad argument");
+    return HQ_ERR_INVALID;
+  }
+  hq_s1_ctx ctx;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  int rc = s1_debug_open(&ctx, prec);
+  if (!rc) {
+    if (prec == HQ_PREC_TF32) s1_resample<float>(&ctx, st, x, out, B, res, C, up);
+    else s1_resample<bf16>(&ctx, st, x, out, B, res, C, up);
+  }
+  return s1_debug_finish(&ctx, st, rc, "hq_debug_s1_resample");
+}
+
+extern "C" int hq_debug_s1_quant(int prec, const int64_t* code_t, const int64_t* code_b, const float* E_t, const float* E_b,
+                                 void* out, int B, int E, int hb, int n_embed, void* stream) {
+  if (!code_t || !code_b || !E_t || !E_b || !out || B < 1 || E < 1 || hb < 2 || hb % 2 != 0 || n_embed < 1) {
+    s1_err(nullptr, "hq_debug_s1_quant: bad argument");
+    return HQ_ERR_INVALID;
+  }
+  hq_s1_ctx ctx;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  int rc = s1_debug_open(&ctx, prec);
+  if (!rc) {
+    if (prec == HQ_PREC_TF32) s1_quant<float>(&ctx, st, code_t, code_b, E_t, E_b, out, B, E, hb, n_embed);
+    else s1_quant<bf16>(&ctx, st, code_t, code_b, E_t, E_b, out, B, E, hb, n_embed);
+  }
+  return s1_debug_finish(&ctx, st, rc, "hq_debug_s1_quant");
+}
+
+extern "C" int hq_debug_s1_attention(int prec, const void* qkv, void* out, int B, int res, int C, int variant, void* stream) {
+  const int N = res * res;
+  const bool simt = variant == 1 || !(prec == HQ_PREC_BF16 ? s1_attn_uses_mma<bf16>(N, C) : s1_attn_uses_mma<float>(N, C));
+  if (!qkv || !out || B < 1 || res < 1 || C < 8 || C % 8 != 0 || (variant != 0 && variant != 1) ||
+      (simt && static_cast<size_t>(S1_ATT_Q) * (C + N) * 4 > static_cast<size_t>(S1_ATT_SMEM_MAX))) {
+    s1_err(nullptr, "hq_debug_s1_attention: bad argument");
+    return HQ_ERR_INVALID;
+  }
+  hq_s1_ctx ctx;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  int rc = s1_debug_open(&ctx, prec);
+  if (!rc) {
+    if (prec == HQ_PREC_TF32) s1_attn_core<float>(&ctx, st, qkv, out, B, res, C, variant == 1);
+    else s1_attn_core<bf16>(&ctx, st, qkv, out, B, res, C, variant == 1);
+  }
+  return s1_debug_finish(&ctx, st, rc, "hq_debug_s1_attention");
 }

@@ -227,3 +227,62 @@ def debug_s1_conv(A: torch.Tensor, weight: torch.Tensor, bias: torch.Tensor, out
         rc = lib.hq_debug_s1_conv(prec, A.data_ptr(), weight.data_ptr(), bias.data_ptr(), B, Hp - 2, Cin, Cout, k, mode,
                                   tile, resid.data_ptr() if resid is not None else None, out.data_ptr(), C.c_void_p(st))
         check_s1(rc, None, lib, "hq_debug_s1_conv")
+
+
+def _s1_prec(t: torch.Tensor) -> int:
+    """Operand type of a stage-1 test hook from its T tensor: bf16 -> HQ_PREC_BF16, fp32 -> HQ_PREC_TF32."""
+    return {torch.bfloat16: _lib.HQ_PREC_BF16, torch.float32: _lib.HQ_PREC_TF32}[t.dtype]
+
+
+def _s1_call(lib, name: str, tensors, *args) -> None:
+    dev = tensors[0].device
+    for t in tensors:
+        assert t.is_cuda and t.is_contiguous() and t.device == dev
+    with torch.cuda.device(dev):
+        st = torch.cuda.current_stream(dev).cuda_stream
+        check_s1(getattr(lib, name)(*args, C.c_void_p(st)), None, lib, name)
+
+
+def debug_s1_groupnorm(x: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, out: torch.Tensor, *, swish: bool,
+                       stat_out: Optional[torch.Tensor] = None) -> None:
+    """GroupNorm(32, eps 1e-6) (+ swish) through hq_debug_s1_groupnorm (the decoder's statistics and apply kernels), in
+    place, synchronous.  x: padded fp32 [B, res+2, res+2, C]; out: padded, bf16 (precision bf16) or fp32 (tf32);
+    stat_out: fp32 [B, 32, 2], the (mean, rstd) the statistics kernel published."""
+    lib = _lib.load()
+    B, Hp, _, Cn = x.shape
+    assert x.dtype == gamma.dtype == beta.dtype == torch.float32
+    ts = (x, gamma, beta, out) + ((stat_out,) if stat_out is not None else ())
+    _s1_call(lib, "hq_debug_s1_groupnorm", ts, _s1_prec(out), x.data_ptr(), gamma.data_ptr(), beta.data_ptr(),
+             out.data_ptr(), B, Hp - 2, Cn, int(swish), stat_out.data_ptr() if stat_out is not None else None)
+
+
+def debug_s1_resample(x: torch.Tensor, out: torch.Tensor, up: int) -> None:
+    """Nearest `up`x upsampling (up = 1: the operand copy) through hq_debug_s1_resample, in place, synchronous.
+    x: padded fp32 [B, res+2, res+2, C]; out: padded bf16 / fp32 [B, up res+2, up res+2, C]."""
+    lib = _lib.load()
+    B, Hp, _, Cn = x.shape
+    assert x.dtype == torch.float32
+    _s1_call(lib, "hq_debug_s1_resample", (x, out), _s1_prec(out), x.data_ptr(), out.data_ptr(), B, Hp - 2, Cn, up)
+
+
+def debug_s1_quant(code_t: torch.Tensor, code_b: torch.Tensor, E_t: torch.Tensor, E_b: torch.Tensor,
+                   out: torch.Tensor) -> None:
+    """Codebook gather + PixelShuffle + concat through hq_debug_s1_quant, in place, synchronous.  code_t int64
+    [B, hb/2, hb/2], code_b int64 [B, hb, hb], E_t fp32 [n_embed, 4E], E_b fp32 [n_embed, E]; out: padded bf16 / fp32
+    [B, hb+2, hb+2, 2E]."""
+    lib = _lib.load()
+    B, hb, _ = code_b.shape
+    n_embed, E = E_b.shape
+    assert code_t.dtype == code_b.dtype == torch.int64 and E_t.dtype == E_b.dtype == torch.float32
+    _s1_call(lib, "hq_debug_s1_quant", (code_t, code_b, E_t, E_b, out), _s1_prec(out), code_t.data_ptr(),
+             code_b.data_ptr(), E_t.data_ptr(), E_b.data_ptr(), out.data_ptr(), B, E, hb, n_embed)
+
+
+def debug_s1_attention(qkv: torch.Tensor, out: torch.Tensor, variant: int = 0) -> None:
+    """AttnBlock core through hq_debug_s1_attention, in place, synchronous.  qkv: padded [B, res+2, res+2, 3C] (q | k | v),
+    out: padded [B, res+2, res+2, C], both bf16 or both fp32.  variant 0: the decoder's choice, 1: the CUDA-core kernel."""
+    lib = _lib.load()
+    B, Hp, _, C3 = qkv.shape
+    assert qkv.dtype == out.dtype
+    _s1_call(lib, "hq_debug_s1_attention", (qkv, out), _s1_prec(out), qkv.data_ptr(), out.data_ptr(), B, Hp - 2, C3 // 3,
+             variant)

@@ -381,9 +381,36 @@ double hq_s1_last_conv_flops(const hq_s1_ctx* ctx);
  * weight fp32 [Cout, Cin, k, k] (k = 1 or 3; packed and rounded as hq_s1_load_param does); bias fp32 [Cout]; Cin a
  * multiple of 64.  mode 0: out fp32 [B, res+2, res+2, Cout], interior written, += resid (fp32, same layout, may equal
  * out) when resid != NULL; 1: out in the operand type (fp32 unrounded under HQ_PREC_TF32), interior written; 2: out fp32
- * image [B, Cout, res, res].  tile: 0 = the planner's width, else a multiple of 32 in [32, 256]. */
+ * image [B, Cout, res, res].  Cout a multiple of 4 in modes 0 and 1.  tile: 0 = the planner's width, else a multiple of
+ * 32 in [32, 256]. */
 int hq_debug_s1_conv(int prec, const void* A, const float* weight, const float* bias, int B, int res, int Cin, int Cout,
                      int k, int mode, int tile, const float* resid, void* out, void* stream);
+
+/* The remaining stage-1 test hooks run one decoder layer through the host function the decode calls, synchronously on
+ * `stream`; device pointers; prec HQ_PREC_BF16 or HQ_PREC_TF32 selects the operand type T (bf16 | fp32 rounded to TF32).
+ * "Padded" tensors are NHWC [B, res+2, res+2, C]; HQ_ERR_INVALID without a launch for arguments the kernels do not take.
+ *
+ * GroupNorm(32 groups, eps 1e-6) (+ swish when swish == 1) of the interior of x (padded fp32, C a multiple of 32, at most
+ * 1024) -> out (padded T, every position written, the border with zeros).  stat_out (optional): fp32 [B, 32, 2], the
+ * (mean, rstd) per image and group the statistics kernel published. */
+int hq_debug_s1_groupnorm(int prec, const float* x, const float* gamma, const float* beta, void* out, int B, int res, int C,
+                          int swish, float* stat_out, void* stream);
+
+/* Nearest-neighbour upsampling by `up` (1 or 2) of the interior of x (padded fp32 [B, res+2, res+2, C], C % 4 == 0) ->
+ * out (padded T [B, up res+2, up res+2, C], every position written, the border with zeros); up = 1 is the operand copy. */
+int hq_debug_s1_resample(int prec, const float* x, void* out, int B, int res, int C, int up, void* stream);
+
+/* Codes -> the padded input of post_quant_conv_b: code_t int64 [B, hb/2, hb/2], code_b int64 [B, hb, hb] (hb even),
+ * E_t fp32 [n_embed, 4E], E_b fp32 [n_embed, E]; out T [B, hb+2, hb+2, 2E] = PixelShuffle(2) of the top entries | the
+ * bottom entries, border zero. */
+int hq_debug_s1_quant(int prec, const int64_t* code_t, const int64_t* code_b, const float* E_t, const float* E_b, void* out,
+                      int B, int E, int hb, int n_embed, void* stream);
+
+/* AttnBlock core softmax(q k^T C^-1/2) v over the res x res pixels of each image: qkv padded T [.., 3C] (q | k | v),
+ * out padded T [.., C], interior written.  variant 0: the decoder's choice (bf16: the tensor-core kernel when N = res^2
+ * is a multiple of 16 and <= 256 and C a multiple of 128 and <= 512); 1: the CUDA-core kernel.  C % 8 == 0; the
+ * CUDA-core kernel needs 32 (C + N) bytes <= 96 KB of shared memory. */
+int hq_debug_s1_attention(int prec, const void* qkv, void* out, int B, int res, int C, int variant, void* stream);
 
 #ifdef __cplusplus
 }

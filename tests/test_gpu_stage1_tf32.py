@@ -1,6 +1,6 @@
-"""-m gpu: the tf32 stage-1 decoder (precision="tf32", HQ_PREC_TF32): single convolutions through hq_debug_s1_conv against
-fp64, whole decodes against the fp32 oracle, its TF32 emulation (tests/tf32_emulation.py) and the oracle run with PyTorch's
-own cuDNN TF32 convolutions on the GPU."""
+"""-m gpu: the tf32 stage-1 decoder (precision="tf32", HQ_PREC_TF32): whole decodes against the fp32 oracle, its TF32
+emulation (tests/tf32_emulation.py) and the oracle run with PyTorch's own cuDNN TF32 convolutions on the GPU.  Its kernels
+one by one: tests/test_gpu_stage1_kernels.py."""
 import os
 
 import pytest
@@ -11,8 +11,6 @@ from tests import tf32_emulation as T
 from tests.helpers import load_golden
 
 pytestmark = pytest.mark.gpu
-
-TILES = (0, 32, 64, 128, 256)
 
 
 def _decoder(cfg, P, max_batch, precision="tf32"):
@@ -40,82 +38,6 @@ def _report(name, got, ref):
     eq8 = float((_pix8(got) == _pix8(ref)).float().mean())
     print(f"\n[tf32 stage 1] {name}: max-abs {float(e.max()):.3e} mean-abs {float(e.mean()):.3e} 8-bit equal {eq8:.4f}")
     return float(e.max()), float(e.mean()), eq8
-
-
-# ---- 1. single convolutions ---------------------------------------------------------------------------------------------
-# (B, res, Cin, Cout, k, mode, in-place residual): the planner picks tile width 32 (Cout 3, the image conv), 64, 96, 128 and
-# 256 (Cout 512 and the fused q | k | v of 1536); Cin 64 ... 512; every output mode
-CASES = [
-    (2, 16, 128, 3, 3, 2, False),
-    (2, 8, 64, 64, 3, 0, False),
-    (1, 8, 256, 96, 3, 0, True),
-    (1, 32, 128, 128, 1, 0, False),
-    (1, 8, 192, 64, 1, 1, False),
-    (2, 16, 512, 512, 3, 0, True),
-    (2, 16, 512, 1536, 1, 1, False),
-]
-
-
-@pytest.mark.parametrize("B,res,Cin,Cout,k,mode,inplace", CASES)
-def test_tf32_conv_against_fp64_at_every_tile(B, res, Cin, Cout, k, mode, inplace):
-    from hqtransformer_b200.stage1 import debug_s1_conv
-    dev = torch.device("cuda", 0)
-    g = torch.Generator(device=dev).manual_seed(Cin * 7 + Cout + k)
-    Hp = res + 2
-    A = torch.zeros(B, Hp, Hp, Cin, device=dev)
-    A[:, 1:-1, 1:-1, :] = T.round_tf32(torch.randn(B, res, res, Cin, generator=g, device=dev))
-    W = torch.randn(Cout, Cin, k, k, generator=g, device=dev) / (Cin * k * k) ** 0.5
-    bias = 0.1 * torch.randn(Cout, generator=g, device=dev)
-    y, scale = T.conv_fp64(A, W, bias, k)
-    resid = torch.randn(B, res, res, Cout, generator=g, device=dev) if inplace else None
-    if resid is not None:
-        y = y + resid.permute(0, 3, 1, 2).double()
-    extra = 4096                                                     # oversized: nothing past the tensor may be written
-    results = []
-    for tile in TILES:
-        if mode == 2:
-            n = B * Cout * res * res
-            buf = torch.full((n + extra,), float("nan"), device=dev)
-            out = buf[:n].view(B, Cout, res, res)
-        else:
-            n = B * Hp * Hp * Cout
-            buf = torch.full((n + extra,), float("nan"), device=dev)
-            out = buf[:n].view(B, Hp, Hp, Cout)
-            if resid is not None:
-                out[:, 1:-1, 1:-1, :] = resid
-        debug_s1_conv(A, W, bias, out, mode, resid=out if inplace else None, tile=tile)
-        assert torch.isnan(buf[n:]).all(), f"tile {tile}: wrote past the output"
-        if mode == 2:
-            got = out
-        else:
-            border = torch.ones(B, Hp, Hp, dtype=torch.bool, device=dev)
-            border[:, 1:-1, 1:-1] = False
-            assert torch.isnan(out[border]).all(), f"tile {tile}: wrote a padding position"
-            got = out[:, 1:-1, 1:-1, :].permute(0, 3, 1, 2)
-        assert torch.isfinite(got).all(), f"tile {tile}: interior not fully written"
-        err = (got.double() - y).abs()
-        # fp32 accumulation of exact TF32 x TF32 products: a few ulp of the sum of |terms|, plus the fp32 store
-        bound = 1e-5 * (scale + (resid.permute(0, 3, 1, 2).abs().double() if resid is not None else 0)) + 1e-6 * y.abs() + 1e-7
-        assert bool((err <= bound).all()), (tile, float((err / bound).max()))
-        if mode == 1:                                                # q | k | v stay UNROUNDED fp32
-            assert float(((got.contiguous().view(torch.int32) & 0x1FFF) != 0).float().mean()) > 0.9
-        results.append(got.clone())
-    for tile, r in zip(TILES[1:], results[1:]):
-        assert torch.equal(r, results[0]), f"tile {tile} differs from the planner's"
-
-
-def test_debug_conv_rejects_bad_plans():
-    import hqtransformer_b200 as H
-    from hqtransformer_b200.stage1 import debug_s1_conv
-    dev = torch.device("cuda", 0)
-    A = torch.zeros(1, 6, 6, 64, device=dev)
-    W, b = torch.zeros(64, 64, 3, 3, device=dev), torch.zeros(64, device=dev)
-    out = torch.zeros(1, 6, 6, 64, device=dev)
-    for tile in (16, 48, 288):
-        with pytest.raises(H.HQError):
-            debug_s1_conv(A, W, b, out, 0, tile=tile)
-    with pytest.raises(H.HQError):                                   # Cin must be a multiple of 64
-        debug_s1_conv(torch.zeros(1, 6, 6, 32, device=dev), torch.zeros(64, 32, 3, 3, device=dev), b, out, 0)
 
 
 # ---- 2. / 3. whole decodes ----------------------------------------------------------------------------------------------

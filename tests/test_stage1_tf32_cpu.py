@@ -114,7 +114,9 @@ def test_header_and_binding_agree_on_abi_9_and_the_stage1_config():
     assert [f for f, _ in fields] == [f for f, _ in _lib.HQS1Config._fields_]
     assert fields[-1][0] == "precision"
     assert ctypes.sizeof(_lib.HQS1Config) == 4 * sum(int(n or 1) for _, n in fields) == 18 * 4
-    assert "hq_debug_s1_conv" in _lib.PROTOTYPES and "hq_debug_s1_conv" in header
+    for hook in ("hq_debug_s1_conv", "hq_debug_s1_groupnorm", "hq_debug_s1_resample", "hq_debug_s1_quant",
+                 "hq_debug_s1_attention"):
+        assert hook in _lib.PROTOTYPES and re.search(r"\bint " + hook + r"\(", header), hook
 
 
 def test_tf32_emulation_with_fp64_accumulation_restores_the_oracle():

@@ -63,11 +63,12 @@ def decode_code(P, cfg, code_t, code_b, accumulate=torch.float32):
     return out.float()
 
 
-def conv_fp64(A_nhwc: torch.Tensor, weight: torch.Tensor, bias: torch.Tensor, k: int):
-    """fp64 convolution of a padded NHWC operand [B, res+2, res+2, Cin] (as stored) with TF32-rounded fp32 weights, and
-    the same of |A| * |W| (the scale of the fp32 accumulation error): both [B, Cout, res, res]."""
+def conv_fp64(A_nhwc: torch.Tensor, weight: torch.Tensor, bias: torch.Tensor, k: int, round_weight=round_tf32):
+    """fp64 convolution of a padded NHWC operand [B, res+2, res+2, Cin] (as stored) with fp32 weights rounded as the
+    decoder packs them (round_weight: TF32 by default), and the same of |A| * |W| (the scale of the fp32 accumulation
+    error): both [B, Cout, res, res]."""
     a = A_nhwc[:, 1:-1, 1:-1, :].permute(0, 3, 1, 2).double()
-    w = round_tf32(weight).double()
+    w = round_weight(weight).double()
     y = F.conv2d(a, w, bias.double(), padding=k // 2)
     s = F.conv2d(a.abs(), w.abs(), None, padding=k // 2)
     return y, s
