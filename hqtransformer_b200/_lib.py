@@ -102,6 +102,8 @@ PROTOTYPES = {
     "hq_s1_load_param": (C.c_int, [C.c_void_p, C.c_char_p, C.c_void_p, C.c_int, C.POINTER(C.c_int64), C.c_int, C.c_int]),
     "hq_s1_params_complete": (C.c_int, [C.c_void_p]),
     "hq_s1_decode_codes": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
+    "hq_s1_reserve_grid": (C.c_int, [C.c_void_p, C.c_int]),
+    "hq_s1_decode_codes_grid": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p]),
     "hq_s1_last_conv_flops": (C.c_double, [C.c_void_p]),
     "hq_debug_s1_conv": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                    C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),

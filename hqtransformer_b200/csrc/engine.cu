@@ -482,6 +482,11 @@ static int set_attn_attrs(hq_ctx* ctx) {
   if ((rc = set_smem(ctx, attention_decode_kernel<bf16>, 64 * 1024))) return rc;
   if ((rc = set_smem(ctx, attention_decode_kernel<f16>, 64 * 1024))) return rc;
   if ((rc = set_smem(ctx, attention_decode_kernel<float>, 64 * 1024))) return rc;
+  if ((rc = set_smem(ctx, attention_decode_kernel<bf16, ATT_MAX_KEYS_LONG>, 64 * 1024))) return rc;
+  if ((rc = set_smem(ctx, attention_decode_kernel<f16, ATT_MAX_KEYS_LONG>, 64 * 1024))) return rc;
+  if ((rc = set_smem(ctx, attention_decode_kernel<float, ATT_MAX_KEYS_LONG>, 64 * 1024))) return rc;
+  if ((rc = set_smem(ctx, attention_prefix_long_kernel<bf16>, attp_long_smem_bytes(ATT_MAX_KEYS_LONG, 2)))) return rc;
+  if ((rc = set_smem(ctx, attention_prefix_long_kernel<f16>, attp_long_smem_bytes(ATT_MAX_KEYS_LONG, 2)))) return rc;
   if ((rc = set_smem(ctx, attention_decode_mma_kernel<bf16>, 112 * 1024))) return rc;
   return set_smem(ctx, attention_decode_mma_kernel<f16>, 112 * 1024);
 }
@@ -689,9 +694,9 @@ static int create_impl(hq_ctx* ctx, const hq_config* cfg, int device, int max_ba
     set_err(ctx, "unsupported vocabulary sizes %d / %d (multiples of 64, <= 32768)", ctx->Vt, ctx->Vb);
     return HQ_ERR_UNSUPPORTED;
   }
-  if (ctx->Tc > ATT_MAX_KEYS || ctx->Smax < 1 || ctx->Smax > cfg->ctx_len_img) {
+  if (ctx->Tc > ATT_MAX_KEYS_LONG || ctx->Smax < 1 || ctx->Smax > cfg->ctx_len_img) {
     set_err(ctx, "unsupported lengths: max_seq_len=%d ctx_len_img=%d ctx_len_txt=%d (cache length %d > %d)", ctx->Smax,
-            cfg->ctx_len_img, cfg->ctx_len_txt, ctx->Tc, ATT_MAX_KEYS);
+            cfg->ctx_len_img, cfg->ctx_len_txt, ctx->Tc, ATT_MAX_KEYS_LONG);
     return HQ_ERR_UNSUPPORTED;
   }
   if (cfg->cond_kind < 0 || cfg->cond_kind > 2 || cfg->precision < HQ_PREC_BF16 || cfg->precision > HQ_PREC_F16) {
@@ -1273,9 +1278,9 @@ static bool attn_prefetch_ok(const hq_ctx* ctx) { return !ctx->dbg.attn_no_prefe
 
 static int attn_sleep_ns(const hq_ctx* ctx) { return ctx->dbg.attn_sleep; }
 
-// Launch plan of attention_decode_kernel for this model: head groups per image, keys per ring stage, dynamic smem.
+// Launch plan of attention_decode_kernel<AT, maxk> for this model: head groups per image, keys per ring stage, dynamic smem.
 template <typename AT>
-static bool attn_decode_plan(const hq_ctx* ctx, int* CH, int* hpc, int* groups, size_t* smem) {
+static bool attn_decode_plan(const hq_ctx* ctx, int maxk, int* CH, int* hpc, int* groups, size_t* smem) {
   const int g = attn_groups(ctx, ctx->nh);
   if (g <= 0) return false;
   *groups = g;
@@ -1285,7 +1290,7 @@ static bool attn_decode_plan(const hq_ctx* ctx, int* CH, int* hpc, int* groups, 
   if (ch < 4) ch = 4;
   if (ch > 16) ch = 16;
   *CH = ch;
-  *smem = static_cast<size_t>(ATTD_STAGES) * ch * row_bytes + static_cast<size_t>(*hpc) * ATT_MAX_KEYS * 4 +
+  *smem = static_cast<size_t>(ATTD_STAGES) * ch * row_bytes + static_cast<size_t>(*hpc) * maxk * 4 +
           2 * ATTD_STAGES * 8 + 128;
   return *smem <= 64 * 1024;
 }
@@ -1357,8 +1362,18 @@ static void attention(hq_ctx* ctx, cudaStream_t st, const AT* q, const AT* K, co
                ctx->nh, ctx->D, Tq, t_stride);
       return;
     }
+    if (ctx->prefix_pass && causal && kbase == 0) {
+      // longer prefixes: one CTA per (image, head, block of 128 queries)
+      launch_k(ctx, st, "attention_prefix", attention_prefix_long_kernel<AT>,
+               dim3((M / Tq) * ctx->nh, (Tq + ATTP_QBLOCK - 1) / ATTP_QBLOCK), dim3(256),
+               static_cast<size_t>(attp_long_smem_bytes((Tq + 15) & ~15, 2)), q, K, V, out, ctx->nh, ctx->D, Tq, t_stride);
+      return;
+    }
   }
-  if (Tq == 1 && !causal && !ctx->dbg.attn_generic && attn_decode_plan<AT>(ctx, &CH, &hpc, &groups, &smem)) {
+  const bool long_keys = (causal ? kbase + Tq : kbase) > ATT_MAX_KEYS;   // the score rows of the 320-key instances
+  // the plan is taken at 128 keys whatever the length: the mma kernel holds no score rows, so its choice must not depend on
+  // the scalar kernel's; past 128 keys the scalar kernel's own plan is checked below
+  if (Tq == 1 && !causal && !ctx->dbg.attn_generic && attn_decode_plan<AT>(ctx, ATT_MAX_KEYS, &CH, &hpc, &groups, &smem)) {
     // spatial decode: (image, head group) work items, K/V streamed through shared memory by bulk async copies
     if (ctx->tracing) ctx->tag_suffix = ":t" + std::to_string(kbase) + ":B" + std::to_string(M);
     int stages = 0, grid = 0;
@@ -1372,9 +1387,13 @@ static void attention(hq_ctx* ctx, cudaStream_t st, const AT* q, const AT* K, co
       launch_attn_mma<AT>(ctx, st, q, K, out, t_stride, kbase, hpc, groups, M * groups, stages, grid, smem2);
       return;
     }
-    launch_k(ctx, st, "attention_decode", attention_decode_kernel<AT>, dim3(M * groups), dim3((hpc + 1) * 32), smem, q, K, V,
-             out, ctx->D, t_stride, kbase, CH, hpc, groups, attn_prefetch_ok(ctx) ? attn_sleep_ns(ctx) : -1);
-    return;
+    if (!long_keys || attn_decode_plan<AT>(ctx, ATT_MAX_KEYS_LONG, &CH, &hpc, &groups, &smem)) {
+      launch_k(ctx, st, "attention_decode", long_keys ? attention_decode_kernel<AT, ATT_MAX_KEYS_LONG> : attention_decode_kernel<AT>,
+               dim3(M * groups), dim3((hpc + 1) * 32), smem, q, K, V, out, ctx->D, t_stride, kbase, CH, hpc, groups,
+               attn_prefetch_ok(ctx) ? attn_sleep_ns(ctx) : -1);
+      return;
+    }
+    ctx->tag_suffix.clear();     // 320-key score rows do not fit beside the ring: the per-(query, head) kernel below
   }
   const int items = M * ctx->nh;
   if (!causal && kbase <= ATT_DEPTH_KEYS && Tq == 4 && !ctx->dbg.attn_fewkeys_old) {
@@ -1389,8 +1408,9 @@ static void attention(hq_ctx* ctx, cudaStream_t st, const AT* q, const AT* K, co
              dim3(ATT_WARPS * 32), 0, q, K, V, out, M, ctx->nh, ctx->D, Tq, t_stride, kbase);
     return;
   }
-  launch_k(ctx, st, "attention_generic", attention_kernel<AT>, dim3((items + ATT_WARPS - 1) / ATT_WARPS),
-           dim3(ATT_WARPS * 32), 0, q, K, V, out, M, ctx->nh, ctx->D, Tq, t_stride, kbase, causal);
+  launch_k(ctx, st, "attention_generic", long_keys ? attention_kernel<AT, ATT_MAX_KEYS_LONG> : attention_kernel<AT>,
+           dim3((items + ATT_WARPS - 1) / ATT_WARPS), dim3(ATT_WARPS * 32), 0, q, K, V, out, M, ctx->nh, ctx->D, Tq, t_stride,
+           kbase, causal);
 }
 
 static void launch_sample(hq_ctx* ctx, cudaStream_t st, const SampleArgs& a) {
@@ -1855,9 +1875,9 @@ static int validate_run(hq_ctx* ctx, const hq_run_args* a) {
       set_err(ctx, "prefix_len %d must be below pos_end %d (at least one position is sampled)", a->prefix_len, a->pos_end);
       return HQ_ERR_INVALID;
     }
-    if (ctx->T0 + a->prefix_len - 1 > ATT_MAX_KEYS) {
+    if (ctx->T0 + a->prefix_len - 1 > ATT_MAX_KEYS_LONG) {
       set_err(ctx, "prefix_len %d: %d prefix tokens exceed the %d keys of the attention kernels", a->prefix_len,
-              ctx->T0 + a->prefix_len - 1, ATT_MAX_KEYS);
+              ctx->T0 + a->prefix_len - 1, ATT_MAX_KEYS_LONG);
       return HQ_ERR_INVALID;
     }
   }
@@ -2091,7 +2111,7 @@ extern "C" int hq_run_host(hq_ctx* ctx, const hq_run_args* args) {
 extern "C" int hq_debug_attention(int prec, const void* q, const void* K, const void* V, void* out, int B, int n_heads,
                                   int t_stride, int n_keys, int variant, void* stream) {
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (B < 1 || n_heads < 1 || n_keys < 1 || n_keys > t_stride || n_keys > ATT_MAX_KEYS || !q || !K || !V || !out) {
+  if (B < 1 || n_heads < 1 || n_keys < 1 || n_keys > t_stride || n_keys > ATT_MAX_KEYS_LONG || !q || !K || !V || !out) {
     set_err(nullptr, "hq_debug_attention: bad argument");
     return HQ_ERR_INVALID;
   }
@@ -2141,7 +2161,7 @@ extern "C" int hq_debug_attention(int prec, const void* q, const void* K, const 
 extern "C" int hq_debug_attention_prefix(int prec, const void* q, const void* K, const void* V, void* out, int B, int n_heads,
                                          int t_stride, int n_q, int variant, void* stream) {
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (B < 1 || n_heads < 1 || n_q < 1 || n_q > t_stride || n_q > ATT_MAX_KEYS || !q || !K || !V || !out) {
+  if (B < 1 || n_heads < 1 || n_q < 1 || n_q > t_stride || n_q > ATT_MAX_KEYS_LONG || !q || !K || !V || !out) {
     set_err(nullptr, "hq_debug_attention_prefix: bad argument");
     return HQ_ERR_INVALID;
   }
@@ -2155,6 +2175,7 @@ extern "C" int hq_debug_attention_prefix(int prec, const void* q, const void* K,
   tmp.D = n_heads * 64;
   tmp.nh = n_heads;
   tmp.prefix_pass = variant != 1;
+  if ((rc = set_attn_attrs(&tmp))) return rc;
   with_act(tmp.prec, [&](auto tag) {
     using AT = decltype(tag);
     attention<AT>(&tmp, st, static_cast<const AT*>(q), static_cast<const AT*>(K), static_cast<const AT*>(V), static_cast<AT*>(out),

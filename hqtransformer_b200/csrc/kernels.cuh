@@ -432,17 +432,20 @@ layernorm_kernel(int trace_id, float* __restrict__ x, const float* __restrict__ 
 //   n_keys = causal ? kbase + i + 1 : kbase      (scores scaled by 1/8 = hs^-1/2, layers.py:102)
 // Used for: spatial decode (Tq = 1, kbase = t + 1), depth pass 1 (Tq = 4, kbase = 5), text prefill (causal).
 // ------------------------------------------------------------------------------------------------
+// MAXK: score-row capacity.  Launches over <= ATT_MAX_KEYS keys use the 128-key instance; longer caches the
+// ATT_MAX_KEYS_LONG one (a 64-token text prefix and 256 image positions need 319 keys).
 constexpr int ATT_MAX_KEYS = 128;
+constexpr int ATT_MAX_KEYS_LONG = 320;
 constexpr int ATT_WARPS = 8;
 
-template <typename AT>
+template <typename AT, int MAXK = ATT_MAX_KEYS>
 __global__ void __launch_bounds__(ATT_WARPS * 32)
 attention_kernel(int trace_id, const AT* __restrict__ q, const AT* __restrict__ K, const AT* __restrict__ V, AT* __restrict__ out,
                  int M, int n_heads, int D, int Tq, int t_stride, int kbase, int causal) {
   TraceScope trace_scope(trace_id);
   pdl_launch_dependents();   // programmatic dependent launch: let the next kernel get resident ...
   pdl_wait();                // ... and wait for the previous kernel's results (no-ops without the launch attribute)
-  __shared__ float sc[ATT_WARPS][ATT_MAX_KEYS];
+  __shared__ float sc[ATT_WARPS][MAXK];
   const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int item = blockIdx.x * ATT_WARPS + w;
   if (item >= M * n_heads) return;
@@ -692,7 +695,7 @@ attention_depth4_kernel(int trace_id, const AT* __restrict__ q, const AT* __rest
 constexpr int ATTD_MAXHPC = 24;   // heads (consumer warps) per CTA
 constexpr int ATTD_STAGES = 4;
 
-template <typename AT>
+template <typename AT, int MAXK = ATT_MAX_KEYS>
 __global__ void __launch_bounds__((ATTD_MAXHPC + 1) * 32)
 attention_decode_kernel(int trace_id, const AT* __restrict__ q, const AT* __restrict__ K, const AT* __restrict__ V,
                         AT* __restrict__ out, int D, int t_stride, int n_keys, int CH, int hpc, int groups,
@@ -704,8 +707,8 @@ attention_decode_kernel(int trace_id, const AT* __restrict__ q, const AT* __rest
   const int row_bytes = slice * static_cast<int>(sizeof(AT));
   const int stage_bytes = CH * row_bytes;
   uint8_t* ring = att_smem;
-  float* sc = reinterpret_cast<float*>(att_smem + ATTD_STAGES * stage_bytes);              // [hpc][ATT_MAX_KEYS]
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(sc + hpc * ATT_MAX_KEYS);
+  float* sc = reinterpret_cast<float*>(att_smem + ATTD_STAGES * stage_bytes);              // [hpc][MAXK]
+  uint64_t* full_bar = reinterpret_cast<uint64_t*>(sc + hpc * MAXK);
   uint64_t* empty_bar = full_bar + ATTD_STAGES;
   const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int b = blockIdx.x / groups, grp = blockIdx.x % groups;
@@ -766,7 +769,7 @@ attention_decode_kernel(int trace_id, const AT* __restrict__ q, const AT* __rest
   load8(q + static_cast<size_t>(b) * D + h * 64 + c * 8, qv);
 #pragma unroll
   for (int e = 0; e < 8; ++e) qv[e] *= 0.125f;     // hs^-1/2 = 2^-3 is exact: same products as scaling K (layers.py:102)
-  float* row = sc + w * ATT_MAX_KEYS;
+  float* row = sc + w * MAXK;
   if (threadIdx.x == 0) phase_mark(2);
   int i = 0;
   for (; i < nck; ++i) {
@@ -1289,6 +1292,161 @@ attention_prefix_kernel(int trace_id, const AT* __restrict__ q, const AT* __rest
       }
     }
   }
+  const float inv_a = 1.0f / sum_a, inv_b = 1.0f / sum_b;
+  AT* oa = out + (static_cast<size_t>(b) * Tq + ra) * D + h * 64 + 2 * tq;
+  AT* ob = out + (static_cast<size_t>(b) * Tq + rb) * D + h * 64 + 2 * tq;
+#pragma unroll
+  for (int nt = 0; nt < 8; ++nt) {
+    if (ra < Tq) *reinterpret_cast<uint32_t*>(oa + nt * 8) = pack2_rn<AT>(o[nt][0] * inv_a, o[nt][1] * inv_a);
+    if (rb < Tq) *reinterpret_cast<uint32_t*>(ob + nt * 8) = pack2_rn<AT>(o[nt][2] * inv_b, o[nt][3] * inv_b);
+  }
+#endif
+}
+
+// ------------------------------------------------------------------------------------------------
+// The same causal prefix attention for ATT_MAX_KEYS < Tq <= ATT_MAX_KEYS_LONG (full-context completions).  Grid
+// (B * n_heads, Tq / 128 rounded up): the CTA of query block qb owns queries 128 qb .. 128 qb + 127 and stages keys and
+// values 0 .. its last query once, in dynamic shared memory (<= 320 rows x 144 B each).  A warp's 16 queries see up to
+// 320 keys, more scores than registers hold, so it sweeps them twice in chunks of 128 keys: the first sweep takes the row
+// maxima, the second recomputes the scores and forms p = exp(s - max), the row sums and P V.  Every p, sum and output
+// is the arithmetic attention_prefix_kernel would do with room for all scores (same mma.sync products, fp32 softmax,
+// split-P value MMA, the same per-lane summation order).
+// ------------------------------------------------------------------------------------------------
+constexpr int ATTP_QBLOCK = 128;  // queries per CTA (8 warps x 16)
+
+__host__ __device__ constexpr int attp_long_smem_bytes(int rows, int esz) { return 2 * rows * ATTP_PITCH * esz; }
+
+template <typename AT>
+__global__ void __launch_bounds__(256)
+attention_prefix_long_kernel(int trace_id, const AT* __restrict__ q, const AT* __restrict__ K, const AT* __restrict__ V,
+                             AT* __restrict__ out, int n_heads, int D, int Tq, int t_stride) {
+#if defined(__CUDA_ARCH__)
+  TraceScope trace_scope(trace_id);
+  pdl_launch_dependents();
+  pdl_wait();
+  extern __shared__ __align__(16) uint8_t attp_smem[];
+  const int b = blockIdx.x / n_heads, h = blockIdx.x % n_heads;
+  const int q0 = blockIdx.y * ATTP_QBLOCK;
+  const int qend = (q0 + ATTP_QBLOCK < Tq) ? q0 + ATTP_QBLOCK : Tq;   // keys 0 .. qend - 1 reach this block
+  const int nrows = (qend + 15) & ~15;
+  AT* ks = reinterpret_cast<AT*>(attp_smem);
+  AT* vs = ks + nrows * ATTP_PITCH;
+  const AT* Kb = K + static_cast<size_t>(b) * t_stride * D + h * 64;
+  const AT* Vb = V + static_cast<size_t>(b) * t_stride * D + h * 64;
+  for (int i = threadIdx.x; i < nrows * 8; i += blockDim.x) {
+    const int t = i >> 3, c = (i & 7) * 8;
+    uint4 kv = make_uint4(0u, 0u, 0u, 0u), vv = kv;
+    if (t < qend) {
+      kv = *reinterpret_cast<const uint4*>(Kb + static_cast<size_t>(t) * D + c);
+      vv = *reinterpret_cast<const uint4*>(Vb + static_cast<size_t>(t) * D + c);
+    }
+    *reinterpret_cast<uint4*>(ks + t * ATTP_PITCH + c) = kv;
+    *reinterpret_cast<uint4*>(vs + t * ATTP_PITCH + c) = vv;
+  }
+  __syncthreads();
+  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int r0 = q0 + w * 16;
+  if (r0 >= Tq) return;
+  const int gq = lane >> 2, tq = lane & 3;
+  const int ra = r0 + gq, rb = ra + 8;
+  const int nks = ((r0 + 16 < Tq ? r0 + 16 : Tq) + 15) >> 4;   // 16-key steps holding keys <= the warp's last query
+
+  uint32_t qa[4][4];
+  {
+    const uint32_t* qra = reinterpret_cast<const uint32_t*>(q + (static_cast<size_t>(b) * Tq + (ra < Tq ? ra : 0)) * D + h * 64);
+    const uint32_t* qrb = reinterpret_cast<const uint32_t*>(q + (static_cast<size_t>(b) * Tq + (rb < Tq ? rb : 0)) * D + h * 64);
+#pragma unroll
+    for (int kk = 0; kk < 4; ++kk) {
+      qa[kk][0] = ra < Tq ? qra[kk * 8 + tq] : 0u;
+      qa[kk][1] = rb < Tq ? qrb[kk * 8 + tq] : 0u;
+      qa[kk][2] = ra < Tq ? qra[kk * 8 + 4 + tq] : 0u;
+      qa[kk][3] = rb < Tq ? qrb[kk * 8 + 4 + tq] : 0u;
+    }
+  }
+  // scaled, causally masked scores of the 16 key tiles of chunk c (keys 128c ..): tile j of the chunk = keys 128c + 8j ..
+  float s[16][4];
+  auto scores = [&](int c) {
+#pragma unroll
+    for (int j = 0; j < 16; ++j) {
+#pragma unroll
+      for (int e = 0; e < 4; ++e) s[j][e] = 0.f;
+      const int jt = 16 * c + j;
+      if (jt < 2 * nks) {
+        const uint32_t* krow = reinterpret_cast<const uint32_t*>(ks + (jt * 8 + gq) * ATTP_PITCH);
+#pragma unroll
+        for (int kk = 0; kk < 4; ++kk)
+          mma_16816<AT>(s[j], qa[kk][0], qa[kk][1], qa[kk][2], qa[kk][3], krow[kk * 8 + tq], krow[kk * 8 + 4 + tq]);
+      }
+#pragma unroll
+      for (int e = 0; e < 4; ++e) {
+        const int key = jt * 8 + 2 * tq + (e & 1);
+        const int row = e < 2 ? ra : rb;
+        s[j][e] = (jt < 2 * nks && key <= row) ? s[j][e] * 0.125f : -INFINITY;
+      }
+    }
+  };
+  const int nchunks = (nks + 7) >> 3;
+  // ---- sweep 1: row maxima ----
+  float mx_a = -INFINITY, mx_b = -INFINITY;
+  for (int c = 0; c < nchunks; ++c) {
+    scores(c);
+#pragma unroll
+    for (int j = 0; j < 16; ++j)
+#pragma unroll
+      for (int e = 0; e < 4; ++e) {
+        if (e < 2) mx_a = fmaxf(mx_a, s[j][e]);
+        else mx_b = fmaxf(mx_b, s[j][e]);
+      }
+  }
+  mx_a = fmaxf(mx_a, __shfl_xor_sync(0xffffffffu, mx_a, 1));
+  mx_a = fmaxf(mx_a, __shfl_xor_sync(0xffffffffu, mx_a, 2));
+  mx_b = fmaxf(mx_b, __shfl_xor_sync(0xffffffffu, mx_b, 1));
+  mx_b = fmaxf(mx_b, __shfl_xor_sync(0xffffffffu, mx_b, 2));
+  // ---- sweep 2: p, row sums, O = P V ----
+  float sum_a = 0.f, sum_b = 0.f;
+  float o[8][4];
+#pragma unroll
+  for (int nt = 0; nt < 8; ++nt)
+#pragma unroll
+    for (int e = 0; e < 4; ++e) o[nt][e] = 0.f;
+  const uint32_t vrow = smem_u32(vs) + static_cast<uint32_t>((lane & 15) * ATTP_PITCH * 2);
+  for (int c = 0; c < nchunks; ++c) {
+    scores(c);
+#pragma unroll
+    for (int j = 0; j < 16; ++j)
+#pragma unroll
+      for (int e = 0; e < 4; ++e) {
+        const float p = expf(s[j][e] - (e < 2 ? mx_a : mx_b));    // masked keys: exp(-inf) = 0
+        s[j][e] = p;
+        if (e < 2) sum_a += p;
+        else sum_b += p;
+      }
+#pragma unroll
+    for (int kk = 0; kk < 8; ++kk) {
+      const int kt = 8 * c + kk;                        // 16-key step
+      if (kt < nks) {
+        uint32_t hd[4], tl[4];
+#pragma unroll
+        for (int r = 0; r < 4; ++r) {
+          const int j = 2 * kk + (r >> 1), e = (r & 1) * 2;
+          hd[r] = pack2_rn<AT>(s[j][e], s[j][e + 1]);
+          const float2 f = unpack2<AT>(hd[r]);
+          tl[r] = pack2_rn<AT>(s[j][e] - f.x, s[j][e + 1] - f.y);
+        }
+#pragma unroll
+        for (int nt = 0; nt < 8; ++nt) {
+          uint32_t b0, b1;
+          ldmatrix_x2_trans(vrow + static_cast<uint32_t>((kt * 16 * ATTP_PITCH + nt * 8) * 2), b0, b1);
+          mma_16816<AT>(o[nt], hd[0], hd[1], hd[2], hd[3], b0, b1);
+          mma_16816<AT>(o[nt], tl[0], tl[1], tl[2], tl[3], b0, b1);
+        }
+      }
+    }
+  }
+  sum_a += __shfl_xor_sync(0xffffffffu, sum_a, 1);
+  sum_a += __shfl_xor_sync(0xffffffffu, sum_a, 2);
+  sum_b += __shfl_xor_sync(0xffffffffu, sum_b, 1);
+  sum_b += __shfl_xor_sync(0xffffffffu, sum_b, 2);
   const float inv_a = 1.0f / sum_a, inv_b = 1.0f / sum_b;
   AT* oa = out + (static_cast<size_t>(b) * Tq + ra) * D + h * 64 + 2 * tq;
   AT* ob = out + (static_cast<size_t>(b) * Tq + rb) * D + h * 64 + 2 * tq;

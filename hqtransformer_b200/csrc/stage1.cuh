@@ -749,6 +749,152 @@ s1_attn_mma_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ out, int H, 
 #endif
 }
 
+// ------------------------------------------------------------------------------------------------
+// The same AttnBlock core for S1A_NMAX < N <= S1AL_NMAX tokens (e.g. the 32 x 32 AttnBlocks of a 512 x 512 decode), bf16.
+// A query row's N scores fit neither registers nor shared memory next to Q, so the CTA sweeps the keys twice in chunks
+// of S1AL_KC: sweep 1 keeps the running row max m and sum l (l rescaled when m grows); sweep 2 recomputes the scores and
+// forms P = exp(s - m) / l - at the point where s1_attn_mma_kernel forms it - straight into A fragments of O += P V, as a
+// bf16 head and tail (attention_prefix_kernel's split: P carried to ~2^-17 instead of bf16's 2^-8).  Over up to 1024
+// keys the 2^-8 rounding of P alone would exceed the CUDA-core kernel's error, which this kernel replaces.
+// CTA = (64 queries, one 128-channel block of the output, image): Q [64][C + 8] resident, K chunk (+ V chunk of the block
+// in sweep 2) double-buffered by cp.async.  Scores are the same mma.sync products as s1_attn_mma_kernel's.
+// N % 16 == 0, C a multiple of 128, <= 512.
+// ------------------------------------------------------------------------------------------------
+constexpr int S1AL_NMAX = 1024, S1AL_KC = 32;
+__host__ __device__ constexpr int s1al_smem_bytes(int C) {
+  return (S1A_Q * (C + S1A_PAD) + 2 * S1AL_KC * (C + S1A_PAD) + 2 * S1AL_KC * (S1A_CB + S1A_PAD)) * 2;
+}
+
+__global__ void __launch_bounds__(128, 1)
+s1_attn_mma_long_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ out, int H, int W, int C) {
+#if defined(__CUDA_ARCH__)
+  extern __shared__ __align__(16) uint8_t s1a_smem[];
+  const int N = H * W, Wp = W + 2;
+  const int qp = C + S1A_PAD, vp = S1A_CB + S1A_PAD;
+  bf16* Qs = reinterpret_cast<bf16*>(s1a_smem);                 // [64][C + 8]
+  bf16* Ks = Qs + S1A_Q * qp;                                   // 2 x [32][C + 8]
+  bf16* Vs = Ks + 2 * S1AL_KC * qp;                             // 2 x [32][128 + 8]
+  const int q0 = blockIdx.x * S1A_Q, cb = blockIdx.y, b = blockIdx.z;
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, t = lane & 3;
+  const size_t img = static_cast<size_t>(b) * (H + 2) * Wp;
+  auto prow = [&](int n) { return img + static_cast<size_t>((n / W + 1) * Wp + (n % W + 1)); };
+  auto load_rows = [&](bf16* dst, int pitch, int rows, int n_first, int col0, int ncol8) {
+    for (int i = tid; i < rows * ncol8; i += 128) {
+      const int r = i / ncol8, c = (i - r * ncol8) * 8, n = n_first + r;
+      if (n < N) cp_async16(smem_u32(dst + r * pitch + c), qkv + prow(n) * 3 * C + col0 + c);
+      else *reinterpret_cast<uint4*>(dst + r * pitch + c) = make_uint4(0u, 0u, 0u, 0u);
+    }
+  };
+  const int nkc = (N + S1AL_KC - 1) / S1AL_KC, steps = 2 * nkc;
+  // step i: sweep i / nkc over key chunk i % nkc; sweep 2 also brings the chunk's values of this channel block
+  auto load_step = [&](int i) {
+    const int kc = i % nkc, buf = i & 1;
+    load_rows(Ks + buf * S1AL_KC * qp, qp, S1AL_KC, kc * S1AL_KC, C, C / 8);
+    if (i >= nkc) load_rows(Vs + buf * S1AL_KC * vp, vp, S1AL_KC, kc * S1AL_KC, 2 * C + cb * S1A_CB, S1A_CB / 8);
+  };
+  load_rows(Qs, qp, S1A_Q, q0, 0, C / 8);
+  load_step(0);
+  cp_async_commit();
+  const uint32_t qs_u32 = smem_u32(Qs), ks_u32 = smem_u32(Ks), vs_u32 = smem_u32(Vs);
+  const int a_row = (lane & 7) + ((lane >> 3) & 1) * 8, a_col = (lane >> 4) * 8;
+  const int b_row = lane & 7, b_col = ((lane >> 3) & 1) * 8;
+  const float scale = rsqrtf(static_cast<float>(C));
+  float m0 = -INFINITY, m1 = -INFINITY, l0 = 0.f, l1 = 0.f, i0 = 0.f, i1 = 0.f;
+  float O[S1A_CB / 8][4];
+#pragma unroll
+  for (int i = 0; i < S1A_CB / 8; ++i) O[i][0] = O[i][1] = O[i][2] = O[i][3] = 0.f;
+  for (int i = 0; i < steps; ++i) {
+    if (i + 1 < steps) load_step(i + 1);
+    cp_async_commit();
+    cp_async_wait<1>();
+    __syncthreads();
+    const int kc = i % nkc, buf = i & 1;
+    const bool sweep2 = i >= nkc;
+    if (i == nkc) {                                             // row sums complete: 1 / l
+      l0 += __shfl_xor_sync(0xffffffffu, l0, 1); l0 += __shfl_xor_sync(0xffffffffu, l0, 2);
+      l1 += __shfl_xor_sync(0xffffffffu, l1, 1); l1 += __shfl_xor_sync(0xffffffffu, l1, 2);
+      i0 = 1.0f / l0;
+      i1 = 1.0f / l1;
+    }
+    // ---- scores of the chunk: 4 tiles of 8 keys ----
+    float S[S1AL_KC / 8][4];
+#pragma unroll
+    for (int j = 0; j < S1AL_KC / 8; ++j) S[j][0] = S[j][1] = S[j][2] = S[j][3] = 0.f;
+    const uint32_t kb_u32 = ks_u32 + static_cast<uint32_t>(buf * S1AL_KC * qp * 2);
+    for (int ks = 0; ks < C / 16; ++ks) {
+      uint32_t a0, a1, a2, a3;
+      ldsm_x4(qs_u32 + static_cast<uint32_t>(((warp * 16 + a_row) * qp + ks * 16 + a_col) * 2), a0, a1, a2, a3);
+#pragma unroll
+      for (int nb = 0; nb < S1AL_KC / 8; ++nb) {
+        uint32_t b0, b1;
+        ldmatrix_x2(kb_u32 + static_cast<uint32_t>(((nb * 8 + b_row) * qp + ks * 16 + b_col) * 2), b0, b1);
+        mma_bf16_16816(S[nb], a0, a1, a2, a3, b0, b1);
+      }
+    }
+#pragma unroll
+    for (int j = 0; j < S1AL_KC / 8; ++j) {
+      const int col = kc * S1AL_KC + j * 8 + 2 * t;
+      S[j][0] = col < N ? S[j][0] * scale : -INFINITY;
+      S[j][1] = col + 1 < N ? S[j][1] * scale : -INFINITY;
+      S[j][2] = col < N ? S[j][2] * scale : -INFINITY;
+      S[j][3] = col + 1 < N ? S[j][3] * scale : -INFINITY;
+    }
+    if (!sweep2) {
+      // ---- sweep 1: running max and (per-lane partial) sum of the rows g and g + 8 ----
+      float c0 = -INFINITY, c1 = -INFINITY;
+#pragma unroll
+      for (int j = 0; j < S1AL_KC / 8; ++j) {
+        c0 = fmaxf(c0, fmaxf(S[j][0], S[j][1]));
+        c1 = fmaxf(c1, fmaxf(S[j][2], S[j][3]));
+      }
+      c0 = fmaxf(c0, __shfl_xor_sync(0xffffffffu, c0, 1)); c0 = fmaxf(c0, __shfl_xor_sync(0xffffffffu, c0, 2));
+      c1 = fmaxf(c1, __shfl_xor_sync(0xffffffffu, c1, 1)); c1 = fmaxf(c1, __shfl_xor_sync(0xffffffffu, c1, 2));
+      const float n0 = fmaxf(m0, c0), n1 = fmaxf(m1, c1);      // >= one real key per chunk: finite
+      l0 *= expf(m0 - n0);                                      // first chunk: exp(-inf) = 0
+      l1 *= expf(m1 - n1);
+#pragma unroll
+      for (int j = 0; j < S1AL_KC / 8; ++j) {
+        l0 += expf(S[j][0] - n0) + expf(S[j][1] - n0);
+        l1 += expf(S[j][2] - n1) + expf(S[j][3] - n1);
+      }
+      m0 = n0;
+      m1 = n1;
+    } else {
+      // ---- sweep 2: P (bf16, normalised) as A fragments; O += P V over the chunk's 32 keys ----
+      const uint32_t vb_u32 = vs_u32 + static_cast<uint32_t>(buf * S1AL_KC * vp * 2);
+#pragma unroll
+      for (int ks = 0; ks < S1AL_KC / 16; ++ks) {
+        uint32_t a[4], at[4];
+#pragma unroll
+        for (int r = 0; r < 4; ++r) {
+          const int j = 2 * ks + (r >> 1);
+          const float p0 = (r & 1) ? expf(S[j][2] - m1) * i1 : expf(S[j][0] - m0) * i0;
+          const float p1 = (r & 1) ? expf(S[j][3] - m1) * i1 : expf(S[j][1] - m0) * i0;
+          a[r] = pack2_rn<bf16>(p0, p1);
+          const float2 f = unpack2<bf16>(a[r]);
+          at[r] = pack2_rn<bf16>(p0 - f.x, p1 - f.y);
+        }
+#pragma unroll
+        for (int nb = 0; nb < S1A_CB / 8; ++nb) {
+          uint32_t b0, b1;
+          ldmatrix_x2_trans(vb_u32 + static_cast<uint32_t>(((ks * 16 + (lane & 7) + ((lane >> 3) & 1) * 8) * vp + nb * 8) * 2), b0, b1);
+          mma_bf16_16816(O[nb], a[0], a[1], a[2], a[3], b0, b1);
+          mma_bf16_16816(O[nb], at[0], at[1], at[2], at[3], b0, b1);
+        }
+      }
+    }
+    __syncthreads();                                            // buffer consumed: step i + 2 may refill it
+  }
+  const int n0 = q0 + warp * 16 + g, n1 = n0 + 8;
+#pragma unroll
+  for (int nb = 0; nb < S1A_CB / 8; ++nb) {
+    const int col = cb * S1A_CB + nb * 8 + 2 * t;
+    if (n0 < N) *reinterpret_cast<__nv_bfloat162*>(out + prow(n0) * C + col) = __floats2bfloat162_rn(O[nb][0], O[nb][1]);
+    if (n1 < N) *reinterpret_cast<__nv_bfloat162*>(out + prow(n1) * C + col) = __floats2bfloat162_rn(O[nb][2], O[nb][3]);
+  }
+#endif
+}
+
 // conv weight [Cout, Cin, k, k] (fp32 / bf16 / fp16 source already converted to fp32) -> T [CoutPad, k*k*Cin] tap-major
 // (bf16, or fp32 rounded to TF32)
 template <typename T>

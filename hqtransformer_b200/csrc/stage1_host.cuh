@@ -46,6 +46,7 @@ struct hq_s1_ctx {
   float2* gn_stat = nullptr;      // [B][32] (mean, rstd) published by the last slice CTA
   unsigned* gn_cnt = nullptr;     // [B] ticket counters (wrap to 0)
   size_t act_elems = 0;                 // elements of X / T / S / H / H2 per buffer
+  int grid_lat = 0;                     // latent resolution the activation buffers and QKV are sized for (>= the config's)
   size_t device_bytes = 0;
   std::vector<void*> allocs;
   cudaError_t launch_err = cudaSuccess;
@@ -71,13 +72,24 @@ static void s1_err(hq_s1_ctx* ctx, const char* fmt, ...) {
     }                                                                                            \
   } while (0)
 
+static size_t s1_round_bytes(size_t bytes) { return (bytes + 255) & ~static_cast<size_t>(255); }
+
 static int s1_alloc(hq_s1_ctx* ctx, void** p, size_t bytes) {
-  bytes = (bytes + 255) & ~static_cast<size_t>(255);
+  bytes = s1_round_bytes(bytes);
   S1_CUDA(ctx, cudaMalloc(p, bytes));
   S1_CUDA(ctx, cudaMemset(*p, 0, bytes));
   ctx->allocs.push_back(*p);
   ctx->device_bytes += bytes;
   return HQ_OK;
+}
+
+// frees a buffer of s1_alloc (bytes: the size it was allocated with); *p becomes null
+static void s1_free(hq_s1_ctx* ctx, void** p, size_t bytes) {
+  if (!*p) return;
+  cudaFree(*p);
+  ctx->allocs.erase(std::find(ctx->allocs.begin(), ctx->allocs.end(), *p));
+  ctx->device_bytes -= s1_round_bytes(bytes);
+  *p = nullptr;
 }
 
 // a [rows, cols] matrix of the ctx's operand type, boxes of one 128-byte swizzled row (64 bf16 | 32 fp32) x box_rows
@@ -186,6 +198,100 @@ static int s1_open(hq_s1_ctx* ctx, int device) {
   S1_CUDA(ctx, cudaFuncSetAttribute(s1_attn_kernel<bf16>, cudaFuncAttributeMaxDynamicSharedMemorySize, S1_ATT_SMEM_MAX));
   S1_CUDA(ctx, cudaFuncSetAttribute(s1_attn_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, S1_ATT_SMEM_MAX));
   S1_CUDA(ctx, cudaFuncSetAttribute(s1_attn_mma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+  S1_CUDA(ctx, cudaFuncSetAttribute(s1_attn_mma_long_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, s1al_smem_bytes(S1A_CMAX)));
+  return HQ_OK;
+}
+
+// whether the AttnBlock core over N tokens of C channels runs on the tensor cores (bf16 only): s1_attn_mma_kernel up to
+// S1A_NMAX tokens, s1_attn_mma_long_kernel up to S1AL_NMAX
+template <typename T>
+static bool s1_attn_uses_mma(int N, int C) {
+  return std::is_same<T, bf16>::value && N % 16 == 0 && N <= S1A_NMAX && C % S1A_CB == 0 && C <= S1A_CMAX;
+}
+template <typename T>
+static bool s1_attn_uses_mma_long(int N, int C) {
+  return std::is_same<T, bf16>::value && N % 16 == 0 && N > S1A_NMAX && N <= S1AL_NMAX && C % S1A_CB == 0 && C <= S1A_CMAX;
+}
+// whether the CUDA-core core's shared memory (S1_ATT_Q rows of C + N fp32) fits
+static bool s1_attn_simt_fits(int N, int C) {
+  return static_cast<size_t>(S1_ATT_Q) * (C + N) * 4 <= static_cast<size_t>(S1_ATT_SMEM_MAX);
+}
+
+static int s1_config_lat(const hq_s1_config& cfg) { return cfg.resolution >> cfg.n_levels; }
+
+// Resolutions of a decode from a latent grid of `lat` cells: the mid blocks at lat, up level i at lat << i.  AttnBlocks stay
+// where the configuration put them (S1Level::has_attn, from each level's resolution at the configured size).
+// Activation elements per image: max over the layer sequence of (padded positions) x channels.
+static size_t s1_act_per_img(const hq_s1_ctx* ctx, int lat) {
+  const hq_s1_config& cfg = ctx->cfg;
+  const int top = ctx->conv_in.Cout;
+  size_t per_img = static_cast<size_t>(lat + 2) * (lat + 2) * std::max(std::max(2 * cfg.embed_dim, cfg.z_channels), top);
+  int res = lat;
+  for (const S1Level& lv : ctx->levels) {
+    for (const S1Res& r : lv.blocks)
+      per_img = std::max(per_img, static_cast<size_t>(res + 2) * (res + 2) * std::max(r.c1.Cin, r.c1.Cout));
+    res *= 2;
+    per_img = std::max(per_img, static_cast<size_t>(res + 2) * (res + 2) * lv.up.Cin);
+  }
+  return per_img;
+}
+
+// Elements of QKV per image (the largest AttnBlock input: 3C channels at its resolution, padded); 0 if C or N is beyond
+// what the attention cores take.
+static size_t s1_qkv_per_img(const hq_s1_ctx* ctx, int lat, bool bf16_core) {
+  size_t per_img = 0;
+  auto att = [&](int res, int C) {
+    const int N = res * res;
+    const bool mma = bf16_core && (s1_attn_uses_mma<bf16>(N, C) || s1_attn_uses_mma_long<bf16>(N, C));
+    if (!mma && !s1_attn_simt_fits(N, C)) return false;
+    per_img = std::max(per_img, static_cast<size_t>(res + 2) * (res + 2) * 3 * C);
+    return true;
+  };
+  if (!att(lat, ctx->mid_attn.n.C)) return 0;
+  int res = lat;
+  for (const S1Level& lv : ctx->levels) {
+    for (const S1Attn& a : lv.attns)
+      if (!att(res, a.n.C)) return 0;
+    res *= 2;
+  }
+  return per_img;
+}
+
+// (Re)allocates X / T / S / H / H2 and QKV for decodes from latent grids up to `lat` cells; no-op if they are that large.
+static int s1_size_buffers(hq_s1_ctx* ctx, int lat) {
+  if (lat <= ctx->grid_lat) return HQ_OK;
+  const size_t qkv = s1_qkv_per_img(ctx, lat, ctx->prec == HQ_PREC_BF16);
+  if (qkv == 0) {
+    s1_err(ctx, "latent grid %d x %d: an AttnBlock there exceeds the attention kernels (tokens x channels)", lat, lat);
+    return HQ_ERR_UNSUPPORTED;
+  }
+  const size_t B = static_cast<size_t>(ctx->max_batch);
+  const size_t elems = s1_act_per_img(ctx, lat) * B;
+  // the new buffers are allocated before the old ones are freed: a failed reserve leaves the decoder as it was
+  void* fresh[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+  const size_t bytes[6] = {elems * 4, elems * 4, elems * 4, elems * ctx->esz, elems * ctx->esz, B * qkv * ctx->esz};
+  for (int i = 0; i < 6; ++i) {
+    const int rc = s1_alloc(ctx, &fresh[i], bytes[i]);
+    if (rc) {
+      cudaGetLastError();                     // an out-of-memory error must not surface as a later launch error
+      for (int j = 0; j < i; ++j) s1_free(ctx, &fresh[j], bytes[j]);
+      return rc;
+    }
+  }
+  s1_free(ctx, reinterpret_cast<void**>(&ctx->X), ctx->act_elems * 4);
+  s1_free(ctx, reinterpret_cast<void**>(&ctx->T), ctx->act_elems * 4);
+  s1_free(ctx, reinterpret_cast<void**>(&ctx->S), ctx->act_elems * 4);
+  s1_free(ctx, &ctx->H, ctx->act_elems * ctx->esz);
+  s1_free(ctx, &ctx->H2, ctx->act_elems * ctx->esz);
+  if (ctx->grid_lat) s1_free(ctx, &ctx->QKV, B * s1_qkv_per_img(ctx, ctx->grid_lat, ctx->prec == HQ_PREC_BF16) * ctx->esz);
+  ctx->X = static_cast<float*>(fresh[0]);
+  ctx->T = static_cast<float*>(fresh[1]);
+  ctx->S = static_cast<float*>(fresh[2]);
+  ctx->H = fresh[3];
+  ctx->H2 = fresh[4];
+  ctx->QKV = fresh[5];
+  ctx->act_elems = elems;
+  ctx->grid_lat = lat;
   return HQ_OK;
 }
 
@@ -215,8 +321,6 @@ static int s1_create_impl(hq_s1_ctx* ctx, const hq_s1_config* cfg, int device, i
   if ((rc = s1_make_res(ctx, &ctx->mid1, "decoder.mid.block_1", top, top))) return rc;
   if ((rc = s1_make_attn(ctx, &ctx->mid_attn, "decoder.mid.attn_1", top))) return rc;
   if ((rc = s1_make_res(ctx, &ctx->mid2, "decoder.mid.block_2", top, top))) return rc;
-  // activation buffer size: max over the layer sequence of (padded positions per image) x channels
-  size_t per_img = static_cast<size_t>(lat + 2) * (lat + 2) * std::max(std::max(2 * E, cfg->z_channels), top);
   int block_in = top, res = lat;
   ctx->levels.resize(L);
   for (int i = 0; i < L; ++i) {
@@ -229,7 +333,6 @@ static int s1_create_impl(hq_s1_ctx* ctx, const hq_s1_config* cfg, int device, i
     if (lv.has_attn) lv.attns.resize(cfg->num_res_blocks + 1);
     for (int j = 0; j <= cfg->num_res_blocks; ++j) {
       const std::string p = "decoder.up." + std::to_string(lvl) + ".block." + std::to_string(j);
-      per_img = std::max(per_img, static_cast<size_t>(res + 2) * (res + 2) * std::max(block_in, block_out));
       if ((rc = s1_make_res(ctx, &lv.blocks[j], p, block_in, block_out))) return rc;
       block_in = block_out;
       if (lv.has_attn &&
@@ -238,23 +341,13 @@ static int s1_create_impl(hq_s1_ctx* ctx, const hq_s1_config* cfg, int device, i
     }
     if ((rc = s1_make_conv(ctx, &lv.up, {"decoder.up." + std::to_string(lvl) + ".upsample.conv"}, block_in, block_in, 3))) return rc;
     res *= 2;
-    per_img = std::max(per_img, static_cast<size_t>(res + 2) * (res + 2) * block_in);
   }
   if ((rc = s1_make_norm(ctx, &ctx->norm_out, "decoder.norm_out", block_in))) return rc;
   if ((rc = s1_make_conv(ctx, &ctx->conv_out, {"decoder.conv_out"}, block_in, cfg->out_ch, 3))) return rc;
-  ctx->act_elems = per_img * max_batch;
-  if ((rc = s1_alloc(ctx, reinterpret_cast<void**>(&ctx->X), ctx->act_elems * 4))) return rc;
-  if ((rc = s1_alloc(ctx, reinterpret_cast<void**>(&ctx->T), ctx->act_elems * 4))) return rc;
-  if ((rc = s1_alloc(ctx, reinterpret_cast<void**>(&ctx->S), ctx->act_elems * 4))) return rc;
-  if ((rc = s1_alloc(ctx, &ctx->H, ctx->act_elems * ctx->esz))) return rc;
-  if ((rc = s1_alloc(ctx, &ctx->H2, ctx->act_elems * ctx->esz))) return rc;
-  const int att_res = cfg->attn_resolution > 0 ? cfg->attn_resolution : lat;
-  if ((rc = s1_alloc(ctx, &ctx->QKV, static_cast<size_t>(max_batch) * (att_res + 2) * (att_res + 2) * 3 * top * ctx->esz)))
-    return rc;
   if ((rc = s1_alloc(ctx, reinterpret_cast<void**>(&ctx->gn_part), static_cast<size_t>(max_batch) * 32 * 64 * 2 * 8))) return rc;
   if ((rc = s1_alloc(ctx, reinterpret_cast<void**>(&ctx->gn_stat), static_cast<size_t>(max_batch) * 32 * 8))) return rc;
   if ((rc = s1_alloc(ctx, reinterpret_cast<void**>(&ctx->gn_cnt), static_cast<size_t>(max_batch) * 4))) return rc;
-  return HQ_OK;
+  return s1_size_buffers(ctx, lat);
 }
 
 extern "C" int hq_s1_create(const hq_s1_config* cfg, int device, int max_batch, hq_s1_ctx** out) {
@@ -435,12 +528,6 @@ static void s1_resblock(hq_s1_ctx* ctx, cudaStream_t st, const S1Res& r, int B, 
   }
 }
 
-// whether the AttnBlock core over N tokens of C channels runs on the tensor cores (s1_attn_mma_kernel, bf16 only)
-template <typename T>
-static bool s1_attn_uses_mma(int N, int C) {
-  return std::is_same<T, bf16>::value && N % 16 == 0 && N <= S1A_NMAX && C % S1A_CB == 0 && C <= S1A_CMAX;
-}
-
 // AttnBlock core: qkv (padded [B, res+2, res+2, 3C]) -> out (padded [B, res+2, res+2, C], interior only).  bf16: the
 // tensor-core kernel where the shape allows (force_simt: the CUDA-core kernel regardless); float: the fp32 core.
 template <typename T>
@@ -451,6 +538,10 @@ static void s1_attn_core(hq_s1_ctx* ctx, cudaStream_t st, const void* qkv, void*
     const size_t smem = static_cast<size_t>(s1a_smem_bytes(C));
     s1_attn_mma_kernel<<<dim3((N + S1A_Q - 1) / S1A_Q, B), 128, smem, st>>>(static_cast<const bf16*>(qkv),
                                                                              static_cast<bf16*>(out), res, res, C);
+  } else if (!force_simt && s1_attn_uses_mma_long<T>(N, C)) {
+    // longer token counts: two sweeps over 32-key chunks, one CTA per (64 queries, 128 output channels, image)
+    s1_attn_mma_long_kernel<<<dim3((N + S1A_Q - 1) / S1A_Q, C / S1A_CB, B), 128, static_cast<size_t>(s1al_smem_bytes(C)), st>>>(
+        static_cast<const bf16*>(qkv), static_cast<bf16*>(out), res, res, C);
   } else {
     const size_t smem = static_cast<size_t>(S1_ATT_Q) * (C + N) * 4;
     s1_attn_kernel<T><<<dim3((N + S1_ATT_Q - 1) / S1_ATT_Q, B), 256, smem, st>>>(static_cast<const T*>(qkv),
@@ -470,9 +561,8 @@ static void s1_attnblock(hq_s1_ctx* ctx, cudaStream_t st, const S1Attn& a, int B
 
 // the layer sequence of decode_code (generator.py:316-367) in operand type T
 template <typename T>
-static void s1_decode(hq_s1_ctx* ctx, cudaStream_t st, const int64_t* code_t, const int64_t* code_b, float* out, int B) {
+static void s1_decode(hq_s1_ctx* ctx, cudaStream_t st, const int64_t* code_t, const int64_t* code_b, float* out, int B, int lat) {
   const hq_s1_config& cfg = ctx->cfg;
-  const int lat = cfg.resolution >> cfg.n_levels;
   // codes -> [quant_t (pixel-shuffled) | quant_b] -> post_quant_conv_b -> conv_in
   s1_quant<T>(ctx, st, code_t, code_b, ctx->E_t, ctx->E_b, ctx->H, B, cfg.embed_dim, lat, cfg.n_embed);
   s1_conv<T>(ctx, st, ctx->post_quant, ctx->H, B, lat, S1_OUT_F32, ctx->X, nullptr, nullptr);
@@ -497,8 +587,8 @@ static void s1_decode(hq_s1_ctx* ctx, cudaStream_t st, const int64_t* code_t, co
   s1_conv<T>(ctx, st, ctx->conv_out, ctx->H, B, res, S1_OUT_IMAGE, out, nullptr, nullptr);
 }
 
-// `SimRQGAN2Generator.decode_code` (generator.py:323-367) with both grids given; device pointers; asynchronous on `stream`.
-extern "C" int hq_s1_decode_codes(hq_s1_ctx* ctx, const int64_t* code_t, const int64_t* code_b, float* out, int B, void* stream) {
+// decode from a latent grid of `lat` cells (buffers sized for it)
+static int s1_decode_at(hq_s1_ctx* ctx, const int64_t* code_t, const int64_t* code_b, float* out, int B, int lat, void* stream) {
   if (!ctx || !code_t || !code_b || !out) return HQ_ERR_INVALID;
   int rc = hq_s1_params_complete(ctx);
   if (rc) return rc;
@@ -506,17 +596,48 @@ extern "C" int hq_s1_decode_codes(hq_s1_ctx* ctx, const int64_t* code_t, const i
     s1_err(ctx, "batch %d outside [1, max_batch=%d]", B, ctx->max_batch);
     return HQ_ERR_INVALID;
   }
+  if (lat > ctx->grid_lat) {
+    s1_err(ctx, "latent grid %d x %d: buffers are sized for %d x %d", lat, lat, ctx->grid_lat, ctx->grid_lat);
+    return HQ_ERR_STATE;
+  }
   S1_CUDA(ctx, cudaSetDevice(ctx->device));
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   ctx->launch_err = cudaSuccess;
   ctx->conv_flops = 0.0;
-  if (ctx->prec == HQ_PREC_TF32) s1_decode<float>(ctx, st, code_t, code_b, out, B);
-  else s1_decode<bf16>(ctx, st, code_t, code_b, out, B);
+  if (ctx->prec == HQ_PREC_TF32) s1_decode<float>(ctx, st, code_t, code_b, out, B, lat);
+  else s1_decode<bf16>(ctx, st, code_t, code_b, out, B, lat);
   if (ctx->launch_err != cudaSuccess) {
     s1_err(ctx, "stage-1 kernel launch failed: %s", cudaGetErrorString(ctx->launch_err));
     return HQ_ERR_CUDA;
   }
   return HQ_OK;
+}
+
+// `SimRQGAN2Generator.decode_code` (generator.py:323-367) with both grids given; device pointers; asynchronous on `stream`.
+extern "C" int hq_s1_decode_codes(hq_s1_ctx* ctx, const int64_t* code_t, const int64_t* code_b, float* out, int B, void* stream) {
+  return s1_decode_at(ctx, code_t, code_b, out, B, ctx ? s1_config_lat(ctx->cfg) : 0, stream);
+}
+
+extern "C" int hq_s1_reserve_grid(hq_s1_ctx* ctx, int top_res) {
+  if (!ctx) return HQ_ERR_INVALID;
+  if (top_res < 1 || top_res > 1024) {
+    s1_err(ctx, "hq_s1_reserve_grid: top grid %d outside [1, 1024]", top_res);
+    return HQ_ERR_INVALID;
+  }
+  S1_CUDA(ctx, cudaSetDevice(ctx->device));
+  S1_CUDA(ctx, cudaDeviceSynchronize());      // decodes in flight may still use the buffers being replaced
+  return s1_size_buffers(ctx, 2 * top_res);
+}
+
+extern "C" int hq_s1_decode_codes_grid(hq_s1_ctx* ctx, const int64_t* code_t, const int64_t* code_b, int top_res, float* out, int B,
+                                       void* stream) {
+  if (!ctx) return HQ_ERR_INVALID;
+  if (top_res < 1 || 2 * top_res > ctx->grid_lat) {
+    s1_err(ctx, "top grid %d x %d: reserved up to %d x %d (hq_s1_reserve_grid)", top_res, top_res, ctx->grid_lat / 2,
+           ctx->grid_lat / 2);
+    return HQ_ERR_INVALID;
+  }
+  return s1_decode_at(ctx, code_t, code_b, out, B, 2 * top_res, stream);
 }
 
 // ---- test hooks (include/hqgraft.h): one decoder layer through the host function the decode calls, on a throw-away ctx ----
@@ -626,9 +747,9 @@ extern "C" int hq_debug_s1_quant(int prec, const int64_t* code_t, const int64_t*
 
 extern "C" int hq_debug_s1_attention(int prec, const void* qkv, void* out, int B, int res, int C, int variant, void* stream) {
   const int N = res * res;
-  const bool simt = variant == 1 || !(prec == HQ_PREC_BF16 ? s1_attn_uses_mma<bf16>(N, C) : s1_attn_uses_mma<float>(N, C));
+  const bool simt = variant == 1 || prec != HQ_PREC_BF16 || !(s1_attn_uses_mma<bf16>(N, C) || s1_attn_uses_mma_long<bf16>(N, C));
   if (!qkv || !out || B < 1 || res < 1 || C < 8 || C % 8 != 0 || (variant != 0 && variant != 1) ||
-      (simt && static_cast<size_t>(S1_ATT_Q) * (C + N) * 4 > static_cast<size_t>(S1_ATT_SMEM_MAX))) {
+      (simt && !s1_attn_simt_fits(N, C))) {
     s1_err(nullptr, "hq_debug_s1_attention: bad argument");
     return HQ_ERR_INVALID;
   }

@@ -67,11 +67,13 @@ def parse_cli(argv) -> Experiment:
 
 
 def load_model(result_path: str, device="cuda", max_batch: int = 50, with_stage1: bool = True,
-               precision: str = "bf16", stage1_precision: str = "bf16") -> ImageGPT2:
-    """:25-31 - config only, no checkpoint: random-init weights of the named architecture."""
+               precision: str = "bf16", stage1_precision: str = "bf16", max_seq_len: int = 64) -> ImageGPT2:
+    """:25-31 - config only, no checkpoint: random-init weights of the named architecture.  max_seq_len: top positions the
+    engine is built for (top_resolution ** 2 in the reference protocol)."""
     dev = torch.device(device)
     return ImageGPT2.from_config(result_path, device=dev.index or 0, precision=precision, max_batch=max_batch,
-                                 with_stage1=with_stage1, stage1_max_batch=min(max_batch, 32), stage1_precision=stage1_precision)
+                                 with_stage1=with_stage1, stage1_max_batch=min(max_batch, 32), stage1_precision=stage1_precision,
+                                 max_seq_len=max_seq_len)
 
 
 def main(args: Experiment):
@@ -85,7 +87,8 @@ def main(args: Experiment):
         raise SystemExit(f"stage1_precision={args.stage1_precision!r}: bf16 or tf32")
     model_ar = load_model(args.model_path, device, args.batch_size,
                           with_stage1=bool(args.stage1) and args.code_levels == 2, precision=args.precision,
-                          stage1_precision=args.stage1_precision).to(device).eval()
+                          stage1_precision=args.stage1_precision,
+                          max_seq_len=args.top_resolution * args.top_resolution).to(device).eval()
     if (args.code_levels == 3) != hasattr(model_ar.stage2, "code_level"):
         raise SystemExit(f"code_levels={args.code_levels} does not match the model type of {args.model_path}")
     title = f"bs{args.batch_size}, sampling loops {args.warmup + 1}-{args.n_loop}"

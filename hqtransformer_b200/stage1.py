@@ -52,6 +52,7 @@ class HQVAEDecoder:
         self.attn_resolution = int(attn_resolutions[0])
         self.latent_res = resolution // 2 ** len(self.ch_mult)
         self.max_batch = int(max_batch)
+        self._reserved_top = self.latent_res // 2          # top grid the decoder's buffers are sized for
         mult = (C.c_int32 * 8)(*(list(self.ch_mult) + [0] * (8 - len(self.ch_mult))))
         cfg = HQS1Config(embed_dim=embed_dim, n_embed=n_embed, z_channels=z_channels, resolution=resolution, ch=ch,
                          ch_mult=mult, n_levels=len(self.ch_mult), num_res_blocks=num_res_blocks,
@@ -188,25 +189,43 @@ class HQVAEDecoder:
     # ---- the reference call ----
     @torch.no_grad()
     def decode_code(self, code_t: torch.Tensor, code_b: torch.Tensor) -> torch.Tensor:
-        """generator.py:323-367 with both grids: code_t int64 [B, h, w], code_b int64 [B, 2h, 2w] -> float32 [B, out_ch, R, R].
-        Batches above `max_batch` are decoded in chunks."""
+        """generator.py:323-367 with both grids: code_t int64 [B, h, h], code_b int64 [B, 2h, 2h] -> float32 [B, out_ch, R, R],
+        R = 2h * 2^len(ch_mult).  Any square grid: the configured one (h = latent_res / 2, R = resolution) or another, e.g.
+        16 x 16 / 32 x 32 -> 512 x 512 on the shipped 256-pixel decoder; AttnBlocks stay at the levels the configuration
+        puts them, as in the reference module.  The first grid larger than any before grows the decoder's buffers
+        (hq_s1_reserve_grid: synchronises the device).  Batches above `max_batch` are decoded in chunks."""
         if code_t is None or code_b is None:
             raise NotImplementedError("decode_code needs both grids (top-only / bottom-only decoding is not implemented)")
-        h = self.latent_res // 2
         ct = code_t.to(device=self.device, dtype=torch.int64).contiguous()
         cb = code_b.to(device=self.device, dtype=torch.int64).contiguous()
-        B = ct.shape[0]
-        if tuple(ct.shape) != (B, h, h) or tuple(cb.shape) != (B, 2 * h, 2 * h):
-            raise ValueError(f"expected code_t [B,{h},{h}] and code_b [B,{2 * h},{2 * h}], got {tuple(ct.shape)} / {tuple(cb.shape)}")
+        if ct.dim() != 3 or cb.dim() != 3:
+            raise ValueError(f"expected code_t [B,h,h] and code_b [B,2h,2h], got {tuple(ct.shape)} / {tuple(cb.shape)}")
+        B, h = ct.shape[0], ct.shape[1]
+        if h < 1 or tuple(ct.shape) != (B, h, h) or tuple(cb.shape) != (B, 2 * h, 2 * h):
+            raise ValueError(f"expected square grids code_t [B,h,h] and code_b [B,2h,2h], got {tuple(ct.shape)} / {tuple(cb.shape)}")
         if B and (int(ct.min()) < 0 or int(ct.max()) >= self.n_embed or int(cb.min()) < 0 or int(cb.max()) >= self.n_embed):
             raise IndexError(f"code indices out of range [0, {self.n_embed})")
-        out = torch.empty(B, self.out_ch, self.resolution, self.resolution, dtype=torch.float32, device=self.device)
+        R = 2 * h * 2 ** len(self.ch_mult)
+        out = torch.empty(B, self.out_ch, R, R, dtype=torch.float32, device=self.device)
+        configured = 2 * h == self.latent_res
+        if not configured and h > self._reserved_top:
+            self.reserve_grid(h)
         st = torch.cuda.current_stream(self.device).cuda_stream
         for lo in range(0, B, self.max_batch):
             hi = min(B, lo + self.max_batch)
-            check_s1(self._lib.hq_s1_decode_codes(self._ctx, ct[lo:hi].data_ptr(), cb[lo:hi].data_ptr(), out[lo:hi].data_ptr(),
-                                                  hi - lo, C.c_void_p(st)), self._ctx, self._lib, "hq_s1_decode_codes")
+            if configured:
+                rc = self._lib.hq_s1_decode_codes(self._ctx, ct[lo:hi].data_ptr(), cb[lo:hi].data_ptr(), out[lo:hi].data_ptr(),
+                                                  hi - lo, C.c_void_p(st))
+            else:
+                rc = self._lib.hq_s1_decode_codes_grid(self._ctx, ct[lo:hi].data_ptr(), cb[lo:hi].data_ptr(), h,
+                                                       out[lo:hi].data_ptr(), hi - lo, C.c_void_p(st))
+            check_s1(rc, self._ctx, self._lib, "hq_s1_decode_codes")
         return out
+
+    def reserve_grid(self, top_res: int) -> None:
+        """Sizes the decoder for square top grids up to top_res x top_res (synchronises the device; never shrinks)."""
+        check_s1(self._lib.hq_s1_reserve_grid(self._ctx, int(top_res)), self._ctx, self._lib, "hq_s1_reserve_grid")
+        self._reserved_top = max(self._reserved_top, int(top_res))
 
 
 def debug_s1_conv(A: torch.Tensor, weight: torch.Tensor, bias: torch.Tensor, out: torch.Tensor, mode: int, *,

@@ -94,7 +94,9 @@ typedef struct hq_config {
   int32_t ctx_len_txt;     /* text prefix length (HQ_COND_TXT only) */
   int32_t cond_kind;       /* hq_cond_kind */
   int32_t precision;       /* hq_precision */
-  int32_t max_seq_len;     /* number of top positions a run may cover (64 for 8x8) */
+  int32_t max_seq_len;     /* number of top positions a run may cover (64 for 8x8, 256 for 16x16): <= ctx_len_img, and the
+                              KV cache length T0 + max_seq_len - 1 <= 320 (T0 = ctx_len_txt for text, else 1).  K / V
+                              memory grows with it: 2 * L * max_batch * (T0 + max_seq_len - 1) * embed_dim elements. */
   int32_t use_cuda_graph;  /* 1: capture each run shape once and replay it; 0: plain stream launches */
   int32_t use_pdl;         /* 1: chain the kernels with programmatic dependent launch (prologue of kernel n+1 and
                               its first weight tiles overlap the tail of kernel n); 0: plain stream order */
@@ -170,7 +172,7 @@ typedef struct hq_run_args {
                                 [P, pos_end) are sampled exactly as the loop samples them after those codes (same Philox
                                 counters).  The spatial KV cache of the prefix is computed in one causal pass over its
                                 T0 + P - 1 tokens (no depth pass, head or draw there).  given_top / given_bot / given_mid apply
-                                at positions >= P; logits are written for positions >= P only. */
+                                at positions >= P; logits are written for positions >= P only.  T0 + P - 1 <= 320. */
 } hq_run_args;
 
 typedef struct hq_ctx hq_ctx;
@@ -282,7 +284,8 @@ int hq_debug_sample(const float* logits, int R, int V, float temperature, int to
 
 /* Single-query attention of B rows over `n_keys` cached keys through the kernels the sampler uses: q / out [B, D],
  * K / V [B, t_stride, D] with D = n_heads * 64, device pointers in the precision's activation type (bf16 / fp16 / fp32).
- * variant: 0 = the engine's choice (bf16 / fp16: persistent ldmatrix/mma kernel), 1 = the scalar bulk-staged kernel. */
+ * variant: 0 = the engine's choice (bf16 / fp16: persistent ldmatrix/mma kernel), 1 = the scalar bulk-staged kernel.
+ * 1 <= n_keys <= min(t_stride, 320); past 128 keys the scalar kernels run their 320-key instances. */
 int hq_debug_attention(int prec, const void* q, const void* K, const void* V, void* out, int B, int n_heads,
                        int t_stride, int n_keys, int variant, void* stream);
 
@@ -290,7 +293,8 @@ int hq_debug_attention(int prec, const void* q, const void* K, const void* V, vo
  * cache rows (K / V [B, t_stride, D]), D = n_heads * 64, device pointers in the precision's activation type.
  * variant 0: the kernel of the prefix pass - bf16 / fp16: the tensor-core prefix kernel, fp32: the per-(query, head) warp
  * kernel the fp32 engine runs there; variant 1: the per-(query, head) warp kernel at every precision (what the text prefill
- * runs).  1 <= n_q <= min(t_stride, 128). */
+ * runs).  1 <= n_q <= min(t_stride, 320); bf16 / fp16 variant 0 past 128 queries: the blocked prefix kernel (one CTA per
+ * image, head and 128 queries). */
 int hq_debug_attention_prefix(int prec, const void* q, const void* K, const void* V, void* out, int B, int n_heads,
                               int t_stride, int n_q, int variant, void* stream);
 
@@ -372,6 +376,18 @@ int hq_s1_params_complete(hq_s1_ctx* ctx);
  * asynchronous on `stream`; B <= max_batch.  Codes must lie in [0, n_embed) (the host layer checks). */
 int hq_s1_decode_codes(hq_s1_ctx* ctx, const int64_t* code_t, const int64_t* code_b, float* out, int B, void* stream);
 
+/* Sizes the decoder's activation buffers and QKV for square top grids up to top_res x top_res (bottom grids 2 top_res,
+ * images top_res * 2^(n_levels + 1) pixels wide); never shrinks them.  Synchronises the device first: call it outside any
+ * stream work.  The bytes count in hq_s1_device_bytes.  AttnBlocks stay at the levels the configuration puts them (as in
+ * the reference module), so a larger grid attends over more pixels there: HQ_ERR_UNSUPPORTED if an attention core cannot
+ * take that many. */
+int hq_s1_reserve_grid(hq_s1_ctx* ctx, int top_res);
+
+/* hq_s1_decode_codes for code_t int64 [B, h, h], code_b [B, 2h, 2h] with h = top_res <= the reserved size (the configured
+ * size needs no reserve) -> out fp32 [B, out_ch, R, R], R = 2h * 2^n_levels.  Allocates nothing. */
+int hq_s1_decode_codes_grid(hq_s1_ctx* ctx, const int64_t* code_t, const int64_t* code_b, int top_res, float* out, int B,
+                            void* stream);
+
 /* 2 * MACs of the convolutions of the last hq_s1_decode_codes call (interior pixels only): the roofline numerator. */
 double hq_s1_last_conv_flops(const hq_s1_ctx* ctx);
 
@@ -408,7 +424,8 @@ int hq_debug_s1_quant(int prec, const int64_t* code_t, const int64_t* code_b, co
 
 /* AttnBlock core softmax(q k^T C^-1/2) v over the res x res pixels of each image: qkv padded T [.., 3C] (q | k | v),
  * out padded T [.., C], interior written.  variant 0: the decoder's choice (bf16: the tensor-core kernel when N = res^2
- * is a multiple of 16 and <= 256 and C a multiple of 128 and <= 512); 1: the CUDA-core kernel.  C % 8 == 0; the
+ * is a multiple of 16 and <= 256 and C a multiple of 128 and <= 512; up to 1024 tokens the two-sweep tensor-core
+ * kernel); 1: the CUDA-core kernel.  C % 8 == 0; the
  * CUDA-core kernel needs 32 (C + N) bytes <= 96 KB of shared memory. */
 int hq_debug_s1_attention(int prec, const void* qkv, void* out, int B, int res, int C, int variant, void* stream);
 
